@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Chamfer+Hausdorff fwd+bwd throughput of the B200 point-set distance path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -119,6 +119,16 @@ class ClockSampler(threading.Thread):
         sm = sorted(self.sm)
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": self.max_mhz,
                 "reasons": sorted(self.reasons), "samples": len(sm)}
+
+
+def dump_outputs(out_dir, rank, world, **arrays):
+    """Write what the timed step returns to its caller (the loss, the four per-sample loss vectors of
+    distance.chamfer / distance.hausdorff and the gradient w.r.t. adv, 1.6 MB per rank) as float32
+    <name>.npy, so that two builds can be compared output for output on the same seeded inputs."""
+    import numpy as np
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), t.detach().float().cpu().numpy())
 
 
 def make_inputs(B, first_sample):
@@ -345,6 +355,9 @@ def run_ours(args):
     total_ms = sum(step_ms)
     launches = launches_per_step * args.steps
     losses = graphed.aux[0]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, loss=graphed.loss, chamfer_1=losses[0], chamfer_2=losses[1],
+                     hausdorff_1=losses[2], hausdorff_2=losses[3], grad_adv=graphed.grad)
     # the replayed graph must reproduce the eager result bit for bit
     ref_losses = step(adv.detach().clone().requires_grad_(True), ori)
     if not torch.equal(ref_losses, losses):
@@ -535,7 +548,15 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (loss, per-sample Chamfer/Hausdorff, gradient) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs needs --impl ours")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -127,9 +127,33 @@ def test_signatures_mirror_the_reference():
         assert callable(getattr(pcd.dis_utils_torch, fn))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not mounted")
-def test_install_patches_reference_modules():
-    sys.path.insert(0, "/root/reference")
+# A stand-in for the reference checkout: its package layout, module names and the names install() patches or must leave
+# alone, with placeholder bodies. dist_utils binds chamfer / hausdorff at import time, as dist_utils.py:6 does.
+REFERENCE_STUB = {
+    "utils/dis_utils_torch.py": "def chamfer(a, b): pass\ndef sgd_hausdorff_dis(a, b): pass\ndef bid_hausdorff_dis(a, b): pass\n",
+    "attack/CW/CW_utils/distance.py": "class ChamferDistance: pass\nclass HausdorffDistance: pass\n"
+                                      "chamfer = ChamferDistance()\nhausdorff = HausdorffDistance()\n",
+    "attack/CW/CW_utils/dist_utils.py": "from attack.CW.CW_utils.distance import chamfer, hausdorff\n"
+                                        "class L2Dist: pass\nclass ChamferDist: pass\nclass HausdorffDist: pass\n"
+                                        "class KNNDist: pass\nclass ChamferkNNDist: pass\n",
+    "attack/CW/CW_utils/clip_utils.py": "class ClipPointsL2: pass\nclass ClipPointsLinf: pass\n"
+                                        "class ProjectInnerPoints: pass\nclass ProjectInnerClipLinf: pass\n",
+    "attack/GeoA3/knn_utils.py": "def knn_points(p1, p2, lengths1=None, lengths2=None, K=1): pass\n"
+                                 "def knn_gather(x, idx, lengths=None): pass\n",
+    "attack/AOF/TAOF_attack.py": "def knn(x, k): pass\ndef get_Laplace_from_pc(ori_pc): pass\n",
+    "model/dgcnn.py": "def knn(x, k): pass\ndef get_graph_feature(x, k=20, idx=None): pass\n",
+    "model/pointnet2_utils.py": "def query_ball_point(radius, nsample, xyz, new_xyz): pass\n"
+                                "def farthest_point_sample(xyz, npoint): pass\n",
+}
+
+
+def test_install_patches_reference_modules(tmp_path):
+    for rel, src in REFERENCE_STUB.items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(src)
+    for pkg in [d for d in tmp_path.rglob("*") if d.is_dir()]:
+        (pkg / "__init__.py").touch()
+    sys.path.insert(0, str(tmp_path))
     try:
         rep = pcd.install.install(modules=["utils.dis_utils_torch", "attack.CW.CW_utils.distance",
                                            "attack.CW.CW_utils.dist_utils", "attack.GeoA3.knn_utils",
@@ -148,7 +172,7 @@ def test_install_patches_reference_modules():
         assert DU.ChamferDist is pcd.dist_utils.ChamferDist and MD.knn is pcd.dgcnn.knn
         assert hasattr(DU, "L2Dist")                       # untouched names stay the reference's
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(str(tmp_path))
         for m in [m for m in sys.modules if m.split(".")[0] in ("attack", "model", "utils")]:
             del sys.modules[m]
 
