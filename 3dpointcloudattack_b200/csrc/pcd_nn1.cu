@@ -81,25 +81,14 @@ constexpr int kFixupMaxWarps = 16384;             // upper bound of the persiste
 
 struct Nn1Layout {
     int Npad, Mpad;
-    size_t rowkey, colkey, maxnorm, counters, partials, rowslot, colslot, queue, pending, rowpk, rowpp, colpk, total;
+    size_t rowkey, colkey, counters, partials, rowpk, rowpp, colpk, total;
     size_t nkeys;
     int partial_slots;     // fix-up partials per sample (one per 32-point unit)
-    int apx_R, apx_nord, apx_nqt;   // approximate sweep: the tiling the slot arrays are sized for (0: no slot arrays)
 };
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-static void choose_tiling(int B, int N, int M, int sms, int force_R, int force_mt, int *R_out, int *mt_out);
-constexpr int kQuadCols = 4;
-// Upper bound of the number of CTAs of a G-CTA stream-K grid that touch one row tile (nq column quads of `units`)
-static inline int apx_nord_bound(long long units, long long nq, long long G) {
-    const long long upc = units / G > 0 ? units / G : 1;       // every CTA owns at least floor(units / G) units
-    long long n = nq / upc + 2;
-    if (n > nq) n = nq;
-    if (n > G) n = G;
-    return (int)(n < 1 ? 1 : n);
-}
 // keys + counters first (all the dense-input path touches), the packed records of the strided
-// path behind them.  sweep_mode == PCD_SWEEP_APPROX adds the slot arrays of the approximate sweep.
-static Nn1Layout nn1_layout(int B, int N, int M, int sweep_mode, int sms) {
+// path behind them
+static Nn1Layout nn1_layout(int B, int N, int M) {
     Nn1Layout L;
     L.Npad = (int)align_up((size_t)N, kRowPadUnit);
     L.Mpad = (int)align_up((size_t)M, kMaxColTile);
@@ -107,28 +96,9 @@ static Nn1Layout nn1_layout(int B, int N, int M, int sweep_mode, int sms) {
     L.rowkey = off; off += (size_t)B * L.Npad * 8;
     L.colkey = off; off += (size_t)B * L.Mpad * 8;
     L.nkeys = (size_t)B * L.Npad + (size_t)B * L.Mpad;
-    L.maxnorm = off; off = align_up(off + (size_t)B * 8, 16);   // APX: per sample ~bits of the largest row / column norm
-    // [B] completion counters, then the length of the near-tie queue (APX) and two development counters
-    L.counters = off; off = align_up(off + (size_t)(B + 4) * 4, 256);
+    L.counters = off; off = align_up(off + (size_t)B * 4, 256);      // [B] completion counters
     L.partial_slots = (N + 31) / 32 + (M + 31) / 32;          // one partial per unit of 32 points: rows first, then columns
     L.partials = off; off = align_up(off + (size_t)B * L.partial_slots * 16, 256);       // (sum, max, bits of argmax, -)
-    L.apx_R = L.apx_nord = L.apx_nqt = 0;
-    L.rowslot = L.colslot = L.queue = L.pending = off;
-    if (sweep_mode == PCD_SWEEP_APPROX && sms > 0) {
-        // one key per (sample, CTA ordinal within the row tile, row) and per (sample, row tile, column): plain stores, one
-        // writer each; sized for the tiling the heuristic picks (a forced tiling that needs more falls back to EXACT)
-        static const int occ_of_R[17] = {0, 0, 6, 0, 5, 0, 0, 0, 4, 0, 0, 0, 0, 0, 0, 0, 2};
-        int R = 16, mt = 0;
-        choose_tiling(B, N, M, sms, 0, 0, &R, &mt);
-        const long long nqt = (N + 128 * R - 1) / (128 * R), nq = (M + kQuadCols - 1) / kQuadCols;
-        L.apx_R = R;
-        L.apx_nqt = (int)nqt;
-        L.apx_nord = apx_nord_bound((long long)B * nqt * nq, nq, (long long)sms * occ_of_R[R]);
-        L.rowslot = off; off = align_up(off + (size_t)B * L.apx_nord * L.Npad * 8, 256);
-        L.colslot = off; off = align_up(off + (size_t)B * L.apx_nqt * L.Mpad * 8, 256);
-        L.queue = off; off = align_up(off + (size_t)B * ((size_t)N + M) * 4, 256);          // every point may be a near tie
-        L.pending = off; off = align_up(off + (size_t)B * L.partial_slots * 4, 256);
-    }
     L.rowpk = off; off = align_up(off + (size_t)B * L.Npad * 16, 256);
     L.rowpp = off; off = align_up(off + (size_t)B * L.Npad * 16, 256);   // the same records in sweep (slot) order
     L.colpk = off; off = align_up(off + (size_t)B * L.Mpad * 16 + 64, 256);   // +64: the sweep prefetches one record past a tile
@@ -245,7 +215,6 @@ struct SweepSmem {
     float rraw[kSweepWarps * 32 * R * 3];            // RAW: xyz of the CTA's row tile
     uint64_t full[2];                                // mbarriers: tile[s] / craw[s] has landed
     uint64_t rfull;                                  // mbarrier: rraw has landed
-    uint32_t colmax[3];                              // APX: bits of the largest column norm of tile it (slot it % 3)
 };
 template <int R>
 struct SweepSmemPacked {
@@ -266,33 +235,11 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
 }
 #endif
 
-// APX (RAW only): the APPROXIMATE sweep.  Only the fix-up has to reproduce the reference's roundings; the sweep may rank the
-// pairs with any value that is provably close.  v = fma(qz,cz, fma(qy,cy, fma(qx,cx, ncol))) feeds the row minima and
-// a = v + nrow the column minima: FOUR packed instructions per two pairs instead of five (6.45 vs 7.26 cycles per pair in
-// tools/sweep_lab.cu).  Both a and the reference's d are within (4 + 5) * 2^-24 * T of the real value, T = nrow + ncol +
-// 2|q.c| <= 2 (nrow + ncol), so the reference's arg-min lies in a chunk (lane group) whose approximate minimum is within
-//     W = kApxWindow * (largest row norm + largest column norm)
-// of the best one.  The sweep therefore publishes a candidate SET instead of one winner, with plain stores (every slot has
-// exactly one writer; no atomics, nothing to arm):
-//   rows     rowslot[b][ord][row] = this CTA's (best v, chunk) for the row, ord = the CTA's ordinal among the CTAs of the
-//            stream-K grid that touch the row tile (computable from the split); bit 31 of the tag = two chunks of THIS CTA
-//            were within the window of each other (one flag per row, updated per chunk);
-//   columns  colslot[b][row tile][column] = (best a, warp and lowest candidate lane); the warp's ballot takes every lane with
-//            partial <= warp minimum + W, bit 31 = several lanes, or another warp of the CTA, are within the window.
-// The fix-up reads the few slots of a point, finds best and second-best itself, rescans the tagged candidates with the
-// reference's arithmetic and, where a second candidate is within the sample's window, the whole row (column).
-constexpr float kApxWindow = 40.0f * 5.9604644775390625e-08f;      // 40 * 2^-24 (needed: 36)
-#ifndef PCD_APX_LEVEL      // development builds only (tools/apx_levels.py, TIMING of the sweep only -- the results are not valid below 4):
-#define PCD_APX_LEVEL 4    // 1 = the cheaper math alone, 2 = + window ballot, 3 = + per-chunk near-tie flags, 4 = + slot stores (the product)
-#endif
-
-template <int FORM, int R, bool RAW, bool APX>
+template <int FORM, int R, bool RAW>
 __global__ void __launch_bounds__(kSweepThreads, (R >= 16) ? 2 : ((R >= 8) ? 4 : ((R >= 4) ? 5 : 6)))
 nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned long long *__restrict__ colkey,
-                 unsigned long long *__restrict__ rowslot, unsigned long long *__restrict__ colslot, int nord,
-                 uint32_t *__restrict__ maxnorm, int N, int Npad, int Mpad, int qpt /* quads per TMA tile */, int nqt, int nq /* quads per row tile */,
+                 int N, int Npad, int Mpad, int qpt /* quads per TMA tile */, int nqt, int nq /* quads per row tile */,
                  int units) {
-    static_assert(RAW || !APX, "the approximate sweep streams raw operands");
     constexpr int QW = 32 * R;            // rows per warp
     constexpr int QT = kSweepWarps * QW;  // rows per CTA tile
     constexpr int kQuadsPerChunk = kColChunk / kQuad;
@@ -306,7 +253,7 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
     // Stream-K at 4-column granularity: the (sample, row tile, column quad) space is cut into
     // gridDim.x equal contiguous ranges, so every CTA sweeps the same number of pairs (+-1 quad).
     // Ranges may start or end inside a 32-column chunk: a row tag only says "the minimum is in
-    // this chunk", and the fix-up rescans the whole chunk, so partial chunks stay exact.
+    // this chunk", and the fix-up re-scans the whole chunk, so partial chunks stay exact.
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 #ifdef PCD_SWEEP_TRACE
     unsigned long long *trace = g_sweep_trace;
@@ -370,8 +317,7 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
         }
     };
     // RAW: craw[s] (ncols raw columns) -> pair records {x0,x1,y0,y1},{z0,z1,n0,n1} in tile[d]
-    auto convert = [&](int s, int d, int ncols, int slot) {
-        (void)slot;
+    auto convert = [&](int s, int d, int ncols) {
         if constexpr (RAW) {
             const int p = tid;                               // pair record index; ncols is a multiple of 4
             if (2 * p < ncols) {
@@ -389,10 +335,6 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
                 const float n0 = sq_norm3(src.norm_kind, x0, y0, z0), n1 = sq_norm3(src.norm_kind, x1, y1, z1);
                 sm.tile[d][2 * p] = make_float4(x0, x1, y0, y1);
                 sm.tile[d][2 * p + 1] = make_float4(z0, z1, n0, n1);
-                if constexpr (APX) {      // norms are >= +0 (or NaN / inf): their bit patterns order like unsigned integers
-                    const uint32_t b0 = __float_as_uint(n0), b1 = __float_as_uint(n1);
-                    atomicMax(&sm.colmax[slot], b0 > b1 ? b0 : b1);
-                }
             }
         }
     };
@@ -400,7 +342,6 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
         mbar_init(&sm.full[0], 1);
         mbar_init(&sm.full[1], 1);
         if constexpr (RAW) mbar_init(&sm.rfull, 1);
-        if constexpr (APX) { sm.colmax[0] = 0u; sm.colmax[1] = 0u; sm.colmax[2] = 0u; }
         fence_mbar_init();
         fence_proxy_async();
         issue(0);
@@ -411,7 +352,7 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
     if constexpr (RAW) {
         // tile 0: convert in front of the loop; its raw buffer is then free for tile 2
         mbar_wait(&sm.full[0], 0);
-        convert(0, 0, seg_len(u0) * kQuad, 0);
+        convert(0, 0, seg_len(u0) * kQuad);
         __syncthreads();
         if (tid == 0) issue(0);
     }
@@ -422,26 +363,11 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
     size_t row_base = 0;
     uint32_t rpar = 0;
     bool armed = !RAW;     // RAW: griddepcontrol.wait not executed yet (keys are armed by our predecessor)
-    // APX: near-tie flags of this lane's rows (bit r), bits of the warp's largest row norm, the window of the current
-    // segment and its running maximum over the segments of the current row tile
-    uint32_t flags = 0u, wrow_bits = 0u;
-    float Wc = 0.f, wrun = 0.f;
     const float pinf = __int_as_float(0x7f800000);
     // publish the running row minima of the current row tile
-    size_t slot_base = 0;                                     // APX: this CTA's slot plane of the current row tile
     auto flush_rows = [&]() {
 #pragma unroll
-        for (int r = 0; r < R; ++r) {
-            if constexpr (APX && PCD_APX_LEVEL >= 4) {
-                const unsigned long long key = make_key(best[r], btag[r] | (((flags >> r) & 1u) << 31));
-                rowslot[slot_base + r * 32] = key;
-            } else {
-                atomicMin(&rowkey[row_base + r * 32], make_key(best[r], btag[r]));
-            }
-        }
-        if constexpr (APX) {
-            if (lane == 0) atomicMin(&maxnorm[2 * (cur_bq / nqt)], ~wrow_bits);
-        }
+        for (int r = 0; r < R; ++r) atomicMin(&rowkey[row_base + r * 32], make_key(best[r], btag[r]));
     };
 #ifdef PCD_SWEEP_TRACE
     long long t_row = 0, t_comp = 0, t_bar = 0, t_flush = 0, t_mark = clock64();
@@ -461,19 +387,11 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
             if (cur_bq >= 0) flush_rows();
             cur_bq = bq;
             row_base = (size_t)b * Npad + (size_t)qt * QT + warp * QW + lane;    // key slot of row r: + r*32
-            if constexpr (APX) {
-                // ordinal of this CTA among the CTAs whose unit range [units*c/G, units*(c+1)/G) meets the tile's [bq*nq, (bq+1)*nq)
-                const long long first = (((long long)bq * nq + 1) * gridDim.x - 1) / units;
-                int ordv = (int)((long long)blockIdx.x - first);
-                ordv = ordv < 0 ? 0 : (ordv >= nord ? nord - 1 : ordv);           // (never clamps: nord is an upper bound)
-                slot_base = ((size_t)b * nord + ordv) * Npad + (size_t)qt * QT + warp * QW + lane;
-            }
             if constexpr (RAW) {
                 mbar_wait(&sm.rfull, rpar);
                 rpar ^= 1u;
                 pulled = true;
                 const int l0 = warp * QW + lane * R;            // first of this lane's rows inside the tile
-                uint32_t mxb = 0u;
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
                     float x = 0.f, y = 0.f, z = 0.f, n = __int_as_float(0x7f800000);
@@ -481,16 +399,10 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
                         if (src.row_cm) { x = sm.rraw[l0 + r]; y = sm.rraw[QT + l0 + r]; z = sm.rraw[2 * QT + l0 + r]; }
                         else { x = sm.rraw[(l0 + r) * 3]; y = sm.rraw[(l0 + r) * 3 + 1]; z = sm.rraw[(l0 + r) * 3 + 2]; }
                         n = sq_norm3(src.norm_kind, x, y, z);
-                        if constexpr (APX) mxb = max(mxb, __float_as_uint(n));
                     }
                     qx[r] = -2.f * x; qy[r] = -2.f * y; qz[r] = -2.f * z; qn[r] = n;
                     best[r] = __int_as_float(0x7f800000);
                     btag[r] = 0;
-                }
-                if constexpr (APX) {
-                    wrow_bits = __reduce_max_sync(0xffffffffu, mxb);      // the live rows of the whole warp (padding excluded)
-                    flags = 0u;
-                    wrun = 0.f;
                 }
             } else {
 #pragma unroll
@@ -509,14 +421,6 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
 #endif
         PCD_PHASE(t_row);
 
-        uint32_t cmax_bits = 0u;
-        if constexpr (APX) {
-            cmax_bits = sm.colmax[it % 3];
-            if (tid == 0) sm.colmax[(it + 2) % 3] = 0u;          // read one iteration ago, written again in the next one
-            Wc = __fmul_ru(kApxWindow, __fadd_ru(__uint_as_float(wrow_bits), __uint_as_float(cmax_bits)));
-            if (!(Wc >= 0.f)) Wc = pinf;                         // NaN norms: everything is a candidate
-            wrun = fmaxf(wrun, Wc);
-        }
         const float4 *t4 = sm.tile[buf];
         uint2 *cp = sm.colpart[buf][warp];
         float4 A = t4[0], Bv = t4[1];                       // operands of the step about to run
@@ -541,17 +445,9 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
                     float lo[R], hi[R];
 #pragma unroll
                     for (int r = 0; r < R; ++r) {
-                        if constexpr (APX) {
-                            const f32x2 v = fma2_s(qz[r], Z, fma2_s(qy[r], Y, fma2_s(qx[r], X, Nn)));
-                            float vl, vh;
-                            unpack2(v, vl, vh);
-                            m[r] = min3(m[r], vl, vh);                       // rows rank by v (their own norm is a constant offset)
-                            unpack2(add2_s(qn[r], v), lo[r], hi[r]);
-                        } else {
-                            const f32x2 d = pair_dist_x2<FORM>(qx[r], qy[r], qz[r], qn[r], X, Y, Z, Nn);
-                            unpack2(d, lo[r], hi[r]);
-                            m[r] = min3(m[r], lo[r], hi[r]);
-                        }
+                        const f32x2 d = pair_dist_x2<FORM>(qx[r], qy[r], qz[r], qn[r], X, Y, Z, Nn);
+                        unpack2(d, lo[r], hi[r]);
+                        m[r] = min3(m[r], lo[r], hi[r]);
                     }
                     float clo = lo[0], chi = hi[0];
 #pragma unroll
@@ -566,23 +462,14 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
                     // retire the previous step's column results (their CREDUX latency is long gone)
                     if (pend_at >= 0) *reinterpret_cast<uint4 *>(&cp[pend_at]) = make_uint4(pend_lo.x, pend_lo.y, pend_hi.x, pend_hi.y);
                     const float vlo = warp_min_f32(clo), vhi = warp_min_f32(chi);
-                    if constexpr (APX && PCD_APX_LEVEL >= 2) {      // every lane whose partial minimum is within the window of the warp's
-                        pend_lo = make_uint2(__float_as_uint(vlo), __ballot_sync(0xffffffffu, clo <= __fadd_ru(vlo, Wc)));
-                        pend_hi = make_uint2(__float_as_uint(vhi), __ballot_sync(0xffffffffu, chi <= __fadd_ru(vhi, Wc)));
-                    } else {
-                        pend_lo = make_uint2(__float_as_uint(vlo), __ballot_sync(0xffffffffu, clo == vlo));
-                        pend_hi = make_uint2(__float_as_uint(vhi), __ballot_sync(0xffffffffu, chi == vhi));
-                    }
+                    pend_lo = make_uint2(__float_as_uint(vlo), __ballot_sync(0xffffffffu, clo == vlo));
+                    pend_hi = make_uint2(__float_as_uint(vhi), __ballot_sync(0xffffffffu, chi == vhi));
                     pend_at = 2 * step;
                     A = An; Bv = Bn;
                 }
             }
 #pragma unroll
             for (int r = 0; r < R; ++r) {
-                if constexpr (APX && PCD_APX_LEVEL >= 3) {      // is the loser of (chunk minimum, running best) within the window of the winner?
-                    const float nb = fminf(m[r], best[r]), ob = fmaxf(m[r], best[r]);
-                    if (ob <= __fadd_ru(nb, wrun)) flags |= 1u << r;
-                }
                 if (m[r] < best[r]) {
                     best[r] = m[r];
                     btag[r] = (uint32_t)chunk;
@@ -597,7 +484,7 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
             // (tile[buf^1] was last read one barrier ago)
             if (u + nseg < u1) {
                 mbar_wait(&sm.full[buf ^ 1], ((it + 1) >> 1) & 1);
-                convert(buf ^ 1, buf ^ 1, seg_len(u + nseg) * kQuad, (it + 1) % 3);
+                convert(buf ^ 1, buf ^ 1, seg_len(u + nseg) * kQuad);
             }
         }
         __syncthreads();  // tile[buf] fully read, colpart[buf] fully written, RAW: tile[buf^1] converted, craw[buf^1] and rraw free
@@ -617,28 +504,18 @@ nn1_sweep_kernel(SweepSrc src, unsigned long long *__restrict__ rowkey, unsigned
         }
         // column flush: min over the CTA's warps (lowest warp on ties), lowest lane of its ballot
         const int ncols = nseg * kQuad;
-        if constexpr (APX) {
-            if (tid == 0) atomicMin(&maxnorm[2 * b + 1], ~cmax_bits);
-        }
         for (int col = tid; col < ncols; col += kSweepThreads) {
             uint2 e = sm.colpart[buf][0][col];
-            float v = __uint_as_float(e.x), second = pinf;
+            float v = __uint_as_float(e.x);
             uint32_t w = 0, msk = e.y;
 #pragma unroll
             for (int k = 1; k < kSweepWarps; ++k) {
                 const uint2 o = sm.colpart[buf][k][col];
                 const float ov = __uint_as_float(o.x);
-                if (ov < v) { second = fminf(second, v); v = ov; w = k; msk = o.y; }
-                else second = fminf(second, ov);
+                if (ov < v) { v = ov; w = k; msk = o.y; }
             }
             const uint32_t ctag = (((uint32_t)qt * kSweepWarps + w) << 5) + (uint32_t)((__ffs(msk) - 1) & 31);
-            if constexpr (APX && PCD_APX_LEVEL >= 4) {
-                // one writer per (row tile, column): a plain store; bit 31 = more than one candidate inside this CTA
-                const bool many = __popc(msk) > 1 || !(second > __fadd_ru(v, Wc));
-                colslot[((size_t)b * nqt + qt) * Mpad + (size_t)q0 * kQuad + col] = make_key(v, ctag | (many ? 0x80000000u : 0u));
-            } else if (v < pinf) {
-                atomicMin(&colkey[(size_t)b * Mpad + (size_t)q0 * kQuad + col], make_key(v, ctag));
-            }
+            if (v < pinf) atomicMin(&colkey[(size_t)b * Mpad + (size_t)q0 * kQuad + col], make_key(v, ctag));
         }
         u += nseg;
         PCD_PHASE(t_flush);
@@ -960,30 +837,15 @@ struct StagedArgs {
     int parts_row, parts_col;   // slices per (sample, side): a row point scans 32 candidates, a column point R, so the
                                 // sides get slice counts in proportion to their work
     int stage_stride;           // channel-major staging: floats between the channel rows (multiple of 32)
-    // APX: what the approximate sweep published (see nn1_sweep_kernel) and the geometry of its grid
-    const unsigned long long *rowslot, *colslot;
-    const uint32_t *maxnorm;
-    int nord, nqt, nq, sweep_grid;
-    long long sweep_units;
-    // near-tie points go to a grid-wide queue that nn1_rescan_kernel serves (entry = b << 16 | side << 15 | point);
-    // pending[b * units_per_sample + unit] = flagged points of the unit still to be settled
-    uint32_t *queue; int *qcount; int *pending;
 };
-constexpr int kSlotRegs = 6;      // slot keys of the NEXT unit held in registers while the current one is evaluated
 
-// APX: the keys come from the approximate sweep (see nn1_sweep_kernel).  The tagged candidates are evaluated with the
-// reference's arithmetic and the exact (minimum, lowest index) is taken over them -- not an equality match with the
-// sweep's value.  Where the second-best approximate value of the point is within the sample's window of the best one the
-// tagged candidates may miss the reference's arg-min: the warp then rescans the whole row (column) of that point
-// together, 32 lanes over the staged cloud, and the lane keeps the exact result.
-template <int FORM, int NORM, bool APX>
-__global__ void __launch_bounds__(kFixupThreads, APX ? 2 : 3)
+template <int FORM, int NORM>
+__global__ void __launch_bounds__(kFixupThreads, 3)
 nn1_fixup_staged_kernel(StagedArgs sa) {
     const FixupArgs &a = sa.f;
     extern __shared__ __align__(128) float stage[];
     __shared__ uint64_t bar;
     __shared__ int s_last;
-    if constexpr (APX) pdl_launch_dependents();      // nn1_rescan_kernel may be scheduled as our CTAs retire; it waits for our completion
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int N = a.N, M = a.M, R = a.R;
     const int per_sample = sa.parts_row + sa.parts_col;
@@ -1023,50 +885,17 @@ nn1_fixup_staged_kernel(StagedArgs sa) {
     const int units = (n_own + 31) >> 5;
     const int u0 = (int)((long long)units * q / parts), u1 = (int)((long long)units * (q + 1) / parts);
     const unsigned long long *keys = side ? a.colkey + (size_t)b * a.Mpad : a.rowkey + (size_t)b * a.Npad;
-    float Wb = 0.f;                                   // the sample's window (see kApxWindow)
-    if constexpr (APX) {
-        const float mr = __uint_as_float(~__ldcg(&sa.maxnorm[2 * b])), mc = __uint_as_float(~__ldcg(&sa.maxnorm[2 * b + 1]));
-        Wb = __fmul_ru(kApxWindow, __fadd_ru(mr, mc));
-        if (!(Wb >= 0.f)) Wb = __int_as_float(0x7f800000);
-    }
     float *out_min = side ? a.col_min + (size_t)b * M : a.row_min + (size_t)b * N;
     int32_t *out_arg = side ? a.col_arg + (size_t)b * M : a.row_arg + (size_t)b * N;
 
-    // The keys of a point.  EXACT: one key.  APX: one slot per CTA of the sweep that met the point's row tile (rows), per row
-    // tile (columns); the first kSlotRegs are requested here, a unit ahead, the reduction happens when the unit is evaluated.
-    struct Keys { unsigned long long k[APX ? kSlotRegs : 1]; int n; size_t base; size_t stride; };
-    auto slot_range = [&](int u, int &n, size_t &base, size_t &stride) {
-        if (side) { n = sa.nqt; base = (size_t)b * sa.nqt * a.Mpad; stride = (size_t)a.Mpad; }
-        else {
-            const long long t = (long long)b * sa.nqt + (u * 32) / (128 * R);             // the unit's row tile
-            const long long first = ((t * sa.nq + 1) * sa.sweep_grid - 1) / sa.sweep_units;
-            const long long last = ((t + 1) * sa.nq * sa.sweep_grid - 1) / sa.sweep_units;
-            n = (int)(last - first + 1);
-            if (n > sa.nord) n = sa.nord;
-            base = (size_t)b * sa.nord * a.Npad; stride = (size_t)a.Npad;
-        }
-    };
+    // the key and the coordinates of a point are requested here, a unit ahead of its evaluation
     unsigned long long key = 0ull;
-    Keys ks, nks;
     float px = 0.f, py = 0.f, pz = 0.f;
-    auto fetch = [&](int u, unsigned long long &k, Keys &kk, float &x, float &y, float &z) {
+    auto fetch = [&](int u, unsigned long long &k, float &x, float &y, float &z) {
         const int p = u * 32 + lane;
         k = 0ull; x = y = z = 0.f;
-        kk.n = 0; kk.base = 0; kk.stride = 0;
-#pragma unroll
-        for (int o = 0; o < (APX ? kSlotRegs : 1); ++o) kk.k[o] = ~0ull;
         if (u < u1 && p < n_own) {
-            const int slot = side ? p : row_slot(p, R);
-            if constexpr (APX) {
-                slot_range(u, kk.n, kk.base, kk.stride);
-                kk.base += slot;
-                const unsigned long long *sl = side ? sa.colslot : sa.rowslot;
-#pragma unroll
-                for (int o = 0; o < kSlotRegs; ++o)
-                    if (o < kk.n) kk.k[o] = sl[kk.base + (size_t)o * kk.stride];
-            } else {
-                k = keys[slot];
-            }
+            k = keys[side ? p : row_slot(p, R)];
             const float *s = own + (size_t)p * own_sp;
             x = __ldg(s); y = __ldg(s + own_sc); z = __ldg(s + 2 * own_sc);
         }
@@ -1092,52 +921,23 @@ nn1_fixup_staged_kernel(StagedArgs sa) {
         const f32x2 d1 = pair_dist_fixed_x2<FORM>(side == 0, m2x, m2y, m2z, fn, X1, Y1, Z1, sq_norm3_x2(NORM, X1, Y1, Z1));
         unpack2(d0, e0, e1); unpack2(d1, e2, e3);
     };
-    // exact (minimum, lowest index) over the candidates seen so far
-    auto take = [](float e, int j, float &bv, int &arg) {      // +inf never becomes an arg-min: "no finite minimum" is arg 0
-        if (e < bv) { bv = e; arg = j; }
-        else if (e == bv && e < __int_as_float(0x7f800000)) arg = min(arg, j);
-    };
-    int done_units = 0;                              // APX: units of this warp whose partial is already final
-    fetch(u0 + warp, key, ks, px, py, pz);
+    fetch(u0 + warp, key, px, py, pz);
     for (int u = u0 + warp; u < u1; u += kFixupThreads / 32) {
         unsigned long long nkey; float nx, ny, nz;
-        fetch(u + kFixupThreads / 32, nkey, nks, nx, ny, nz);
+        fetch(u + kFixupThreads / 32, nkey, nx, ny, nz);
         const int p = u * 32 + lane;
         float val = 0.f;
         const float pn = sq_norm3(NORM, px, py, pz);
         const float m2x = -2.f * px, m2y = -2.f * py, m2z = -2.f * pz;
-        float bv = __int_as_float(0x7f800000);         // APX: exact minimum over the candidates
+        float bv = __int_as_float(0x7f800000);
         int arg = 0x7fffffff;
-        bool amb = false;
         if (p < n_own) {
-            if constexpr (APX) {
-                // best and second-best of the point's slots (ordered values); equal values count as two candidates
-                const unsigned long long *sl = side ? sa.colslot : sa.rowslot;
-                unsigned long long bk = ~0ull;
-                uint32_t sv = 0xffffffffu;
-                auto offer = [&](unsigned long long k2) {
-                    const uint32_t kv = (uint32_t)(k2 >> 32), bvv = (uint32_t)(bk >> 32);
-                    if (kv < bvv) { sv = sv < bvv ? sv : bvv; bk = k2; }
-                    else sv = sv < kv ? sv : kv;
-                };
-#pragma unroll
-                for (int o = 0; o < kSlotRegs; ++o)
-                    if (o < ks.n) offer(ks.k[o]);
-                for (int o = kSlotRegs; o < ks.n; ++o) offer(sl[ks.base + (size_t)o * ks.stride]);
-                key = bk;
-                const float bvf = ordered_to_f32((uint32_t)(bk >> 32));
-                // a second candidate within the window of the best (or flagged inside its CTA, or no usable window): rescan everything
-                amb = ((uint32_t)bk >> 31) != 0u || (sv != 0xffffffffu && !(ordered_to_f32(sv) > __fadd_ru(bvf, Wb)));
-#ifdef PCD_APX_DEBUG
-                if (amb) atomicAdd(&a.counters[a.B + 1 + side], 1);      // development build: flagged points per side
-#endif
-            }
             const float v = ordered_to_f32((uint32_t)(key >> 32));
-            const uint32_t tag = APX ? ((uint32_t)key & 0x7fffffffu) : (uint32_t)key;
+            const uint32_t tag = (uint32_t)key;
             // Candidates come in groups of four (three LDS.128 in either dense layout) and are evaluated two at a time with the
             // sweep's packed instruction sequence; the fixed point carries the exact factor -2 whichever side it is on.
             int c0 = 0, ngroups = 0;                         // first candidate, groups of 4
-            const bool scan = APX || v < __int_as_float(0x7f800000);       // EXACT: a non-finite minimum has no arg-min (arg 0)
+            const bool scan = v < __int_as_float(0x7f800000);       // a non-finite minimum has no arg-min (arg 0)
             if (!scan) {
             } else if (side == 0) {
                 if (tag < (uint32_t)a.nchunks) { c0 = (int)tag * kColChunk; ngroups = 8; }              // the 32 columns of the winning chunk
@@ -1152,14 +952,10 @@ nn1_fixup_staged_kernel(StagedArgs sa) {
                     if (j < n_opp) {                                                                      // n_opp % 4 == 0: whole groups
                         float e0, e1, e2, e3;
                         eval4(j, m2x, m2y, m2z, pn, e0, e1, e2, e3);
-                        if constexpr (APX) {
-                            take(e0, j, bv, arg); take(e1, j + 1, bv, arg); take(e2, j + 2, bv, arg); take(e3, j + 3, bv, arg);
-                        } else {
-                            if (e3 == v) arg = min(arg, j + 3);
-                            if (e2 == v) arg = min(arg, j + 2);
-                            if (e1 == v) arg = min(arg, j + 1);
-                            if (e0 == v) arg = min(arg, j);
-                        }
+                        if (e3 == v) arg = min(arg, j + 3);
+                        if (e2 == v) arg = min(arg, j + 2);
+                        if (e1 == v) arg = min(arg, j + 1);
+                        if (e0 == v) arg = min(arg, j);
                     }
                 }
             } else if (scan && side == 1 && R < 4 && (tag >> 5) < (uint32_t)a.nrowgroups) {
@@ -1170,172 +966,27 @@ nn1_fixup_staged_kernel(StagedArgs sa) {
                         if (opp_cm) { x = stage[i]; y = stage[sa.stage_stride + i]; z = stage[2 * sa.stage_stride + i]; }
                         else { x = stage[3 * i]; y = stage[3 * i + 1]; z = stage[3 * i + 2]; }
                         const float e = pair_dist_scalar<FORM>(-2.f * x, -2.f * y, -2.f * z, sq_norm3(NORM, x, y, z), px, py, pz, pn);
-                        if constexpr (APX) take(e, i, bv, arg);
-                        else if (e == v) arg = min(arg, i);
+                        if (e == v) arg = min(arg, i);
                     }
                 }
             }
-            if constexpr (!APX) bv = v;
+            bv = v;
         }
         if (p < n_own) {
             if (arg == 0x7fffffff) arg = 0;        // no finite minimum (NaN / inf inputs)
             val = apply_transform(a.transform, bv);
-            out_min[p] = val; out_arg[p] = arg;    // APX: provisional for a flagged point
+            out_min[p] = val; out_arg[p] = arg;
         }
-        const int unit_in_sample = (side ? (N + 31) >> 5 : 0) + u;
-        if constexpr (APX) {
-            // near ties leave for the grid-wide queue; the unit's partial is formed by whoever settles its last flagged point
-            const unsigned fm = __ballot_sync(0xffffffffu, amb);
-            if (fm) {
-                int base = 0;
-                if (lane == 0) {
-                    base = atomicAdd(sa.qcount, __popc(fm));
-                    sa.pending[(size_t)b * a.slots + unit_in_sample] = __popc(fm);
-                }
-                base = __shfl_sync(0xffffffffu, base, 0);
-                if (amb) sa.queue[base + __popc(fm & ((1u << lane) - 1u))] = ((uint32_t)b << 16) | ((uint32_t)side << 15) | (uint32_t)p;
-            } else {
-                store_unit_partial(a, b, unit_in_sample, p < n_own, val, p, lane);
-                ++done_units;
-            }
-        } else {
-            store_unit_partial(a, b, unit_in_sample, p < n_own, val, p, lane);
-        }
-        key = nkey; ks = nks; px = nx; py = ny; pz = nz;
+        store_unit_partial(a, b, (side ? (N + 31) >> 5 : 0) + u, p < n_own, val, p, lane);
+        key = nkey; px = nx; py = ny; pz = nz;
     }
-    if constexpr (APX) {
-        // unit-granular completion: the warp (here or in nn1_rescan_kernel) that completes the sample's last unit folds it
-        int last = 0;
-        if (lane == 0 && done_units > 0) {
-            __threadfence();
-            last = atomicAdd(&a.counters[b], done_units) + done_units == a.slots;
-        }
-        last = __shfl_sync(0xffffffffu, last, 0);
-        if (last) {
-            __threadfence();
-            fold_sample_side(a, b, 0, lane);
-            fold_sample_side(a, b, 1, lane);
-        }
-    } else {
-        if (lane == 0) __threadfence();       // this warp's unit partials are visible before the CTA reports completion
-        __syncthreads();
-        if (tid == 0) s_last = atomicAdd(&a.counters[b], 1) == per_sample - 1;
-        __syncthreads();
-        if (!s_last || warp >= 2) return;
-        __threadfence();
-        fold_sample_side(a, b, warp, lane);   // last CTA of sample b: one warp per side
-    }
-}
-
-// ---------------------------------------------------------------- near-tie rescans (approximate sweep)
-// One warp per queue entry, grid-stride: the point's whole row (column) with the reference's arithmetic, 32 lanes over
-// consecutive groups of four candidates -- coalesced from global memory, so any warp of the grid can serve any point and
-// the clusters of near-duplicate points (consecutive indices, one fix-up warp) spread over the machine.  The warp that
-// settles the last flagged point of a unit forms the unit's partial; the one that completes a sample folds its statistics.
-template <int FORM, int NORM>
-__global__ void __launch_bounds__(256) nn1_rescan_kernel(StagedArgs sa) {
-    const FixupArgs &a = sa.f;
-    const int lane = threadIdx.x & 31;
-    const int N = a.N, M = a.M;
-    pdl_wait();                                            // the queue is complete
-    const int count = *reinterpret_cast<volatile int *>(sa.qcount);
-    const int nwarps = (gridDim.x * blockDim.x) >> 5;
-    const float pinf = __int_as_float(0x7f800000);
-    for (int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; e < count; e += nwarps) {
-        const uint32_t ent = __ldcg(&sa.queue[e]);
-        const int b = (int)(ent >> 16), side = (int)((ent >> 15) & 1u), p = (int)(ent & 0x7fffu);
-        const int n_opp = side ? N : M;
-        const float *own = side ? a.cols + (size_t)b * a.c_sb + (size_t)p * a.c_sp : a.rows + (size_t)b * a.r_sb + (size_t)p * a.r_sp;
-        const long long own_sc = side ? a.c_sc : a.r_sc;
-        const float *opp = side ? a.rows + (size_t)b * a.r_sb : a.cols + (size_t)b * a.c_sb;
-        const bool opp_cm = (side ? a.r_sp : a.c_sp) == 1;
-        const long long opp_sc = side ? a.r_sc : a.c_sc;
-        const float px = __ldg(own), py = __ldg(own + own_sc), pz = __ldg(own + 2 * own_sc);
-        const float pn = sq_norm3(NORM, px, py, pz);
-        const float m2x = -2.f * px, m2y = -2.f * py, m2z = -2.f * pz;
-        float bv = pinf;
-        int arg = 0x7fffffff;
-        auto take = [&](float d, int j) {
-            if (d < bv) { bv = d; arg = j; }
-            else if (d == bv && d < pinf) arg = min(arg, j);
-        };
-        // kUn groups of four candidates per lane and round: all their loads (L2 hits, ~1 us away) are in flight together
-        constexpr int kUn = 4;
-        for (int j0 = 4 * lane; j0 < n_opp; j0 += 128 * kUn) {
-            float4 f[kUn][3];
-#pragma unroll
-            for (int t = 0; t < kUn; ++t) {
-                const int j = j0 + 128 * t;
-                if (j < n_opp) {
-                    if (opp_cm) {
-                        f[t][0] = __ldg(reinterpret_cast<const float4 *>(opp + j));
-                        f[t][1] = __ldg(reinterpret_cast<const float4 *>(opp + opp_sc + j));
-                        f[t][2] = __ldg(reinterpret_cast<const float4 *>(opp + 2 * opp_sc + j));
-                    } else {
-                        const float4 *g = reinterpret_cast<const float4 *>(opp + (size_t)j * 3);
-                        f[t][0] = __ldg(g); f[t][1] = __ldg(g + 1); f[t][2] = __ldg(g + 2);
-                    }
-                }
-            }
-#pragma unroll
-            for (int t = 0; t < kUn; ++t) {
-                const int j = j0 + 128 * t;
-                if (j < n_opp) {
-                    f32x2 X0, X1, Y0, Y1, Z0, Z1;
-                    if (opp_cm) {
-                        X0 = pack2(f[t][0].x, f[t][0].y); X1 = pack2(f[t][0].z, f[t][0].w);
-                        Y0 = pack2(f[t][1].x, f[t][1].y); Y1 = pack2(f[t][1].z, f[t][1].w);
-                        Z0 = pack2(f[t][2].x, f[t][2].y); Z1 = pack2(f[t][2].z, f[t][2].w);
-                    } else {
-                        X0 = pack2(f[t][0].x, f[t][0].w); X1 = pack2(f[t][1].z, f[t][2].y);
-                        Y0 = pack2(f[t][0].y, f[t][1].x); Y1 = pack2(f[t][1].w, f[t][2].z);
-                        Z0 = pack2(f[t][0].z, f[t][1].y); Z1 = pack2(f[t][2].x, f[t][2].w);
-                    }
-                    const f32x2 d0 = pair_dist_fixed_x2<FORM>(side == 0, m2x, m2y, m2z, pn, X0, Y0, Z0, sq_norm3_x2(NORM, X0, Y0, Z0));
-                    const f32x2 d1 = pair_dist_fixed_x2<FORM>(side == 0, m2x, m2y, m2z, pn, X1, Y1, Z1, sq_norm3_x2(NORM, X1, Y1, Z1));
-                    float e0, e1, e2, e3;
-                    unpack2(d0, e0, e1); unpack2(d1, e2, e3);
-                    take(e0, j); take(e1, j + 1); take(e2, j + 2); take(e3, j + 3);
-                }
-            }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-            const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
-            if (ov < bv || (ov == bv && oa < arg)) { bv = ov; arg = oa; }
-        }
-        const int n_own = side ? M : N;
-        float *out_min = side ? a.col_min + (size_t)b * M : a.row_min + (size_t)b * N;
-        int32_t *out_arg = side ? a.col_arg + (size_t)b * M : a.row_arg + (size_t)b * N;
-        const int unit_in_sample = (side ? (N + 31) >> 5 : 0) + (p >> 5);
-        int left = 1;
-        if (lane == 0) {
-            out_min[p] = apply_transform(a.transform, bv);
-            out_arg[p] = arg == 0x7fffffff ? 0 : arg;
-            __threadfence();
-            left = atomicSub(&sa.pending[(size_t)b * a.slots + unit_in_sample], 1) - 1;
-        }
-        left = __shfl_sync(0xffffffffu, left, 0);
-        if (left != 0) continue;
-        // the unit is settled: its partial, then the sample's completion count
-        __threadfence();
-        const int q = (p & ~31) + lane;
-        const bool live = q < n_own;
-        const float val = live ? __ldcg(&out_min[q]) : 0.f;
-        store_unit_partial(a, b, unit_in_sample, live, val, q, lane);
-        int last = 0;
-        if (lane == 0) {
-            __threadfence();
-            last = atomicAdd(&a.counters[b], 1) + 1 == a.slots;
-        }
-        last = __shfl_sync(0xffffffffu, last, 0);
-        if (last) {
-            __threadfence();
-            fold_sample_side(a, b, 0, lane);
-            fold_sample_side(a, b, 1, lane);
-        }
-    }
+    if (lane == 0) __threadfence();       // this warp's unit partials are visible before the CTA reports completion
+    __syncthreads();
+    if (tid == 0) s_last = atomicAdd(&a.counters[b], 1) == per_sample - 1;
+    __syncthreads();
+    if (!s_last || warp >= 2) return;
+    __threadfence();
+    fold_sample_side(a, b, warp, lane);   // last CTA of sample b: one warp per side
 }
 
 // -------------------------------------------------------------------------------- backward
@@ -1458,17 +1109,8 @@ __global__ void __launch_bounds__(256) nn1_bwd_kernel(BwdArgs a) {
 }
 
 // ----------------------------------------------------------------------------- host helpers
-struct SweepOut {
-    unsigned long long *rowkey, *colkey;
-    unsigned long long *rowslot, *colslot;      // APX
-    int nord;
-    uint32_t *maxnorm;
-    int grid;                                   // out: CTAs of the sweep grid (the fix-up derives the slot ordinals from it)
-    long long units;                            // out
-};
-
-template <int FORM, int R, bool RAW, bool APX>
-static cudaError_t launch_sweep(const SweepSrc &src, SweepOut &o, int B, int N,
+template <int FORM, int R, bool RAW>
+static cudaError_t launch_sweep(const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey, int B, int N,
                                 int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
     using Smem = typename std::conditional<RAW, SweepSmem<R>, SweepSmemPacked<R>>::type;
     const int QT = kSweepWarps * 32 * R;
@@ -1480,50 +1122,42 @@ static cudaError_t launch_sweep(const SweepSrc &src, SweepOut &o, int B, int N,
     const int dev = current_device();
     if (dev < 0) return cudaErrorInvalidDevice;
     if (occ_cache.v[dev] == 0) {
-        cudaError_t e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW, APX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        cudaError_t e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)sizeof(Smem));
         if (e != cudaSuccess) return e;
         // ask for the shared-memory carve-out explicitly: the register-limited residency (2 CTAs at R = 16) needs
         // 2 x 55 KB, more than the default split provides
-        e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW, APX>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  (int)cudaSharedmemCarveoutMaxShared);
         if (e != cudaSuccess) return e;
         int occ = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, nn1_sweep_kernel<FORM, R, RAW, APX>, kSweepThreads, sizeof(Smem));
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, nn1_sweep_kernel<FORM, R, RAW>, kSweepThreads, sizeof(Smem));
         if (e != cudaSuccess) return e;
         occ_cache.v[dev] = occ < 1 ? 1 : occ;
     }
     long long grid = (long long)sms * occ_cache.v[dev];
     if (grid > units) grid = units;
-    o.grid = (int)grid;
-    o.units = units;
-    if constexpr (APX) {
-        if (apx_nord_bound(units, nq, grid) > o.nord) return cudaErrorInvalidConfiguration;      // the caller sized the slots for this tiling
-    }
-    return launch_kernel(nn1_sweep_kernel<FORM, R, RAW, APX>, dim3((unsigned)grid), dim3(kSweepThreads), sizeof(Smem), st, true,
-                         src, o.rowkey, o.colkey, o.rowslot, o.colslot, o.nord, o.maxnorm, N, Npad, Mpad, mt / kQuad, nqt, nq,
-                         (int)units);
+    return launch_kernel(nn1_sweep_kernel<FORM, R, RAW>, dim3((unsigned)grid), dim3(kSweepThreads), sizeof(Smem), st, true,
+                         src, rowkey, colkey, N, Npad, Mpad, mt / kQuad, nqt, nq, (int)units);
 }
 
-template <int FORM, bool RAW, bool APX>
-static cudaError_t launch_sweep_r(int R, const SweepSrc &src, SweepOut &o, int B,
+template <int FORM, bool RAW>
+static cudaError_t launch_sweep_r(int R, const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey, int B,
                                   int N, int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
     switch (R) {
-    case 16: return launch_sweep<FORM, 16, RAW, APX>(src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    case 8: return launch_sweep<FORM, 8, RAW, APX>(src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    case 4: return launch_sweep<FORM, 4, RAW, APX>(src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    default: return launch_sweep<FORM, 2, RAW, APX>(src, o, B, N, M, Npad, Mpad, mt, sms, st);
+    case 16: return launch_sweep<FORM, 16, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
+    case 8: return launch_sweep<FORM, 8, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
+    case 4: return launch_sweep<FORM, 4, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
+    default: return launch_sweep<FORM, 2, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
     }
 }
 
-// the approximate sweep ranks with ONE instruction sequence whatever the reference's form is (the form only matters to the fix-up)
-template <bool RAW, bool APX>
-static cudaError_t launch_sweep_f(int form, int R, const SweepSrc &src, SweepOut &o,
+template <bool RAW>
+static cudaError_t launch_sweep_f(int form, int R, const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey,
                                   int B, int N, int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
-    if constexpr (APX) return launch_sweep_r<PCD_FORM_SUM_FIRST, RAW, true>(R, src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    if (form == PCD_FORM_ROW_COL) return launch_sweep_r<PCD_FORM_ROW_COL, RAW, false>(R, src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    if (form == PCD_FORM_COL_ROW) return launch_sweep_r<PCD_FORM_COL_ROW, RAW, false>(R, src, o, B, N, M, Npad, Mpad, mt, sms, st);
-    return launch_sweep_r<PCD_FORM_SUM_FIRST, RAW, false>(R, src, o, B, N, M, Npad, Mpad, mt, sms, st);
+    if (form == PCD_FORM_ROW_COL) return launch_sweep_r<PCD_FORM_ROW_COL, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
+    if (form == PCD_FORM_COL_ROW) return launch_sweep_r<PCD_FORM_COL_ROW, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
+    return launch_sweep_r<PCD_FORM_SUM_FIRST, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
 }
 
 template <bool RAW, int NORM>
@@ -1546,15 +1180,15 @@ constexpr size_t kStageMaxBytes = 200 * 1024;
 
 // One CTA per (sample, side, slice); `parts` slices per job are chosen so that the whole grid is resident at once
 // (a second wave of CTAs would wait for the first one to drain: +40 % at BASELINE config 2).
-template <int FORM, int NORM, bool APX>
-static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int max_parts, int sms, size_t smem, cudaStream_t st) {
+template <int FORM, int NORM>
+static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int sms, size_t smem, cudaStream_t st) {
     static PerDeviceInt attr_set = {};
     const int dev = current_device();
     if (dev < 0) return cudaErrorInvalidDevice;
     if (!attr_set.v[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM, APX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStageMaxBytes);
+        cudaError_t e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStageMaxBytes);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM, APX>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  (int)cudaSharedmemCarveoutMaxShared);
         if (e != cudaSuccess) return e;
         attr_set.v[dev] = 1;
@@ -1563,7 +1197,7 @@ static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int max_parts, i
     static PerDeviceInt occ_smem = {}, occ_val = {};
     if (occ_smem.v[dev] != (int)smem || occ_val.v[dev] == 0) {
         int o = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, nn1_fixup_staged_kernel<FORM, NORM, APX>, kFixupThreads, smem);
+        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, nn1_fixup_staged_kernel<FORM, NORM>, kFixupThreads, smem);
         if (e != cudaSuccess) return e;
         occ_val.v[dev] = o < 1 ? 1 : o;
         occ_smem.v[dev] = (int)smem;
@@ -1582,31 +1216,18 @@ static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int max_parts, i
     const int wpc = kFixupThreads / 32;
     if (pr > (urow + wpc - 1) / wpc) pr = (urow + wpc - 1) / wpc;
     if (pc > (ucol + wpc - 1) / wpc) pc = (ucol + wpc - 1) / wpc;
-    (void)max_parts;
     sa.parts_row = pr; sa.parts_col = pc;
-    return launch_kernel(nn1_fixup_staged_kernel<FORM, NORM, APX>, dim3((unsigned)(B * (pr + pc))), dim3(kFixupThreads), smem, st, true, sa);
+    return launch_kernel(nn1_fixup_staged_kernel<FORM, NORM>, dim3((unsigned)(B * (pr + pc))), dim3(kFixupThreads), smem, st, true, sa);
 }
-template <int NORM, bool APX>
-static cudaError_t launch_fixup_staged_n(int form, const StagedArgs &sa, int B, int max_parts, int sms, size_t smem, cudaStream_t st) {
-    if (form == PCD_FORM_ROW_COL) return launch_fixup_staged_fn<PCD_FORM_ROW_COL, NORM, APX>(sa, B, max_parts, sms, smem, st);
-    if (form == PCD_FORM_COL_ROW) return launch_fixup_staged_fn<PCD_FORM_COL_ROW, NORM, APX>(sa, B, max_parts, sms, smem, st);
-    return launch_fixup_staged_fn<PCD_FORM_SUM_FIRST, NORM, APX>(sa, B, max_parts, sms, smem, st);
-}
-template <bool APX>
-static cudaError_t launch_fixup_staged(int form, int norm_kind, const StagedArgs &sa, int B, int max_parts, int sms, size_t smem, cudaStream_t st) {
-    return norm_kind == PCD_NORM_FMA ? launch_fixup_staged_n<PCD_NORM_FMA, APX>(form, sa, B, max_parts, sms, smem, st)
-                                     : launch_fixup_staged_n<PCD_NORM_MULSUM, APX>(form, sa, B, max_parts, sms, smem, st);
-}
-
 template <int NORM>
-static cudaError_t launch_rescan_n(int form, const StagedArgs &sa, int sms, cudaStream_t st) {
-    const dim3 grid((unsigned)(sms * 4)), block(256);
-    if (form == PCD_FORM_ROW_COL) return launch_kernel(nn1_rescan_kernel<PCD_FORM_ROW_COL, NORM>, grid, block, 0, st, true, sa);
-    if (form == PCD_FORM_COL_ROW) return launch_kernel(nn1_rescan_kernel<PCD_FORM_COL_ROW, NORM>, grid, block, 0, st, true, sa);
-    return launch_kernel(nn1_rescan_kernel<PCD_FORM_SUM_FIRST, NORM>, grid, block, 0, st, true, sa);
+static cudaError_t launch_fixup_staged_n(int form, const StagedArgs &sa, int B, int sms, size_t smem, cudaStream_t st) {
+    if (form == PCD_FORM_ROW_COL) return launch_fixup_staged_fn<PCD_FORM_ROW_COL, NORM>(sa, B, sms, smem, st);
+    if (form == PCD_FORM_COL_ROW) return launch_fixup_staged_fn<PCD_FORM_COL_ROW, NORM>(sa, B, sms, smem, st);
+    return launch_fixup_staged_fn<PCD_FORM_SUM_FIRST, NORM>(sa, B, sms, smem, st);
 }
-static cudaError_t launch_rescan(int form, int norm_kind, const StagedArgs &sa, int sms, cudaStream_t st) {
-    return norm_kind == PCD_NORM_FMA ? launch_rescan_n<PCD_NORM_FMA>(form, sa, sms, st) : launch_rescan_n<PCD_NORM_MULSUM>(form, sa, sms, st);
+static cudaError_t launch_fixup_staged(int form, int norm_kind, const StagedArgs &sa, int B, int sms, size_t smem, cudaStream_t st) {
+    return norm_kind == PCD_NORM_FMA ? launch_fixup_staged_n<PCD_NORM_FMA>(form, sa, B, sms, smem, st)
+                                     : launch_fixup_staged_n<PCD_NORM_MULSUM>(form, sa, B, sms, smem, st);
 }
 
 // Tile-shape heuristic.  R rows per lane (register blocking: the per-step overhead -- operand
@@ -1657,8 +1278,9 @@ extern "C" int pcd_debug_set_sweep_trace(void *buf) {
 #endif
 
 extern "C" size_t pcd_nn1_workspace_bytes(int B, int N, int M, int sweep_mode) {
+    (void)sweep_mode;      // kept for ABI compatibility: every mode needs the same workspace
     if (B <= 0 || N <= 0 || M <= 0) return 0;
-    return nn1_layout(B, N, M, sweep_mode, sweep_mode == PCD_SWEEP_APPROX ? num_sms() : 0).total;
+    return nn1_layout(B, N, M).total;
 }
 
 extern "C" int pcd_nn1_query_tiling(int B, int N, int M, int *rows_per_lane, int *col_tile) {
@@ -1686,7 +1308,7 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
         return PCD_ERR_ARG;
     }
     if (B <= 0 || N <= 0 || M <= 0 || form < 0 || form > 2 || norm_kind < 0 || norm_kind > 1 || transform < 0 ||
-        transform > 1 || B > 65535 || sweep_mode < PCD_SWEEP_AUTO || sweep_mode > PCD_SWEEP_APPROX) {
+        transform > 1 || B > 65535 || sweep_mode < 0 || sweep_mode > 2) {
         set_error("pcd_nn1_forward: bad argument B=%d N=%d M=%d form=%d norm=%d transform=%d sweep_mode=%d", B, N, M, form,
                   norm_kind, transform, sweep_mode);
         return PCD_ERR_ARG;
@@ -1702,7 +1324,7 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     }
     const int sms = num_sms();
     if (sms <= 0) return cuda_fail(cudaGetLastError(), "no CUDA device");
-    const Nn1Layout L = nn1_layout(B, N, M, sweep_mode, sms);
+    const Nn1Layout L = nn1_layout(B, N, M);
     if (workspace_bytes < L.total) {
         set_error("pcd_nn1_forward: workspace %zu < required %zu bytes", workspace_bytes, L.total);
         return PCD_ERR_WORKSPACE;
@@ -1729,21 +1351,13 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     SweepSrc src{rows, (long long)r_sb, (long long)r_sc, cols, (long long)c_sb, (long long)c_sc, row_cm, col_cm, norm_kind,
                  rowpp, (const float4 *)colpk};
 
-    // approximate sweep + exact fix-up (opt-in: the sweep is faster, the chain not yet, DESIGN.md 4.1): dense operands whose
-    // clouds the staged fix-up can hold, with the tiling the slot arrays of the workspace were sized for; everything else
-    // ranks with the reference's own instruction sequence
     const int nmax = N > M ? N : M;
     const size_t stage_stride = align_up((size_t)nmax, 32);
     const size_t stage_bytes = stage_stride * 12;
     const bool staged = raw && stage_bytes <= kStageMaxBytes;
-    const bool apx = staged && sweep_mode == PCD_SWEEP_APPROX && L.apx_R == R;
     if (raw) {
-        const int ncnt = B + 3;      // completion counters, queue length, two development counters
-        // EXACT: keys = all-ones; APX: only the norm maxima (the slots have one writer each and need no arming)
-        ulonglong2 *arm_ptr = apx ? (ulonglong2 *)(ws + L.maxnorm) : (ulonglong2 *)rowkey;
-        const size_t npairs = apx ? (L.counters - L.maxnorm) / 16 : (L.counters - L.rowkey) / 16;
         PCD_CUDA_CHECK(launch_kernel(nn1_arm_kernel, dim3((unsigned)(sms * 2)), dim3(256), 0, st, false,
-                                     arm_ptr, npairs, counters, ncnt));
+                                     (ulonglong2 *)rowkey, L.nkeys / 2, counters, B));
     } else {
         const long long total = (long long)B * (L.Npad + L.Mpad);
         const int grid = (int)((total + 255) / 256 < (long long)sms * 8 ? (total + 255) / 256 : (long long)sms * 8);
@@ -1751,18 +1365,11 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
                                      c_sp, c_sc, B, N, M, L.Npad, L.Mpad, R, norm_kind, swap_norms, rowpk, rowpp, colpk, rowkey,
                                      colkey, counters));
     }
-    SweepOut so{rowkey, colkey, (unsigned long long *)(ws + L.rowslot), (unsigned long long *)(ws + L.colslot), L.apx_nord,
-                (uint32_t *)(ws + L.maxnorm), 0, 0};
     // an event between two kernels turns the programmatic edge into a full dependency: timing the sweep
     // alone (bench.py's roofline) costs the overlap, nothing else
     if (sweep_start_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_start_event, st));
-    {
-        cudaError_t e;
-        if (apx) e = launch_sweep_f<true, true>(form, R, src, so, B, N, M, L.Npad, L.Mpad, mt, sms, st);
-        else if (raw) e = launch_sweep_f<true, false>(form, R, src, so, B, N, M, L.Npad, L.Mpad, mt, sms, st);
-        else e = launch_sweep_f<false, false>(form, R, src, so, B, N, M, L.Npad, L.Mpad, mt, sms, st);
-        PCD_CUDA_CHECK(e);
-    }
+    PCD_CUDA_CHECK(raw ? launch_sweep_f<true>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st)
+                       : launch_sweep_f<false>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st));
     if (sweep_stop_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_stop_event, st));
     {
         // persistent grid: every warp of every resident CTA owns a contiguous range of units (32 points of one side)
@@ -1782,12 +1389,8 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
                     (float4 *)zero0, zero0_floats / 4, (float4 *)zero1, zero1_floats / 4};
         if (staged) {
             // one CTA per (sample, side, slice): the re-scanned cloud is staged in shared memory
-            StagedArgs sa{a, 1, 1, (int)stage_stride, so.rowslot, so.colslot, so.maxnorm, L.apx_nord, L.apx_nqt,
-                          (M + kQuad - 1) / kQuad, so.grid, so.units, (uint32_t *)(ws + L.queue), counters + B, (int *)(ws + L.pending)};
-            const cudaError_t e = apx ? launch_fixup_staged<true>(form, norm_kind, sa, B, L.partial_slots, sms, stage_bytes, st)
-                                      : launch_fixup_staged<false>(form, norm_kind, sa, B, L.partial_slots, sms, stage_bytes, st);
-            PCD_CUDA_CHECK(e);
-            if (apx) PCD_CUDA_CHECK(launch_rescan(form, norm_kind, sa, sms, st));
+            const StagedArgs sa{a, 1, 1, (int)stage_stride};
+            PCD_CUDA_CHECK(launch_fixup_staged(form, norm_kind, sa, B, sms, stage_bytes, st));
         } else {
             const dim3 grid((unsigned)((nwarps + kFixupThreads / 32 - 1) / (kFixupThreads / 32)));
             PCD_CUDA_CHECK(raw ? launch_fixup<true>(form, a, grid, st) : launch_fixup<false>(form, a, grid, st));

@@ -98,21 +98,6 @@ def force_tiling(rows_per_lane=0, col_tile=0):
     _tiling = (int(rows_per_lane), int(col_tile))
 
 
-_keep_workspace = False      # development aid (tools/apx_debug.py): keep the last NN-1 workspace in _last_workspace
-_last_workspace = None
-SWEEP_AUTO, SWEEP_EXACT, SWEEP_APPROX = 0, 1, 2
-_sweep_mode = SWEEP_AUTO
-
-
-def force_sweep_mode(mode=SWEEP_AUTO):
-    """Tests / measurements: SWEEP_EXACT ranks the pairs with the reference's instruction sequence, SWEEP_APPROX with the
-    cheaper provably-close one (the fix-up settles value and index exactly either way: identical results; experimental,
-    slower end to end for now); SWEEP_AUTO = exact (pcd_sweep_mode in include/pcdist.h).  Returns the previous setting."""
-    global _sweep_mode
-    prev, _sweep_mode = _sweep_mode, int(mode)
-    return prev
-
-
 class _NN1(torch.autograd.Function):
     @staticmethod
     def forward(ctx, rows, cols, form, norm, swap_norms, transform, row_scale, col_scale, token):
@@ -130,7 +115,7 @@ class _NN1(torch.autograd.Function):
             col_arg = torch.empty((B, M), dtype=torch.int32, device=dev)
             stats = torch.empty((4, B), dtype=torch.float32, device=dev)
             stats_i = torch.empty((2, B), dtype=torch.int32, device=dev)
-            ws_bytes = lib.pcd_nn1_workspace_bytes(B, N, M, _sweep_mode)
+            ws_bytes = lib.pcd_nn1_workspace_bytes(B, N, M, 0)
             ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
             # gradient buffers of the coming backward: the forward's last kernel clears them on the way, so the
             # backward is ONE launch (atomics into zeroed memory) instead of memset + memset + kernel
@@ -142,13 +127,11 @@ class _NN1(torch.autograd.Function):
                                      stats.data_ptr(), stats_i.data_ptr(),
                                      _ptr(grad_rows), 0 if grad_rows is None else grad_rows.numel(),
                                      _ptr(grad_cols), 0 if grad_cols is None else grad_cols.numel(),
-                                     ws.data_ptr(), ws_bytes, _tiling[0], _tiling[1], _sweep_mode,
+                                     ws.data_ptr(), ws_bytes, _tiling[0], _tiling[1], 0,
                                      None if ev is None else ev[0].cuda_event, None if ev is None else ev[1].cuda_event,
                                      _stream(dev))
             _lib.check(st, "pcd_nn1_forward")
-            if _keep_workspace:
-                globals()["_last_workspace"] = ws
-        _launch_count += 4 if _sweep_mode == SWEEP_APPROX else 3
+        _launch_count += 3
         ctx.save_for_backward(rows, cols, row_arg, col_arg, row_min, col_min, stats_i)
         ctx.cfg = (int(swap_norms), transform, row_scale, col_scale)
         ctx.token = token

@@ -66,7 +66,8 @@ enum pcd_transform { PCD_VALUE_SQUARED = 0, PCD_VALUE_SQRT_CLAMP = 1 };
  * the library reads no environment): the default four-pass pipeline, the chunk-minima bound followed by the
  * warp-per-row select, or the warp-per-row select alone. */
 enum pcd_knn_strategy { PCD_KNN_AUTO = 0, PCD_KNN_BOUND_SELECT = 1, PCD_KNN_SELECT_ONLY = 2 };
-/* pcd_nn1_forward `sweep_mode` (identical results; see pcd_nn1_forward) */
+/* pcd_nn1_forward / pcd_nn1_workspace_bytes `sweep_mode`: kept for ABI compatibility.  Every value runs the same exact
+ * sweep, with the same results, speed and workspace size. */
 enum pcd_sweep_mode { PCD_SWEEP_AUTO = 0, PCD_SWEEP_EXACT = 1, PCD_SWEEP_APPROX = 2 };
 
 int pcd_version(void);
@@ -112,12 +113,9 @@ const char *pcd_last_error(void);
  * rows_per_lane / col_tile: 0 = the built-in tile-shape heuristic; 2, 4, 8, 16 / a power of two in
  * 32..256 force the sweep's register blocking / TMA stage width (tests, tuning sweeps; results
  * are identical for every tiling).
- * sweep_mode (pcd_sweep_mode; results are identical bit for bit in every mode): PCD_SWEEP_EXACT ranks the pairs with the
- * reference's own instruction sequence; PCD_SWEEP_APPROX ranks them with a cheaper sequence that is provably within a
- * window of it and lets the fix-up settle value and index with the reference's arithmetic (dense operands whose clouds fit
- * the fix-up's shared-memory stage; silently EXACT otherwise; pass the same mode to pcd_nn1_workspace_bytes, the slot
- * arrays and the near-tie queue live in the workspace) -- experimental: its sweep is 5 % faster, its fix-up chain slower
- * (DESIGN.md section 4.1); PCD_SWEEP_AUTO = EXACT.
+ * sweep_mode (pcd_sweep_mode): kept for ABI compatibility.  0, 1 and 2 are accepted, and any other value is rejected with
+ * PCD_ERR_ARG.  No accepted value changes the results, the speed or the workspace size: every one runs the exact sweep,
+ * which ranks the pairs with the reference's own instruction sequence.
  * sweep_start_event / sweep_stop_event (optional cudaEvent_t): recorded on `stream` immediately
  * before / after the sweep kernel launch so a caller can time the dominant kernel live with
  * CUDA events (bench.py's roofline); per call, no global state.

@@ -656,12 +656,12 @@ def test_nn1_nan_and_inf_points_do_not_fault(n):
 
 
 @pytest.mark.parametrize("B,N,M,kind", [(3, 1024, 1024, "perturbed"), (2, 4096, 2048, "random"), (2, 512, 1500 // 4 * 4, "duplicates"),
-                                         (1, 2048, 2048, "identical"), (2, 1024, 1024, "nan"), (4, 260, 36, "tiny")])
-def test_nn1_approximate_sweep_is_bit_identical(B, N, M, kind):
-    """pcd_sweep_mode: the approximate sweep (four packed instructions per two pairs, candidate sets, near-tie rescans) and
-    the exact one give the same bits -- minima, indices, per-sample statistics -- for every form, on perturbed clouds (a few
-    per cent of the points take the rescan path), unrelated clouds, clouds full of exact duplicates (every point rescans),
-    NaN / inf coordinates, and against the oracle."""
+                                         (1, 2048, 2048, "identical"), (4, 260, 36, "tiny"), (2, 216, 512, "lattice")])
+def test_nn1_near_ties_and_duplicates_against_oracle(B, N, M, kind):
+    """Minima and lowest-index arg-mins bit-equal to the oracle for every form on the hardest near-tie inputs: perturbed
+    clouds (many close second-best candidates), unrelated clouds, clouds full of exact duplicates (every point has a tie),
+    all-identical clouds, tiny clouds, and a shuffled lattice whose distances are exact ties (every point has several
+    equidistant nearest neighbours, so only the lowest-index rule decides)."""
     rs = np.random.RandomState(B * N + M)
     cols = rs.randn(B, M, 3).astype(np.float32)
     if kind == "perturbed":
@@ -671,31 +671,22 @@ def test_nn1_approximate_sweep_is_bit_identical(B, N, M, kind):
         cols[:, M // 2:] = cols[:, :M - M // 2]                      # every column exists twice
     elif kind == "identical":
         rows = np.tile(cols[:, :1], (1, N, 1)); cols = np.tile(cols[:, :1], (1, M, 1))
+    elif kind == "lattice":
+        # columns on an 8^3 grid of step 1/4, rows at the centres of 6^3 of its cells: every coordinate, norm and distance is
+        # exact in fp32, so each row has 8 equidistant nearest columns and each inner column 8 equidistant nearest rows
+        g = lambda idx: np.stack(np.meshgrid(idx, idx, idx, indexing="ij"), -1).reshape(-1, 3).astype(np.float32) * 0.25
+        grid_c, grid_r = g(np.arange(8) - 3.5), g(np.arange(1, 7) - 3.0)
+        assert grid_c.shape[0] == M and grid_r.shape[0] == N
+        cols = np.stack([grid_c[rs.permutation(M)] for _ in range(B)])
+        rows = np.stack([grid_r[rs.permutation(N)] for _ in range(B)])
     else:
         rows = rs.randn(B, N, 3).astype(np.float32)
-    if kind == "nan":
-        rows[0, 5] = np.nan; cols[0, 7, 1] = np.inf; cols[1] = np.nan
     for form_key in FORMS:
         form, norm, oform, onorm = FORMS[form_key]
-        outs = []
-        for mode in (F.SWEEP_EXACT, F.SWEEP_APPROX):
-            prev = F.force_sweep_mode(mode)
-            try:
-                r = F.nn1(cu(rows), cu(cols), form, norm, cache=False)
-                outs.append([npy(x) for x in (r.row_min, r.row_arg, r.col_min, r.col_arg, r.row_sum, r.col_sum, r.row_max, r.col_max,
-                                              r.row_argmax, r.col_argmax)])
-            finally:
-                F.force_sweep_mode(prev)
-        if kind == "nan":          # non-finite minima may come out as NaN or +inf; the finite ones and all indices must agree
-            fin = [np.isfinite(a) & np.isfinite(b) for a, b in zip(outs[0], outs[1])]
-            assert all(np.array_equal(a[f], b[f]) for a, b, f in zip(outs[0][:4], outs[1][:4], fin[:4]))
-            assert np.array_equal(np.isfinite(outs[0][0]), np.isfinite(outs[1][0])) and np.array_equal(np.isfinite(outs[0][2]), np.isfinite(outs[1][2]))
-            continue
-        for a, b in zip(outs[0], outs[1]):
-            assert np.array_equal(a, b)
+        r = F.nn1(cu(rows), cu(cols), form, norm, cache=False)
         o = oracle_nn1(rows, cols, oform, onorm)
-        assert np.array_equal(outs[1][0], o.row_min) and np.array_equal(outs[1][1], o.row_arg)
-        assert np.array_equal(outs[1][2], o.col_min) and np.array_equal(outs[1][3], o.col_arg)
+        assert np.array_equal(npy(r.row_min), o.row_min) and np.array_equal(npy(r.row_arg), o.row_arg)
+        assert np.array_equal(npy(r.col_min), o.col_min) and np.array_equal(npy(r.col_arg), o.col_arg)
 
 
 def test_nn1_raw_and_packed_paths_agree():
