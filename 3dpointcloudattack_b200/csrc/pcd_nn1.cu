@@ -1057,9 +1057,10 @@ __global__ void __launch_bounds__(256) nn1_bwd_kernel(BwdArgs a) {
             if (OWN && a.grad_rows) {
                 float3 o;
                 if (a.swap_norms) {
-                    // entry (i,j): -2 g c_j ; column-direction entry (i*, j=i): +2 g' r_i
+                    // entry (i,j): -f c_j ; column-direction entry (i*, j=i): +f' r_i, f' the chain factor of column i
                     const float g2 = upstream(a.g_col, a.w_col_all, a.ws2, a.w_col_max, a.ws3, a.col_argmax, b, i, a.M, a.col_scale);
-                    o = make_float3(-f * c.x + 2.f * g2 * r.x, -f * c.y + 2.f * g2 * r.y, -f * c.z + 2.f * g2 * r.z);
+                    const float f2 = chain_factor(a.transform, g2, a.col_min, (size_t)b * a.M + i);
+                    o = make_float3(-f * c.x + f2 * r.x, -f * c.y + f2 * r.y, -f * c.z + f2 * r.z);
                 } else {
                     o = make_float3(f * (r.x - c.x), f * (r.y - c.y), f * (r.z - c.z));
                 }
@@ -1085,9 +1086,10 @@ __global__ void __launch_bounds__(256) nn1_bwd_kernel(BwdArgs a) {
             if (OWN && a.grad_cols) {
                 float3 o;
                 if (a.swap_norms) {
-                    // entry (i*,j): -2 g' r_i* ; row-direction entry (i=j, j*): +2 g c_j
+                    // entry (i*,j): -f' r_i* ; row-direction entry (i=j, j*): +f c_j, f the chain factor of row j
                     const float g1 = upstream(a.g_row, a.w_row_all, a.ws0, a.w_row_max, a.ws1, a.row_argmax, b, j, a.N, a.row_scale);
-                    o = make_float3(-f * r.x + 2.f * g1 * c.x, -f * r.y + 2.f * g1 * c.y, -f * r.z + 2.f * g1 * c.z);
+                    const float f1 = chain_factor(a.transform, g1, a.row_min, (size_t)b * a.N + j);
+                    o = make_float3(-f * r.x + f1 * c.x, -f * r.y + f1 * c.y, -f * r.z + f1 * c.z);
                 } else {
                     o = make_float3(f * (c.x - r.x), f * (c.y - r.y), f * (c.z - r.z));
                 }

@@ -76,9 +76,16 @@ def curvature_loss(adv_pc, ori_pc, adv_kappa, ori_kappa, k=2):
 # fp32 rounding.  Whatever a loss reads off the neighbours (their squared distances included) is recomputed from the
 # gathered points in the reference's direct form, so values carry no expansion-form cancellation error.
 def _neighbours(pc, k):
-    """[b,3,n] -> (idx [b,n,k] int64 of the k nearest other points, nn_pts [b,3,n,k] gathered, differentiable)."""
+    """[b,3,n] -> (idx [b,n,k] int64 of the k nearest other points, nn_pts [b,3,n,k] gathered, differentiable).
+    In the reference's direct form d(i,i) = 0 exactly, so self is always dropped.  In the expansion form a twin less than
+    ~3e-4 away (unit scale) can rank before self, so the entry equal to the point's own index is dropped wherever it is
+    (the last one when self is not among the k + 1)."""
+    b, _, n = pc.size()
     pts, idx = _self_knn(pc, k + 1)
-    idx = idx[:, :, 1:].long()
+    idx = idx.long()
+    is_self = idx == torch.arange(n, device=idx.device).view(1, n, 1)
+    drop = torch.where(is_self.any(2), is_self.int().argmax(2), torch.full_like(idx[:, :, 0], k))
+    idx = idx[torch.arange(k + 1, device=idx.device) != drop.unsqueeze(2)].view(b, n, k)
     nn_pts = knn_gather(pts, idx).permute(0, 3, 1, 2)
     return idx, nn_pts
 

@@ -149,7 +149,8 @@ int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, int64_t r_sc,
  * either may be NULL when that cloud needs no gradient.  grads_prezeroed != 0: the caller
  * guarantees both buffers are zero (pcd_nn1_forward's zero fill) -- one kernel launch, atomics only.
  * swap_norms: gradients of the swapped-norm surrogate exactly as autograd produces them
- * (norm terms land on the *other* index, attack/GeoA3/knn_utils.py:13-15).
+ * (norm terms land on the *other* index, attack/GeoA3/knn_utils.py:13-15).  Under PCD_VALUE_SQRT_CLAMP each
+ * term, those norm terms included, is scaled by g / v of the minimum it belongs to.
  * ---------------------------------------------------------------------------------- */
 int pcd_nn1_backward(const float *rows, int64_t r_sb, int64_t r_sp, int64_t r_sc,
                      const float *cols, int64_t c_sb, int64_t c_sp, int64_t c_sc,

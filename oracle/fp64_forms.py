@@ -20,6 +20,64 @@ def _gather_pm(x_pm, idx):                      # x [B,M,U], idx [B,L,K] -> [B,L
     return x_pm[:, :, None].expand(B, M, K, U).gather(1, idx[:, :, :, None].expand(B, L, K, U))
 
 
+VALUE_SQUARED, VALUE_SQRT_CLAMP = 0, 1          # include/pcdist.h pcd_value_transform
+
+
+def _i64(a):
+    return a.long() if torch.is_tensor(a) else torch.from_numpy(np.asarray(a, np.int64))
+
+
+def _gather_pts(x, idx, taps=None):
+    """x [B,M,3] float64, idx [B,L] -> x[b, idx[b,l]] [B,L,3].  With `taps` (a list) the gathered copy keeps its gradient --
+    the per-pair contributions before autograd scatters them onto x -- and (x, idx, copy) is appended to it."""
+    g = torch.gather(x, 1, idx[:, :, None].expand(-1, -1, x.shape[2]))
+    if taps is not None:
+        g.retain_grad()
+        taps.append((x, idx, g))
+    return g
+
+
+def _pair_d2(rows, cols, i, j, swap, taps):
+    """d2 of the pairs (i[b,l], j[b,l]): sum((r_i - c_j)^2), or with swapped norms |c_i|^2 - 2 r_i.c_j + |r_j|^2
+    (attack/GeoA3/knn_utils.py:13-15, N == M)."""
+    r_i, c_j = _gather_pts(rows, i, taps), _gather_pts(cols, j, taps)
+    if not swap:
+        return ((r_i - c_j) ** 2).sum(-1)
+    c_i, r_j = _gather_pts(cols, i, taps), _gather_pts(rows, j, taps)
+    return (c_i * c_i).sum(-1) - 2.0 * (r_i * c_j).sum(-1) + (r_j * r_j).sum(-1)
+
+
+def _transform64(d2, v32, transform):
+    if transform == VALUE_SQUARED:
+        return d2
+    v = torch.from_numpy(np.asarray(v32, np.float64))
+    pos = v > 0
+    return torch.where(pos, d2 / torch.where(pos, 2.0 * v, torch.ones_like(v)), d2 * 0.0)
+
+
+def nn1_surrogates64(rows, cols, row_arg, col_arg, row_min32, col_min32, swap, transform, taps=None):
+    """Differentiable per-point values (v_row [B,N], v_col [B,M]) of the NN-1 minima at the given arg-mins.
+    rows [B,N,3], cols [B,M,3]: float64 torch tensors (the caller's leaves).  VALUE_SQUARED: v = d2.  VALUE_SQRT_CLAMP:
+    v = d2 / (2 v32), v32 the stored fp32 minimum (0 where v32 == 0) -- linear in d2, with the gradient of sqrt(d2) taken at
+    the value torch's cdist backward divides by; its value is not the minimum.  Every loss over the minima (sums, maxima
+    at a given arg-max, per-point weights) is then a torch expression of these, differentiated by autograd."""
+    B, N, _ = rows.shape
+    M = cols.shape[1]
+    own_r = torch.arange(N).expand(B, N)
+    own_c = torch.arange(M).expand(B, M)
+    v_row = _transform64(_pair_d2(rows, cols, own_r, _i64(row_arg), swap, taps), row_min32, transform)
+    v_col = _transform64(_pair_d2(rows, cols, _i64(col_arg), own_c, swap, taps), col_min32, transform)
+    return v_row, v_col
+
+
+def knn_pairs64(rows, cols, idx, swap, taps=None):
+    """d2 [B,N,K] of the pairs (i, idx[b,i,k]) in float64 (forms as nn1_surrogates64); rows, cols float64 torch tensors
+    (may be the same tensor)."""
+    B, N, K = idx.shape
+    i = torch.arange(N).repeat_interleave(K).expand(B, N * K)
+    return _pair_d2(rows, cols, i, _i64(idx).reshape(B, N * K), swap, taps).reshape(B, N, K)
+
+
 def kappa64(adv_pm, normal_pm, idx_self, nidx=None):
     """attack/GeoA3/loss_utils.py:60-90 in float64 (differentiable torch expression)."""
     idx = torch.from_numpy(np.asarray(idx_self[:, :, 1:], np.int64))

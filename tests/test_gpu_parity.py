@@ -579,11 +579,10 @@ def test_f4_kappa_and_knn_losses_vs_reference():
         a = cu(adv, True)
         v = fn(a)
         (v * cu(gN)).sum().backward()
-        # a neighbour set may differ from the brute-force topk only where two candidates tie to fp32 rounding: compare the
-        # per-point values with the 1e-5 bar on all but a handful of points and the gradient globally
+        # every neighbour set matches the brute-force topk on this fixture (self is dropped by index, not by rank)
         rel = np.abs(npy(v) - g[name]) / (np.abs(g[name]).max() + 1e-30)
-        assert (rel < RTOL).mean() > 0.995, (name, float((rel < RTOL).mean()))
-        assert rel_inf(npy(a.grad), g[name + "_g"]) < 1e-3 or (np.abs(npy(a.grad) - g[name + "_g"]).max(1) < RTOL * np.abs(g[name + "_g"]).max()).mean() > 0.995, name
+        assert (rel < RTOL).all(), (name, float((rel < RTOL).mean()))
+        assert rel_inf(npy(a.grad), g[name + "_g"]) < RTOL, name
 
 
 def test_f4_graph_laplacian_vs_reference():

@@ -273,3 +273,61 @@ def test_f1_clip_epilogues():
     d = g["linf"] - ori
     assert (np.abs(np.sqrt((d ** 2).sum(1)) - 0.03) < 1e-6).sum() > 100 and (g["linf"] == adv).all(1).sum() > 10
     assert (g["project_linf"][1, :, 5:9] == ori[1, :, 5:9]).all() and (g["lp_clip"] == off).all(1).sum() > 10
+
+
+@pytest.mark.parametrize("swap", [False, True])
+@pytest.mark.parametrize("transform", [0, 1])          # VALUE_SQUARED, VALUE_SQRT_CLAMP
+def test_fp64_nn1_and_knn_references_vs_central_differences(swap, transform):
+    """The float64 references of the NN-1 / k-NN backward tests (oracle/fp64_forms.py) against central differences of the
+    losses they stand for, recomputed from scratch at every step (brute-force minima / k smallest, sqrt where asked) on small
+    inputs without ties: the references' gradients are those of the real losses, not of a restated kernel formula."""
+    import torch
+    from oracle import fp64_forms as F64
+    rs = np.random.RandomState(17 + 2 * swap + transform)
+    B, N = 2, 7
+    M = N if swap else 5
+    K = 3
+    cols0 = rs.randn(B, M, 3)
+    # swapped norms: rows near the columns keep the surrogate's minima positive (the (i, i) entry is |r_i - c_i|^2)
+    rows0 = cols0 + 0.2 * rs.randn(B, N, 3) if swap else rs.randn(B, N, 3)
+    g_row, g_col, w_max = rs.randn(B, N), rs.randn(B, M), rs.randn(B)
+    g_knn = rs.randn(B, N, K)
+
+    def mat(rows, cols):                                   # d[b,i,j] in the form the references evaluate
+        if swap:
+            return (cols ** 2).sum(-1)[:, :, None] - 2 * rows @ cols.transpose(0, 2, 1) + (rows ** 2).sum(-1)[:, None, :]
+        return ((rows[:, :, None] - cols[:, None]) ** 2).sum(-1)
+
+    def val(d):
+        return np.sqrt(d) if transform == F64.VALUE_SQRT_CLAMP else d
+
+    def loss(rows, cols):
+        d = mat(rows, cols)
+        vr, vc = val(d.min(2)), val(d.min(1))
+        knn = np.sort(d, 2)[:, :, :K]
+        return (g_row * vr).sum() + (g_col * vc).sum() + (w_max * vr.max(1)).sum() + (g_knn * knn).sum()
+
+    d = mat(rows0, cols0)
+    srt = np.sort(d, 2)
+    assert (np.diff(srt, axis=2)[:, :, :K] > 1e-3).all() and (np.diff(np.sort(d, 1), axis=1)[:, 0] > 1e-3).all()   # no ties
+    assert transform == F64.VALUE_SQUARED or min(d.min(2).min(), d.min(1).min()) > 1e-3      # sqrt away from its kink
+    row_arg, col_arg = d.argmin(2), d.argmin(1)
+    row_min32, col_min32 = val(d.min(2)).astype(np.float32), val(d.min(1)).astype(np.float32)
+    r, c = torch.tensor(rows0, requires_grad=True), torch.tensor(cols0, requires_grad=True)
+    v_row, v_col = F64.nn1_surrogates64(r, c, row_arg, col_arg, row_min32, col_min32, swap, transform)
+    amax = torch.from_numpy(row_min32.argmax(1))
+    d2k = F64.knn_pairs64(r, c, np.argsort(d, 2, kind="stable")[:, :, :K], swap)
+    L = ((torch.from_numpy(g_row) * v_row).sum() + (torch.from_numpy(g_col) * v_col).sum()
+         + (torch.from_numpy(w_max) * v_row.gather(1, amax[:, None])[:, 0]).sum() + (torch.from_numpy(g_knn) * d2k).sum())
+    L.backward()
+    h = 1e-6
+    for leaf, x0 in ((r, rows0), (c, cols0)):
+        fd = np.zeros_like(x0)
+        for e in np.ndindex(x0.shape):
+            xp, xm = x0.copy(), x0.copy()
+            xp[e] += h; xm[e] -= h
+            args_p = (xp, cols0) if leaf is r else (rows0, xp)
+            args_m = (xm, cols0) if leaf is r else (rows0, xm)
+            fd[e] = (loss(*args_p) - loss(*args_m)) / (2 * h)
+        # fp32 minima under sqrt: the chain factor is taken at v32, 2^-24 relative from the exact root
+        assert rel_inf(leaf.grad.numpy(), fd) < (1e-6 if transform == F64.VALUE_SQRT_CLAMP else 1e-8), (swap, transform)
