@@ -14,13 +14,14 @@ through the reference's own Python call surface:
     dgcnn             <- model/dgcnn.py (knn, get_graph_feature)
     curvenet_util     <- model/curvenet_util.py (knn, normal_knn)
     pointnet2_utils   <- model/pointnet2_utils.py (square_distance, query_ball_point)
+    defense           <- attack/SIadv/baselines/defense/drop_points/SOR.py (SORDefense; float64, no install() patch)
 
 `install.install()` patches these into an importable copy of the reference.  The package
 directory name starts with a digit; import it with importlib or through the `pcdist` alias
 module at the repository root.
 """
 from . import _lib, functional  # noqa: F401
-from . import (curvenet_util, cw_loop, dgcnn, dis_utils_torch, dist_utils, distance, geoa3_loop, graph, install,  # noqa: F401
+from . import (curvenet_util, cw_loop, defense, dgcnn, dis_utils_torch, dist_utils, distance, geoa3_loop, graph, install,  # noqa: F401
                knn_utils, loss_utils, pointnet2_utils, set_distance, taof, utility)
 
 __version__ = "0.1.0"

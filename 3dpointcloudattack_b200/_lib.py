@@ -14,6 +14,7 @@ FORM_ROW_COL, FORM_COL_ROW, FORM_SUM_FIRST = 0, 1, 2
 NORM_MULSUM, NORM_FMA = 0, 1
 VALUE_SQUARED, VALUE_SQRT_CLAMP = 0, 1
 KNN_MAX_K, KNN_MAX_C = 64, 128
+SOR_MAX_K = 15
 EDGE_CENTER, EDGE_NEIGHBOR, EDGE_DIFF = 0, 1, 2
 
 _c = ctypes
@@ -47,6 +48,7 @@ SIGNATURES = {
     "pcd_kappa_forward": (_I, _CLOUD + _CLOUD + [_P, _P, _I, _I, _I, _I, _P, _P]),
     "pcd_kappa_backward": (_I, _CLOUD + _CLOUD + [_P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "pcd_graph_laplacian": (_I, _CLOUD + [_P, _I, _I, _I, _P, _P]),
+    "pcd_sor_forward": (_I, _CLOUD + [_I, _I, _I, _c.c_double, _P, _P, _P, _P, _P, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),
 }
 

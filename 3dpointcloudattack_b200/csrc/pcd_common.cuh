@@ -199,6 +199,24 @@ __device__ __forceinline__ void tma_load_1d(void *smem_dst, const void *gmem_src
         : "memory");
 }
 
+// ------------------------------------------------------------------- block-wide reduction
+// Sum over a block of THREADS threads (a multiple of 32) in a fixed order: an xor butterfly per warp, then one over the
+// warp totals.  sh holds THREADS / 32 values.  Every thread gets the total.
+template <typename T, int THREADS>
+__device__ __forceinline__ T block_sum(T v, T *sh) {
+    static_assert(THREADS % 32 == 0 && THREADS <= 1024, "block_sum: whole warps, at most 32");
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    __syncthreads();                   // sh may still be read from the previous call
+    if (lane == 0) sh[warp] = v;
+    __syncthreads();
+    T t = lane < THREADS / 32 ? sh[lane] : T(0);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    return t;
+}
+
 // ------------------------------------------------- programmatic dependent launch (sm_90+)
 // A kernel launched with the programmatic-stream-serialization attribute may become resident
 // while its predecessor in the stream is still running; it must execute pdl_wait() before it

@@ -15,19 +15,6 @@ namespace pcd {
 
 constexpr int kLossThreads = 1024;
 
-__device__ __forceinline__ float block_sum(float v, float *sh) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    __syncthreads();                   // sh may still be read from the previous call
-    if (lane == 0) sh[warp] = v;
-    __syncthreads();
-    float t = lane < kLossThreads / 32 ? sh[lane] : 0.f;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-    return t;                          // every thread holds the total
-}
-
 __global__ void __launch_bounds__(kLossThreads) knn_outlier_fwd_kernel(const float *__restrict__ dists, int N, int K1, int first, float alpha,
                                                                        float *__restrict__ value, float *__restrict__ mask,
                                                                        float *__restrict__ loss, float *__restrict__ thr_out,
@@ -47,13 +34,13 @@ __global__ void __launch_bounds__(kLossThreads) knn_outlier_fwd_kernel(const flo
         val[i] = a;
         s += a;
     }
-    const float mean = block_sum(s, sh) / (float)N;
+    const float mean = block_sum<float, kLossThreads>(s, sh) / (float)N;
     float q = 0.f;
     for (int i = threadIdx.x; i < N; i += kLossThreads) {
         const float c = val[i] - mean;           // written by this very thread
         q += c * c;
     }
-    const float var = block_sum(q, sh) / (float)(N - 1);      // unbiased, torch.std default (NaN for N == 1, as torch)
+    const float var = block_sum<float, kLossThreads>(q, sh) / (float)(N - 1);      // unbiased, torch.std default (NaN for N == 1, as torch)
     const float thr = mean + alpha * sqrtf(var);
     float l = 0.f;
     for (int i = threadIdx.x; i < N; i += kLossThreads) {
@@ -62,7 +49,7 @@ __global__ void __launch_bounds__(kLossThreads) knn_outlier_fwd_kernel(const flo
         msk[i] = m;
         l += v * m;
     }
-    const float tot = block_sum(l, sh);
+    const float tot = block_sum<float, kLossThreads>(l, sh);
     if (threadIdx.x == 0) {
         loss[b] = tot / (float)N;
         if (thr_out) thr_out[b] = thr;

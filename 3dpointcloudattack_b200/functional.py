@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import contextlib
 import ctypes
+import math
 from collections import namedtuple
 
 import torch
@@ -17,7 +18,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
                    VALUE_SQRT_CLAMP, VALUE_SQUARED)
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
-           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss",
+           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -496,6 +497,43 @@ def knn_outlier_loss(pc, k, alpha, form=FORM_COL_ROW, norm=NORM_MULSUM, swap_nor
     if not 1 <= k + 1 <= min(pc.shape[1], _lib.KNN_MAX_K):
         raise ValueError(f"k={k} out of range for N={pc.shape[1]}")
     return _KnnOutlierLoss.apply(pc, k, float(alpha), form, norm, bool(swap_norms))
+
+
+# ------------------------------------------------ statistical outlier removal (SOR defence), float64
+SORResult = namedtuple("SORResult", "value threshold keep kept_idx lengths")
+# value [B,N] f64 mean distance to the k nearest neighbours; threshold [B] f64; keep [B,N] bool;
+# kept_idx [B,N] int64 kept point indices ascending, then -1; lengths [B] int64 number of kept points
+
+
+def sor(pc, k=2, alpha=1.1):
+    """Statistical outlier removal in float64 (pcd_sor_forward in include/pcdist.h; the statistic of
+    attack/SIadv/baselines/defense/drop_points/SOR.py:24-54): pc [B,N,3] fp32 (any strides) -> SORResult.
+    Two kernels, no host synchronisation; pc is detached (the statistic carries no gradient)."""
+    global _launch_count
+    _check_cloud(pc, "pc")
+    k, alpha = int(k), float(alpha)
+    B, N, _ = pc.shape
+    if not 1 <= k <= _lib.SOR_MAX_K or N < k + 1:
+        raise ValueError(f"SOR needs 1 <= k <= {_lib.SOR_MAX_K} and N >= k + 1, got k={k}, N={N}")
+    if not math.isfinite(alpha):
+        raise ValueError(f"alpha must be finite, got {alpha}")
+    if B == 0:
+        raise ValueError("pc holds no sample")
+    lib = _lib.load()
+    dev = pc.device
+    with _on(dev):
+        x = pc.detach()
+        value = torch.empty((B, N), dtype=torch.float64, device=dev)
+        thr = torch.empty((B,), dtype=torch.float64, device=dev)
+        keep = torch.empty((B, N), dtype=torch.uint8, device=dev)
+        kept = torch.empty((B, N), dtype=torch.int32, device=dev)
+        lengths = torch.empty((B,), dtype=torch.int32, device=dev)
+        st = lib.pcd_sor_forward(*_cloud_args(x), B, N, k, alpha, value.data_ptr(), thr.data_ptr(), keep.data_ptr(),
+                                 kept.data_ptr(), lengths.data_ptr(), _stream(dev))
+        _lib.check(st, "pcd_sor_forward")
+        res = SORResult(value, thr, keep.view(torch.bool), kept.long(), lengths.long())
+    _launch_count += 2
+    return res
 
 
 # ------------------------------------------------ local geometry on a k-NN graph (SURVEY 8f row 4)

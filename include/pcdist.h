@@ -338,6 +338,40 @@ int pcd_find_offset(const float *adv, const float *ori, const int32_t *idx, int 
                     void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * Statistical outlier removal (SOR), the standard point-cloud defence, evaluated in float64.
+ * Replaces attack/SIadv/baselines/defense/drop_points/SOR.py:24-54 (outlier_removal): its two
+ * [B,N,N] float64 matrices and topk(k + 1) are never materialised.
+ *
+ * pc [B,N,3] fp32 via element strides (sb, sp, sc): point-major and transposed channel-first
+ * views both work.  For each sample b, in float64 on the exactly converted coordinates:
+ *     xx[i]     = (x_i*x_i + y_i*y_i) + z_i*z_i
+ *     dot(i,j)  = (x_i*x_j + y_i*y_j) + z_i*z_j                 (channels ascending)
+ *     d(i,j)    = (xx[j] + (-2 * dot(i,j))) + xx[i]             (dist = xx + inner + xx^T)
+ *     value[i]  = (s_1 + s_2 + ... + s_k) / k                   s_0 <= s_1 <= ... <= s_k are the k + 1 smallest
+ *                                                               d(i,.) over ALL j, self included; s_0 is dropped;
+ *                                                               the sum runs left to right
+ *     mean      = mean_i value[i],  std = unbiased std_i value[i]   (a fixed order that depends on N only)
+ *     threshold = mean + alpha * std
+ *     keep[i]   = value[i] <= threshold
+ * Only distance values enter, so tie order and which entry is "self" cannot change the result; d(i,i)
+ * is exactly 0.  Results for sample b are bit-identical whatever B is, whatever else is in the batch
+ * and whatever the input layout.
+ * Outputs (all required, contiguous, written in full): value [B,N], threshold [B], keep [B,N] (0/1),
+ * kept_idx [B,N] (the kept indices ascending, then -1), lengths [B] (the number of kept points).
+ * Constraints: B >= 1, 1 <= k <= PCD_SOR_MAX_K, N >= k + 1, alpha finite; anything else returns
+ * PCD_ERR_ARG before any CUDA call.  Non-finite coordinates never fault: a sample that holds one may
+ * end with any lengths[b] in [0, N], and the other samples are unaffected.
+ * Launches: two kernels (the pair sweep, then one CTA per sample for the statistics and the
+ * compaction); no workspace.
+ * ---------------------------------------------------------------------------------- */
+#define PCD_SOR_MAX_K 15
+
+int pcd_sor_forward(const float *pc, int64_t sb, int64_t sp, int64_t sc, int B, int N, int k, double alpha,
+                    double *value /*[B,N]*/, double *threshold /*[B]*/, uint8_t *keep /*[B,N] 0/1*/,
+                    int32_t *kept_idx /*[B,N]: kept indices ascending, then -1*/, int32_t *lengths /*[B]*/,
+                    void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
