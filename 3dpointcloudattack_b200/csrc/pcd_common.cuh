@@ -7,6 +7,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/pcdist.h"
 
 namespace pcd {
@@ -244,8 +246,7 @@ static inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// Per-device cache of a small integer property (SM count, occupancy of one kernel): the queries cost
-// microseconds and the answer differs between the devices of one process.
+// Per-device cache of the SM count: the query costs microseconds and the answer differs between the devices of one process.
 struct PerDeviceInt {
     int v[64];
 };
@@ -268,11 +269,42 @@ static inline int num_sms() {
 // Opt a kernel in to more than 48 KB of dynamic shared memory ONCE per (kernel, device) and size: the attribute call
 // costs microseconds and the entry points are meant to be allocation- and configuration-free in steady state.  The memo is
 // keyed by the kernel's ADDRESS (instantiations of one template share their pointer type, so a per-type static would
-// let one instantiation's opt-in stand for another's).
-cudaError_t opt_in_smem_fn(const void *kernel, size_t bytes);     // pcd_nn1.cu
+// let one instantiation's opt-in stand for another's).  max_carveout also asks for the largest shared-memory carve-out
+// (residency limited by registers may need more shared memory than the default split); the occupancy that ctas_per_sm
+// reports depends on it, so opt in before the first ctas_per_sm of that kernel.
+cudaError_t opt_in_smem_fn(const void *kernel, size_t bytes, bool max_carveout);     // pcd_host.cu
 template <typename K>
-static inline cudaError_t opt_in_smem(K kernel, size_t bytes) {
-    return opt_in_smem_fn(reinterpret_cast<const void *>(kernel), bytes);
+static inline cudaError_t opt_in_smem(K kernel, size_t bytes, bool max_carveout = false) {
+    return opt_in_smem_fn(reinterpret_cast<const void *>(kernel), bytes, max_carveout);
+}
+// Resident CTAs per SM (at least 1) of `kernel` at `threads` threads and `smem` bytes of dynamic shared memory, queried once
+// per (kernel, device, threads, smem).
+cudaError_t ctas_per_sm_fn(const void *kernel, int threads, size_t smem, int *ctas);  // pcd_host.cu
+template <typename K>
+static inline cudaError_t ctas_per_sm(K kernel, int threads, size_t smem, int *ctas) {
+    return ctas_per_sm_fn(reinterpret_cast<const void *>(kernel), threads, smem, ctas);
+}
+
+// Grid of a grid-stride kernel: one CTA per `per_cta` work items, at most `cap` CTAs.
+static inline int capped_grid(long long work, int per_cta, long long cap) {
+    const long long want = (work + per_cta - 1) / per_cta;
+    return (int)(want < cap ? want : cap);
+}
+
+// Runtime value -> template argument: call the generic lambda `fn` with std::integral_constant<int, value>, which converts
+// to a template argument inside it (fn(F) ... kernel<F><<<...>>>).  fn is instantiated for every value, and with it every
+// kernel it names.
+template <int V> using IntC = std::integral_constant<int, V>;
+template <typename Fn>
+static inline decltype(auto) with_form(int form, Fn &&fn) {
+    if (form == PCD_FORM_ROW_COL) return fn(IntC<PCD_FORM_ROW_COL>{});
+    if (form == PCD_FORM_COL_ROW) return fn(IntC<PCD_FORM_COL_ROW>{});
+    return fn(IntC<PCD_FORM_SUM_FIRST>{});
+}
+template <typename Fn>
+static inline decltype(auto) with_norm(int norm_kind, Fn &&fn) {
+    if (norm_kind == PCD_NORM_FMA) return fn(IntC<PCD_NORM_FMA>{});
+    return fn(IntC<PCD_NORM_MULSUM>{});
 }
 
 }  // namespace pcd

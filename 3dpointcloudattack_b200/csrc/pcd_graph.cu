@@ -557,11 +557,9 @@ extern "C" int pcd_edge_feature_forward(const float *x, const int32_t *idx, int 
     if (slices < 1) slices = 1;
     const long long sps = (nslots + slices - 1) / slices;
     const dim3 grid((unsigned)((nslots + sps - 1) / sps), cgroups, B);
-    if (smem > 48 * 1024) {      // per device and function: requested on every call (~1 us), no process-wide memo
-        PCD_CUDA_CHECK(vec ? opt_in_smem(edge_feature_fwd_kernel<4>, smem) : opt_in_smem(edge_feature_fwd_kernel<1>, smem));
-    }
-    if (vec) edge_feature_fwd_kernel<4><<<grid, kEdgeThreads, smem, st>>>(x, idx, C, N, k, nblocks, packed, CG, sps, out);
-    else edge_feature_fwd_kernel<1><<<grid, kEdgeThreads, smem, st>>>(x, idx, C, N, k, nblocks, packed, CG, sps, out);
+    const auto kernel = vec ? edge_feature_fwd_kernel<4> : edge_feature_fwd_kernel<1>;
+    if (smem > 48 * 1024) PCD_CUDA_CHECK(opt_in_smem(kernel, smem));
+    kernel<<<grid, kEdgeThreads, smem, st>>>(x, idx, C, N, k, nblocks, packed, CG, sps, out);
     PCD_CUDA_CHECK(cudaGetLastError());
     return PCD_OK;
 }
@@ -572,6 +570,9 @@ extern "C" size_t pcd_edge_feature_backward_workspace(int B, int N, int k, int n
     return p.ws_bytes;
 }
 
+// A function template, not a lambda: it is instantiated at the end of the file, so the gather kernels' 128-byte aligned
+// dynamic shared array is declared after those of the FPS kernels, whose dynamic shared memory it would otherwise align
+// to 128 bytes as well (64 bytes more per CTA at T = 128).
 template <int TPT>
 static cudaError_t launch_eg_gather(const EgPlan &p, const float *g, const uint16_t *sub, const uint16_t *list, int B, int C,
                                     int N, int k, int nblocks, int packed, float *gx, cudaStream_t st) {
@@ -619,11 +620,9 @@ extern "C" int pcd_edge_feature_backward(const float *g, const int32_t *idx, int
         return PCD_ERR_UNSUPPORTED;
     }
     const bool vec = (k & 3) == 0;
-    if (smem > 48 * 1024) {
-        PCD_CUDA_CHECK(vec ? opt_in_smem(edge_feature_bwd_kernel<4>, smem) : opt_in_smem(edge_feature_bwd_kernel<1>, smem));
-    }
-    if (vec) edge_feature_bwd_kernel<4><<<dim3(C, B), kEdgeThreads, smem, st>>>(g, idx, C, N, k, nblocks, packed, gx);
-    else edge_feature_bwd_kernel<1><<<dim3(C, B), kEdgeThreads, smem, st>>>(g, idx, C, N, k, nblocks, packed, gx);
+    const auto kernel = vec ? edge_feature_bwd_kernel<4> : edge_feature_bwd_kernel<1>;
+    if (smem > 48 * 1024) PCD_CUDA_CHECK(opt_in_smem(kernel, smem));
+    kernel<<<dim3(C, B), kEdgeThreads, smem, st>>>(g, idx, C, N, k, nblocks, packed, gx);
     PCD_CUDA_CHECK(cudaGetLastError());
     return PCD_OK;
 }
@@ -635,30 +634,24 @@ extern "C" int pcd_fps(const float *xyz, int64_t sb, int64_t sp, int64_t sc, int
         return PCD_ERR_ARG;
     }
     cudaStream_t st = (cudaStream_t)stream;
-#define PCD_FPS(T, PPT)                                                                                          \
-    do {                                                                                                         \
-        constexpr size_t sm_bytes = (size_t)(T) * (PPT) * sizeof(float4);                                        \
-        if (sm_bytes > 48 * 1024)                                                                                \
-            PCD_CUDA_CHECK(opt_in_smem(fps_kernel<T, PPT>, sm_bytes));                                                                                                        \
-        fps_kernel<T, PPT><<<B, T, sm_bytes, st>>>(xyz, sb, sp, sc, N, npoint, start, out);                      \
-    } while (0)
-    if (N <= 256) PCD_FPS(128, 2);
-    else if (N <= 512) PCD_FPS(128, 4);
-    else if (N <= 1024) PCD_FPS(256, 4);
-    else if (N <= 2048) PCD_FPS(256, 8);
-    else if (N <= 4096) PCD_FPS(512, 8);
-    else if (N <= 8192) PCD_FPS(1024, 8);
-    else {
-        const size_t smem = (size_t)N * sizeof(float);
-        if (smem > 200 * 1024) {
-            set_error("pcd_fps: N=%d exceeds the shared-memory distance array (N <= 51200)", N);
-            return PCD_ERR_UNSUPPORTED;
-        }
-        if (smem > 48 * 1024)
-            PCD_CUDA_CHECK(opt_in_smem(fps_large_kernel<1024>, smem));
-        fps_large_kernel<1024><<<B, 1024, smem, st>>>(xyz, sb, sp, sc, N, npoint, start, out);
+    // up to 8192 points, each of T threads holds PPT points in registers (the cloud once more in shared memory, T * PPT
+    // float4); beyond, the running distances live in shared memory
+    const auto launch = [&](auto kernel, int threads, size_t smem) -> int {
+        if (smem > 48 * 1024) PCD_CUDA_CHECK(opt_in_smem(kernel, smem));
+        kernel<<<B, threads, smem, st>>>(xyz, sb, sp, sc, N, npoint, start, out);
+        PCD_CUDA_CHECK(cudaGetLastError());
+        return PCD_OK;
+    };
+    if (N <= 256) return launch(fps_kernel<128, 2>, 128, 128 * 2 * sizeof(float4));
+    if (N <= 512) return launch(fps_kernel<128, 4>, 128, 128 * 4 * sizeof(float4));
+    if (N <= 1024) return launch(fps_kernel<256, 4>, 256, 256 * 4 * sizeof(float4));
+    if (N <= 2048) return launch(fps_kernel<256, 8>, 256, 256 * 8 * sizeof(float4));
+    if (N <= 4096) return launch(fps_kernel<512, 8>, 512, 512 * 8 * sizeof(float4));
+    if (N <= 8192) return launch(fps_kernel<1024, 8>, 1024, 1024 * 8 * sizeof(float4));
+    const size_t smem = (size_t)N * sizeof(float);
+    if (smem > 200 * 1024) {
+        set_error("pcd_fps: N=%d exceeds the shared-memory distance array (N <= 51200)", N);
+        return PCD_ERR_UNSUPPORTED;
     }
-#undef PCD_FPS
-    PCD_CUDA_CHECK(cudaGetLastError());
-    return PCD_OK;
+    return launch(fps_large_kernel<1024>, 1024, smem);
 }

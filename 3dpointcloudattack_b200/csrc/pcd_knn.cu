@@ -1166,8 +1166,7 @@ extern "C" int pcd_knn_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     if (sms <= 0) return cuda_fail(cudaGetLastError(), "no CUDA device");
     cudaStream_t st = (cudaStream_t)stream;
     char *ws = (char *)workspace;
-    const long long total = (long long)B * (L.Npad + L.Mpad);
-    const int pgrid = (int)((total + 255) / 256 < (long long)sms * 8 ? (total + 255) / 256 : (long long)sms * 8);
+    const int pgrid = capped_grid((long long)B * (L.Npad + L.Mpad), 256, (long long)sms * 8);
     const dim3 grid(L.Npad / (kKnnWarps * kKnnRQ), B);
     const int NL = (K + 31) / 32;
     if (C == 3) {
@@ -1193,53 +1192,50 @@ extern "C" int pcd_knn_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
             if (csplit < 1) csplit = 1;
             const int cps = (G + (int)csplit - 1) / (int)csplit;
             const dim3 pg(L.Npad / (128 * kPreR), B, (G + cps - 1) / cps);
-            if (form == PCD_FORM_ROW_COL) knn3_chunkmin_kernel<PCD_FORM_ROW_COL><<<pg, 128, 0, st>>>(rowq, (const float4 *)colpk, L.Npad, L.Mpad, M, W, G, cps, cm);
-            else if (form == PCD_FORM_COL_ROW) knn3_chunkmin_kernel<PCD_FORM_COL_ROW><<<pg, 128, 0, st>>>(rowq, (const float4 *)colpk, L.Npad, L.Mpad, M, W, G, cps, cm);
-            else knn3_chunkmin_kernel<PCD_FORM_SUM_FIRST><<<pg, 128, 0, st>>>(rowq, (const float4 *)colpk, L.Npad, L.Mpad, M, W, G, cps, cm);
+            with_form(form, [&](auto F) { knn3_chunkmin_kernel<F><<<pg, 128, 0, st>>>(rowq, (const float4 *)colpk, L.Npad, L.Mpad, M, W, G, cps, cm); });
             PCD_CUDA_CHECK(cudaGetLastError());
             if (G <= 32) knn_threshold_kernel<32><<<dim3(L.Npad / 128, B), 128, 0, st>>>(cm, L.Npad, G, K, thr0);
             else knn_threshold_kernel<64><<<dim3(L.Npad / 128, B), 128, 0, st>>>(cm, L.Npad, G, K, thr0);
             PCD_CUDA_CHECK(cudaGetLastError());
         }
         const float *thr_arg = prepass ? thr0 : nullptr;
-#define PCD_LAUNCH_KNN3(F, OC, OR)                                                                                        \
-    do {                                                                                                          \
-        if (NL == 1) knn3_kernel<F, 1><<<grid, kKnnThreads, 0, st>>>(rowq, colq, thr_arg, N, M, L.Npad, L.Mpad, K, dists, idx, OC, OR); \
-        else knn3_kernel<F, 2><<<grid, kKnnThreads, 0, st>>>(rowq, colq, thr_arg, N, M, L.Npad, L.Mpad, K, dists, idx, OC, OR);    \
-    } while (0)
+        // warp-per-row select: of every row, or of the rows listed in (ovf_cnt, ovf_rows)
+        const auto launch_select = [&](const int *oc, const int *orows) {
+            with_form(form, [&](auto F) {
+                if (NL == 1) knn3_kernel<F, 1><<<grid, kKnnThreads, 0, st>>>(rowq, colq, thr_arg, N, M, L.Npad, L.Mpad, K, dists, idx, oc, orows);
+                else knn3_kernel<F, 2><<<grid, kKnnThreads, 0, st>>>(rowq, colq, thr_arg, N, M, L.Npad, L.Mpad, K, dists, idx, oc, orows);
+            });
+        };
         if (collect) {
             unsigned long long *cand = (unsigned long long *)(ws + L.cand);
             unsigned int *cnt_g = (unsigned int *)(ws + L.cnt);
             const dim3 cg((L.Npad / (128 * kPreR)) * L.nsplit, B);
-            if (form == PCD_FORM_ROW_COL) knn3_collect_kernel<PCD_FORM_ROW_COL><<<cg, 128, 0, st>>>(rowq, (const float4 *)colpk, thr0, B, L.Npad, L.Mpad, M, L.nsplit, L.tps, L.caps, cand, cnt_g);
-            else if (form == PCD_FORM_COL_ROW) knn3_collect_kernel<PCD_FORM_COL_ROW><<<cg, 128, 0, st>>>(rowq, (const float4 *)colpk, thr0, B, L.Npad, L.Mpad, M, L.nsplit, L.tps, L.caps, cand, cnt_g);
-            else knn3_collect_kernel<PCD_FORM_SUM_FIRST><<<cg, 128, 0, st>>>(rowq, (const float4 *)colpk, thr0, B, L.Npad, L.Mpad, M, L.nsplit, L.tps, L.caps, cand, cnt_g);
+            with_form(form, [&](auto F) {
+                knn3_collect_kernel<F><<<cg, 128, 0, st>>>(rowq, (const float4 *)colpk, thr0, B, L.Npad, L.Mpad, M, L.nsplit, L.tps, L.caps, cand, cnt_g);
+            });
             PCD_CUDA_CHECK(cudaGetLastError());
             const dim3 fg((N + 127) / 128, B);
-#define PCD_LAUNCH_FINAL(KT) knn3_final_kernel<KT><<<fg, 128, (size_t)128 * K * sizeof(uint32_t), st>>>(cand, cnt_g, B, N, L.Npad, L.nsplit, L.caps, K, dists, idx, ovf_cnt, ovf_rows)
+            const auto launch_final = [&](auto KT) {
+                knn3_final_kernel<KT><<<fg, 128, (size_t)128 * K * sizeof(uint32_t), st>>>(cand, cnt_g, B, N, L.Npad, L.nsplit, L.caps, K,
+                                                                                            dists, idx, ovf_cnt, ovf_rows);
+            };
             switch ((K + 3) / 4) {                           // KT = K rounded up to a multiple of 4 (48 / 64 beyond 32)
-                case 1: PCD_LAUNCH_FINAL(4); break;
-                case 2: PCD_LAUNCH_FINAL(8); break;
-                case 3: PCD_LAUNCH_FINAL(12); break;
-                case 4: PCD_LAUNCH_FINAL(16); break;
-                case 5: PCD_LAUNCH_FINAL(20); break;
-                case 6: PCD_LAUNCH_FINAL(24); break;
-                case 7: PCD_LAUNCH_FINAL(28); break;
-                case 8: PCD_LAUNCH_FINAL(32); break;
-                default: if (K <= 48) PCD_LAUNCH_FINAL(48); else PCD_LAUNCH_FINAL(64); break;
+                case 1: launch_final(IntC<4>{}); break;
+                case 2: launch_final(IntC<8>{}); break;
+                case 3: launch_final(IntC<12>{}); break;
+                case 4: launch_final(IntC<16>{}); break;
+                case 5: launch_final(IntC<20>{}); break;
+                case 6: launch_final(IntC<24>{}); break;
+                case 7: launch_final(IntC<28>{}); break;
+                case 8: launch_final(IntC<32>{}); break;
+                default: if (K <= 48) launch_final(IntC<48>{}); else launch_final(IntC<64>{}); break;
             }
-#undef PCD_LAUNCH_FINAL
             PCD_CUDA_CHECK(cudaGetLastError());
             // rows whose candidate lists overflowed (none for randomly ordered clouds): warp-per-row select
-            if (form == PCD_FORM_ROW_COL) PCD_LAUNCH_KNN3(PCD_FORM_ROW_COL, ovf_cnt, ovf_rows);
-            else if (form == PCD_FORM_COL_ROW) PCD_LAUNCH_KNN3(PCD_FORM_COL_ROW, ovf_cnt, ovf_rows);
-            else PCD_LAUNCH_KNN3(PCD_FORM_SUM_FIRST, ovf_cnt, ovf_rows);
+            launch_select(ovf_cnt, ovf_rows);
         } else {
-            if (form == PCD_FORM_ROW_COL) PCD_LAUNCH_KNN3(PCD_FORM_ROW_COL, nullptr, nullptr);
-            else if (form == PCD_FORM_COL_ROW) PCD_LAUNCH_KNN3(PCD_FORM_COL_ROW, nullptr, nullptr);
-            else PCD_LAUNCH_KNN3(PCD_FORM_SUM_FIRST, nullptr, nullptr);
+            launch_select(nullptr, nullptr);
         }
-#undef PCD_LAUNCH_KNN3
         PCD_CUDA_CHECK(cudaGetLastError());
     } else {
         float *rowf = (float *)(ws + L.a), *rown = (float *)(ws + L.b);
@@ -1249,22 +1245,9 @@ extern "C" int pcd_knn_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
         PCD_CUDA_CHECK(cudaGetLastError());
         const size_t smem = knnc_smem_bytes(C);
         const dim3 fgrid(L.Npad / kFcCtaRows, B);
-        static PerDeviceInt smem_set[2] = {};                    // largest dynamic shared-memory size opted in so far, per device
-        const int dv = current_device();
-        if (dv < 0) return cuda_fail(cudaErrorInvalidDevice, "cudaGetDevice");
-        if (NL == 1) {
-            if (smem_set[0].v[dv] < (int)smem) {
-                PCD_CUDA_CHECK(cudaFuncSetAttribute(knnc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                smem_set[0].v[dv] = (int)smem;
-            }
-            knnc_kernel<1><<<fgrid, kKnnThreads, smem, st>>>(rowf, rown, colS, N, M, C, L.Npad, L.Mpad, K, form, dists, idx);
-        } else {
-            if (smem_set[1].v[dv] < (int)smem) {
-                PCD_CUDA_CHECK(cudaFuncSetAttribute(knnc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                smem_set[1].v[dv] = (int)smem;
-            }
-            knnc_kernel<2><<<fgrid, kKnnThreads, smem, st>>>(rowf, rown, colS, N, M, C, L.Npad, L.Mpad, K, form, dists, idx);
-        }
+        const auto kernel = NL == 1 ? knnc_kernel<1> : knnc_kernel<2>;
+        PCD_CUDA_CHECK(opt_in_smem(kernel, smem));
+        kernel<<<fgrid, kKnnThreads, smem, st>>>(rowf, rown, colS, N, M, C, L.Npad, L.Mpad, K, form, dists, idx);
         PCD_CUDA_CHECK(cudaGetLastError());
     }
     return PCD_OK;
@@ -1288,9 +1271,7 @@ extern "C" int pcd_knn_backward(const float *rows, int64_t r_sb, int64_t r_sp, i
     if (sms <= 0) return cuda_fail(cudaGetLastError(), "no CUDA device");
     KnnBwdArgs a{rows, r_sb, r_sp, r_sc, cols, c_sb, c_sp, c_sc, B, N, M, K, swap_norms, idx, g_dists,
                  grad_rows, gr_sb, gr_sp, gr_sc, grad_cols, gc_sb, gc_sp, gc_sc};
-    const long long total = (long long)B * (N + M);
-    const long long want = (total + 255) / 256;
-    const int grid = (int)(want < (long long)sms * 16 ? want : (long long)sms * 16);
+    const int grid = capped_grid((long long)B * (N + M), 256, (long long)sms * 16);
     cudaStream_t st = (cudaStream_t)stream;
     knn_bwd_kernel<false><<<grid, 256, 0, st>>>(a);
     PCD_CUDA_CHECK(cudaGetLastError());
@@ -1308,9 +1289,7 @@ extern "C" int pcd_ball_query(const float *xyz, int64_t x_sb, int64_t x_sp, int6
     }
     const int sms = num_sms();
     if (sms <= 0) return cuda_fail(cudaGetLastError(), "no CUDA device");
-    const long long rows = (long long)B * S;
-    const long long want = (rows + 7) / 8;
-    const int grid = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);
+    const int grid = capped_grid((long long)B * S, 8, (long long)sms * 8);     // a warp per query row
     ball_query_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(xyz, x_sb, x_sp, x_sc, new_xyz, q_sb, q_sp, q_sc, B, N, S,
                                                              radius2, nsample, idx);
     PCD_CUDA_CHECK(cudaGetLastError());

@@ -23,51 +23,11 @@
 //
 // Reference semantics served: utils/dis_utils_torch.py:8-28, attack/CW/CW_utils/distance.py:15-70,
 // attack/GeoA3/knn_utils.py:10-55 (K=1); see include/pcdist.h.
-#include <cstdarg>
-#include <cstdio>
-#include <cstdlib>
-#include <cstring>
-
-#include <mutex>
 #include <type_traits>
 
 #include "pcd_common.cuh"
 
 namespace pcd {
-
-// ------------------------------------------------------------------------------ error state
-static thread_local char g_err[512] = "";
-void set_error(const char *fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-}
-int cuda_fail(cudaError_t e, const char *what) {
-    set_error("CUDA error %d (%s) at %s", (int)e, cudaGetErrorString(e), what);
-    return PCD_ERR_CUDA;
-}
-
-// shared-memory opt-in memo, keyed by (kernel address, device); see pcd_common.cuh
-cudaError_t opt_in_smem_fn(const void *kernel, size_t bytes) {
-    struct Entry { const void *fn; int bytes[64]; };
-    static Entry table[128] = {};
-    static std::mutex mu;
-    const int dev = current_device();
-    if (dev < 0) return cudaErrorInvalidDevice;
-    std::lock_guard<std::mutex> lock(mu);
-    Entry *slot = nullptr;
-    for (Entry &e : table) {
-        if (e.fn == kernel || e.fn == nullptr) { slot = &e; break; }
-    }
-    if (slot && slot->fn == kernel && slot->bytes[dev] >= (int)bytes) return cudaSuccess;
-    const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (err == cudaSuccess && slot) {            // a full table only means the attribute is set again next time
-        slot->fn = kernel;
-        slot->bytes[dev] = (int)bytes;
-    }
-    return err;
-}
 
 // ---------------------------------------------------------------------------------- layout
 constexpr int kSweepWarps = 4;
@@ -1111,70 +1071,45 @@ __global__ void __launch_bounds__(256) nn1_bwd_kernel(BwdArgs a) {
 }
 
 // ----------------------------------------------------------------------------- host helpers
-template <int FORM, int R, bool RAW>
-static cudaError_t launch_sweep(const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey, int B, int N,
-                                int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
-    using Smem = typename std::conditional<RAW, SweepSmem<R>, SweepSmemPacked<R>>::type;
-    const int QT = kSweepWarps * 32 * R;
-    const int nqt = (N + QT - 1) / QT;                       // fully inert row tiles are skipped
-    const int nq = (M + kQuad - 1) / kQuad;                  // ... and fully inert column quads
-    const long long units = (long long)B * nqt * nq;
-    if (units >= (1LL << 31)) return cudaErrorInvalidValue;
-    static PerDeviceInt occ_cache = {};                      // per instantiation and device; the query costs microseconds
-    const int dev = current_device();
-    if (dev < 0) return cudaErrorInvalidDevice;
-    if (occ_cache.v[dev] == 0) {
-        cudaError_t e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)sizeof(Smem));
-        if (e != cudaSuccess) return e;
+template <bool RAW>
+static cudaError_t launch_sweep(int form, int R, const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey,
+                                int B, int N, int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
+    const auto launch = [&](auto FORM, auto RR) -> cudaError_t {
+        const auto kernel = nn1_sweep_kernel<FORM, RR, RAW>;
+        const size_t smem = sizeof(typename std::conditional<RAW, SweepSmem<RR>, SweepSmemPacked<RR>>::type);
+        const int QT = kSweepWarps * 32 * RR;
+        const int nqt = (N + QT - 1) / QT;                       // fully inert row tiles are skipped
+        const int nq = (M + kQuad - 1) / kQuad;                  // ... and fully inert column quads
+        const long long units = (long long)B * nqt * nq;
+        if (units >= (1LL << 31)) return cudaErrorInvalidValue;
         // ask for the shared-memory carve-out explicitly: the register-limited residency (2 CTAs at R = 16) needs
         // 2 x 55 KB, more than the default split provides
-        e = cudaFuncSetAttribute(nn1_sweep_kernel<FORM, R, RAW>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 (int)cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return e;
+        cudaError_t e = opt_in_smem(kernel, smem, true);
         int occ = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, nn1_sweep_kernel<FORM, R, RAW>, kSweepThreads, sizeof(Smem));
+        if (e == cudaSuccess) e = ctas_per_sm(kernel, kSweepThreads, smem, &occ);
         if (e != cudaSuccess) return e;
-        occ_cache.v[dev] = occ < 1 ? 1 : occ;
-    }
-    long long grid = (long long)sms * occ_cache.v[dev];
-    if (grid > units) grid = units;
-    return launch_kernel(nn1_sweep_kernel<FORM, R, RAW>, dim3((unsigned)grid), dim3(kSweepThreads), sizeof(Smem), st, true,
-                         src, rowkey, colkey, N, Npad, Mpad, mt / kQuad, nqt, nq, (int)units);
+        long long grid = (long long)sms * occ;
+        if (grid > units) grid = units;
+        return launch_kernel(kernel, dim3((unsigned)grid), dim3(kSweepThreads), smem, st, true,
+                             src, rowkey, colkey, N, Npad, Mpad, mt / kQuad, nqt, nq, (int)units);
+    };
+    return with_form(form, [&](auto FORM) {
+        switch (R) {
+        case 16: return launch(FORM, IntC<16>{});
+        case 8: return launch(FORM, IntC<8>{});
+        case 4: return launch(FORM, IntC<4>{});
+        default: return launch(FORM, IntC<2>{});
+        }
+    });
 }
 
-template <int FORM, bool RAW>
-static cudaError_t launch_sweep_r(int R, const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey, int B,
-                                  int N, int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
-    switch (R) {
-    case 16: return launch_sweep<FORM, 16, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    case 8: return launch_sweep<FORM, 8, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    case 4: return launch_sweep<FORM, 4, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    default: return launch_sweep<FORM, 2, RAW>(src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    }
-}
-
-template <bool RAW>
-static cudaError_t launch_sweep_f(int form, int R, const SweepSrc &src, unsigned long long *rowkey, unsigned long long *colkey,
-                                  int B, int N, int M, int Npad, int Mpad, int mt, int sms, cudaStream_t st) {
-    if (form == PCD_FORM_ROW_COL) return launch_sweep_r<PCD_FORM_ROW_COL, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    if (form == PCD_FORM_COL_ROW) return launch_sweep_r<PCD_FORM_COL_ROW, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-    return launch_sweep_r<PCD_FORM_SUM_FIRST, RAW>(R, src, rowkey, colkey, B, N, M, Npad, Mpad, mt, sms, st);
-}
-
-template <bool RAW, int NORM>
-static cudaError_t launch_fixup_n(int form, const FixupArgs &a, dim3 grid, cudaStream_t st) {
-    if (form == PCD_FORM_ROW_COL) return launch_kernel(nn1_fixup_kernel<PCD_FORM_ROW_COL, RAW, NORM>, grid, dim3(kFixupThreads), 0, st, true, a);
-    if (form == PCD_FORM_COL_ROW) return launch_kernel(nn1_fixup_kernel<PCD_FORM_COL_ROW, RAW, NORM>, grid, dim3(kFixupThreads), 0, st, true, a);
-    return launch_kernel(nn1_fixup_kernel<PCD_FORM_SUM_FIRST, RAW, NORM>, grid, dim3(kFixupThreads), 0, st, true, a);
-}
-template <bool RAW>
-static cudaError_t launch_fixup(int form, const FixupArgs &a, dim3 grid, cudaStream_t st) {
-    // the norm rounding is a template parameter of the streamed variant only (the packed records carry their norms)
-    if constexpr (RAW) {
-        if (a.norm_kind == PCD_NORM_FMA) return launch_fixup_n<true, PCD_NORM_FMA>(form, a, grid, st);
-    }
-    return launch_fixup_n<RAW, PCD_NORM_MULSUM>(form, a, grid, st);
+static cudaError_t launch_fixup(int form, bool raw, const FixupArgs &a, dim3 grid, cudaStream_t st) {
+    const auto kernel = with_form(form, [&](auto FORM) {
+        // the norm rounding is a template parameter of the streamed variant only (the packed records carry their norms)
+        if (!raw) return nn1_fixup_kernel<FORM, false, PCD_NORM_MULSUM>;
+        return with_norm(a.norm_kind, [&](auto NORM) { return nn1_fixup_kernel<FORM, true, NORM>; });
+    });
+    return launch_kernel(kernel, grid, dim3(kFixupThreads), 0, st, true, a);
 }
 
 // Shared-memory staged fix-up (dense clouds of up to kStageMaxBytes): see nn1_fixup_staged_kernel.
@@ -1182,29 +1117,15 @@ constexpr size_t kStageMaxBytes = 200 * 1024;
 
 // One CTA per (sample, side, slice); `parts` slices per job are chosen so that the whole grid is resident at once
 // (a second wave of CTAs would wait for the first one to drain: +40 % at BASELINE config 2).
-template <int FORM, int NORM>
-static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int sms, size_t smem, cudaStream_t st) {
-    static PerDeviceInt attr_set = {};
-    const int dev = current_device();
-    if (dev < 0) return cudaErrorInvalidDevice;
-    if (!attr_set.v[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStageMaxBytes);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(nn1_fixup_staged_kernel<FORM, NORM>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 (int)cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return e;
-        attr_set.v[dev] = 1;
-    }
-    // residency for this staging size: 1 .. 3 CTAs per SM (register bound 3); queried once per (device, size)
-    static PerDeviceInt occ_smem = {}, occ_val = {};
-    if (occ_smem.v[dev] != (int)smem || occ_val.v[dev] == 0) {
-        int o = 0;
-        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, nn1_fixup_staged_kernel<FORM, NORM>, kFixupThreads, smem);
-        if (e != cudaSuccess) return e;
-        occ_val.v[dev] = o < 1 ? 1 : o;
-        occ_smem.v[dev] = (int)smem;
-    }
-    const int per_sm = occ_val.v[dev];
+static cudaError_t launch_fixup_staged(int form, int norm_kind, StagedArgs sa, int B, int sms, size_t smem, cudaStream_t st) {
+    const auto kernel = with_form(form, [&](auto FORM) {
+        return with_norm(norm_kind, [&](auto NORM) { return nn1_fixup_staged_kernel<FORM, NORM>; });
+    });
+    cudaError_t e = opt_in_smem(kernel, kStageMaxBytes, true);
+    // residency for this staging size: 1 .. 3 CTAs per SM (register bound 3)
+    int per_sm = 0;
+    if (e == cudaSuccess) e = ctas_per_sm(kernel, kFixupThreads, smem, &per_sm);
+    if (e != cudaSuccess) return e;
     // slices per sample, split between the sides in proportion to their scan work (32 candidates per row point, R per column point)
     const int urow = (sa.f.N + 31) / 32, ucol = (sa.f.M + 31) / 32;
     int total = sms * per_sm / B;
@@ -1219,17 +1140,7 @@ static cudaError_t launch_fixup_staged_fn(StagedArgs sa, int B, int sms, size_t 
     if (pr > (urow + wpc - 1) / wpc) pr = (urow + wpc - 1) / wpc;
     if (pc > (ucol + wpc - 1) / wpc) pc = (ucol + wpc - 1) / wpc;
     sa.parts_row = pr; sa.parts_col = pc;
-    return launch_kernel(nn1_fixup_staged_kernel<FORM, NORM>, dim3((unsigned)(B * (pr + pc))), dim3(kFixupThreads), smem, st, true, sa);
-}
-template <int NORM>
-static cudaError_t launch_fixup_staged_n(int form, const StagedArgs &sa, int B, int sms, size_t smem, cudaStream_t st) {
-    if (form == PCD_FORM_ROW_COL) return launch_fixup_staged_fn<PCD_FORM_ROW_COL, NORM>(sa, B, sms, smem, st);
-    if (form == PCD_FORM_COL_ROW) return launch_fixup_staged_fn<PCD_FORM_COL_ROW, NORM>(sa, B, sms, smem, st);
-    return launch_fixup_staged_fn<PCD_FORM_SUM_FIRST, NORM>(sa, B, sms, smem, st);
-}
-static cudaError_t launch_fixup_staged(int form, int norm_kind, const StagedArgs &sa, int B, int sms, size_t smem, cudaStream_t st) {
-    return norm_kind == PCD_NORM_FMA ? launch_fixup_staged_n<PCD_NORM_FMA>(form, sa, B, sms, smem, st)
-                                     : launch_fixup_staged_n<PCD_NORM_MULSUM>(form, sa, B, sms, smem, st);
+    return launch_kernel(kernel, dim3((unsigned)(B * (pr + pc))), dim3(kFixupThreads), smem, st, true, sa);
 }
 
 // Tile-shape heuristic.  R rows per lane (register blocking: the per-step overhead -- operand
@@ -1267,9 +1178,6 @@ static bool dense_layout(const float *p, int64_t sb, int64_t sp, int64_t sc, int
 
 // =================================================================================== C ABI
 using namespace pcd;
-
-extern "C" int pcd_version(void) { return PCD_VERSION; }
-extern "C" const char *pcd_last_error(void) { return g_err; }
 
 #ifdef PCD_SWEEP_TRACE
 extern "C" int pcd_debug_set_sweep_trace(void *buf) {
@@ -1361,8 +1269,7 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
         PCD_CUDA_CHECK(launch_kernel(nn1_arm_kernel, dim3((unsigned)(sms * 2)), dim3(256), 0, st, false,
                                      (ulonglong2 *)rowkey, L.nkeys / 2, counters, B));
     } else {
-        const long long total = (long long)B * (L.Npad + L.Mpad);
-        const int grid = (int)((total + 255) / 256 < (long long)sms * 8 ? (total + 255) / 256 : (long long)sms * 8);
+        const int grid = capped_grid((long long)B * (L.Npad + L.Mpad), 256, (long long)sms * 8);
         PCD_CUDA_CHECK(launch_kernel(nn1_prep_kernel, dim3(grid), dim3(256), 0, st, false, rows, r_sb, r_sp, r_sc, cols, c_sb,
                                      c_sp, c_sc, B, N, M, L.Npad, L.Mpad, R, norm_kind, swap_norms, rowpk, rowpp, colpk, rowkey,
                                      colkey, counters));
@@ -1370,8 +1277,8 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     // an event between two kernels turns the programmatic edge into a full dependency: timing the sweep
     // alone (bench.py's roofline) costs the overlap, nothing else
     if (sweep_start_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_start_event, st));
-    PCD_CUDA_CHECK(raw ? launch_sweep_f<true>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st)
-                       : launch_sweep_f<false>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st));
+    PCD_CUDA_CHECK(raw ? launch_sweep<true>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st)
+                       : launch_sweep<false>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st));
     if (sweep_stop_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_stop_event, st));
     {
         // persistent grid: every warp of every resident CTA owns a contiguous range of units (32 points of one side)
@@ -1395,7 +1302,7 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
             PCD_CUDA_CHECK(launch_fixup_staged(form, norm_kind, sa, B, sms, stage_bytes, st));
         } else {
             const dim3 grid((unsigned)((nwarps + kFixupThreads / 32 - 1) / (kFixupThreads / 32)));
-            PCD_CUDA_CHECK(raw ? launch_fixup<true>(form, a, grid, st) : launch_fixup<false>(form, a, grid, st));
+            PCD_CUDA_CHECK(launch_fixup(form, raw, a, grid, st));
         }
     }
     return PCD_OK;
@@ -1438,9 +1345,7 @@ extern "C" int pcd_nn1_backward(const float *rows, int64_t r_sb, int64_t r_sp, i
               w_strides ? w_strides[0] : 1, w_strides ? w_strides[1] : 1, w_strides ? w_strides[2] : 1,
               w_strides ? w_strides[3] : 1, row_sum_scale, col_sum_scale,
               grad_rows, gr_sb, gr_sp, gr_sc, grad_cols, gc_sb, gc_sp, gc_sc};
-    const long long total = (long long)B * (N + M);
-    const long long want = (total + 255) / 256;
-    const int grid = (int)(want < (long long)sms * 16 ? want : (long long)sms * 16);
+    const int grid = capped_grid((long long)B * (N + M), 256, (long long)sms * 16);
     cudaStream_t st = (cudaStream_t)stream;
     const bool dense_r = !grad_rows || (gr_sc == 1 && gr_sp == 3 && gr_sb == (int64_t)N * 3);
     const bool dense_c = !grad_cols || (gc_sc == 1 && gc_sp == 3 && gc_sb == (int64_t)M * 3);
