@@ -15,6 +15,7 @@ through the reference's own Python call surface:
     curvenet_util     <- model/curvenet_util.py (knn, normal_knn)
     pointnet2_utils   <- model/pointnet2_utils.py (square_distance, query_ball_point)
     defense           <- attack/SIadv/baselines/defense/drop_points/SOR.py (SORDefense; float64, no install() patch)
+    metrics           <- utils/dis_utils_numpy.py (float64 Chamfer / Hausdorff for reporting; no install() patch)
 
 `install.install()` patches these into an importable copy of the reference.  The package
 directory name starts with a digit; import it with importlib or through the `pcdist` alias
@@ -22,6 +23,6 @@ module at the repository root.
 """
 from . import _lib, functional  # noqa: F401
 from . import (curvenet_util, cw_loop, defense, dgcnn, dis_utils_torch, dist_utils, distance, geoa3_loop, graph, install,  # noqa: F401
-               knn_utils, loss_utils, pointnet2_utils, set_distance, taof, utility)
+               knn_utils, loss_utils, metrics, pointnet2_utils, set_distance, taof, utility)
 
 __version__ = "0.1.0"

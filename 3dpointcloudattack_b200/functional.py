@@ -18,7 +18,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
                    VALUE_SQRT_CLAMP, VALUE_SQUARED)
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
-           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult",
+           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "nn_dist64", "NNDist64Result",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -532,6 +532,71 @@ def sor(pc, k=2, alpha=1.1):
                                  kept.data_ptr(), lengths.data_ptr(), _stream(dev))
         _lib.check(st, "pcd_sor_forward")
         res = SORResult(value, thr, keep.view(torch.bool), kept.long(), lengths.long())
+    _launch_count += 2
+    return res
+
+
+# ------------------------------------------------ exact float64 nearest-neighbour distances (Chamfer / Hausdorff metrics)
+NNDist64Result = namedtuple("NNDist64Result", "a_min a_arg b_min b_arg a_mean_sq a_mean a_max_sq a_max a_argmax "
+                                              "b_mean_sq b_mean b_max_sq b_max b_argmax")
+# a_min [B,N] f64 squared distance of each a point to its nearest valid b point, a_arg [B,N] int64 its index (NaN / -1
+# past a's length); b_min / b_arg [B,M] the same from b to a.  Per sample [B], over the valid rows: a_mean_sq = mean of
+# a_min, a_mean = mean of sqrt(a_min), a_max_sq = max of a_min, a_max = sqrt(a_max_sq), a_argmax = its first index; b_*
+# the same for b.
+
+
+def _lengths32(lengths, B, n, name, dev):
+    if lengths is None:
+        return None
+    if not isinstance(lengths, torch.Tensor) or lengths.dtype.is_floating_point or lengths.dtype.is_complex \
+            or lengths.dtype == torch.bool or tuple(lengths.shape) != (B,):
+        raise ValueError(f"{name} must be None or an integer tensor of shape ({B},), got {lengths!r:.80}")
+    lengths = lengths.detach().to(dev)
+    if lengths.dtype != torch.int32:
+        lengths = lengths.clamp(0, n).to(torch.int32)     # clamped first: a cast alone would wrap values past 2^31
+    return lengths.contiguous()
+
+
+def nn_dist64(a, b, a_lengths=None, b_lengths=None, col_split=0):
+    """Exact float64 nearest-neighbour distances between a [B,N,3] and b [B,M,3] fp32 (any strides), both directions,
+    with per-sample means and maxima (pcd_nn_dist64_forward in include/pcdist.h) -> NNDist64Result.
+    a_lengths / b_lengths: None (all points) or an integer tensor [B]; sample i uses a[i, :a_lengths[i]] and
+    b[i, :b_lengths[i]], clamped to [0, N] / [0, M] on the device.  Two kernels, no host synchronisation, no autograd.
+    col_split > 0 forces the number of column ranges per row tile (testing and tuning only; results do not change)."""
+    global _launch_count
+    _check_cloud(a, "a")
+    _check_cloud(b, "b")
+    if a.device != b.device:
+        raise ValueError(f"a is on {a.device} and b on {b.device}")
+    B, N, _ = a.shape
+    M = b.shape[1]
+    if b.shape[0] != B:
+        raise ValueError(f"a and b hold {B} and {b.shape[0]} samples")
+    if B == 0 or N == 0 or M == 0:
+        raise ValueError(f"nn_dist64 needs B, N, M >= 1, got B={B}, N={N}, M={M}")
+    col_split = int(col_split)
+    if col_split < 0:
+        raise ValueError(f"col_split must be >= 0, got {col_split}")
+    lib = _lib.load()
+    dev = a.device
+    with _on(dev):
+        la = _lengths32(a_lengths, B, N, "a_lengths", dev)
+        lb = _lengths32(b_lengths, B, M, "b_lengths", dev)
+        a_min = torch.empty((B, N), dtype=torch.float64, device=dev)
+        a_arg = torch.empty((B, N), dtype=torch.int32, device=dev)
+        b_min = torch.empty((B, M), dtype=torch.float64, device=dev)
+        b_arg = torch.empty((B, M), dtype=torch.int32, device=dev)
+        stats = torch.empty((2, B, 4), dtype=torch.float64, device=dev)
+        argmax = torch.empty((2, B), dtype=torch.int32, device=dev)
+        ws_bytes = lib.pcd_nn_dist64_workspace_bytes(B, N, M, col_split)
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        st = lib.pcd_nn_dist64_forward(*_cloud_args(a.detach()), *_cloud_args(b.detach()), B, N, M, _ptr(la), _ptr(lb),
+                                       col_split, a_min.data_ptr(), a_arg.data_ptr(), b_min.data_ptr(), b_arg.data_ptr(),
+                                       stats.data_ptr(), argmax.data_ptr(), ws.data_ptr(), ws_bytes, _stream(dev))
+        _lib.check(st, "pcd_nn_dist64_forward")
+        argmax = argmax.long()
+        res = NNDist64Result(a_min, a_arg.long(), b_min, b_arg.long(), *stats[0].unbind(1), argmax[0],
+                             *stats[1].unbind(1), argmax[1])
     _launch_count += 2
     return res
 

@@ -372,6 +372,54 @@ int pcd_sor_forward(const float *pc, int64_t sb, int64_t sp, int64_t sc, int B, 
                     void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * Exact float64 nearest-neighbour distances between two clouds, both directions, with the
+ * per-sample Chamfer and Hausdorff reductions, for batches of clouds of unequal valid sizes.
+ * The arithmetic of utils/dis_utils_numpy.py:13-38 (scipy distance_matrix in float64) without
+ * the N x M matrix.
+ *
+ * a [B,N,3] and b [B,M,3] fp32 via element strides; a_len / b_len: int32 [B] on the device, or
+ * NULL for "all N" / "all M".  Each length is clamped to [0, N] / [0, M] on the device (no host
+ * synchronisation); n = a_len[b], m = b_len[b] below.  For each sample, in float64 on the
+ * exactly converted coordinates, with every operation correctly rounded and none contracted:
+ *     dx = b_x[j] - a_x[i]   (likewise dy, dz)
+ *     s(i,j) = ((dx*dx) + (dy*dy)) + (dz*dz)
+ * so sqrt_rn(s) is scipy's cdist(a, b, 'euclidean') / distance_matrix bit for bit.  s is
+ * symmetric: (-d)*(-d) == d*d, so the b-side rows evaluate the same s.
+ *   a_min[b,i] = min_{j<m} s(i,j), a_arg[b,i] = its index          (i < n)
+ *   b_min[b,j] = min_{i<n} s(i,j), b_arg[b,j] = its index          (j < m)
+ * with numpy's min / argmin semantics: the lowest index among equal minima; a NaN entry wins
+ * and arg is the first NaN index.  Rows past their length, and every row when the other side
+ * has length 0, get NaN and -1.  The ranking is on s, not on sqrt(s): where two different s
+ * round to the same square root, an argmin over scipy's Euclidean matrix may pick another
+ * index than a_arg / b_arg.
+ * Per sample and direction (d = 0: the a rows, d = 1: the b rows), over the valid rows only,
+ * numpy's reductions of the per-point minima v (a_min[b,:n] or b_min[b,:m]):
+ *   stats[d,b,0] = mean(v)          stats[d,b,1] = mean(sqrt_rn(v))
+ *   stats[d,b,2] = max(v)           stats[d,b,3] = sqrt_rn(max(v))      argmax[d,b] = argmax(v)
+ * NaN propagates as in numpy (argmax = the first NaN index); no valid row gives NaN and -1.
+ * The sums run in a fixed order that depends only on the number of valid rows, so every
+ * output of a sample is bit-identical whatever B, the rest of the batch, the strides or
+ * col_split; the means are within the recursive-summation bound (n-1)*2^-53*sum|v| (plus the
+ * rounding of the division) of the exact mean.
+ * col_split: 0 picks the number of column ranges per row tile from B, N and M (more when
+ * B * row tiles is small); any value > 0 forces it (testing and tuning only; the results do
+ * not depend on it).
+ * Outputs (all required, contiguous, written in full): a_min [B,N], a_arg [B,N], b_min [B,M],
+ * b_arg [B,M], stats [2,B,4], argmax [2,B].  Workspace: at least
+ * pcd_nn_dist64_workspace_bytes(B, N, M, col_split) bytes, else PCD_ERR_WORKSPACE.
+ * Constraints: B >= 1, N >= 1, M >= 1, col_split >= 0, no NULL pointer (a_len / b_len aside);
+ * anything else returns PCD_ERR_ARG before any CUDA call.  Non-finite coordinates never fault.
+ * Launches: two kernels (the sweep of both directions, then one CTA per sample and direction
+ * that merges the column ranges and reduces); no host synchronisation.
+ * ---------------------------------------------------------------------------------- */
+size_t pcd_nn_dist64_workspace_bytes(int B, int N, int M, int col_split);
+int pcd_nn_dist64_forward(const float *a, int64_t sab, int64_t sap, int64_t sac, const float *b, int64_t sbb,
+                          int64_t sbp, int64_t sbc, int B, int N, int M, const int32_t *a_len, const int32_t *b_len,
+                          int col_split, double *a_min /*[B,N]*/, int32_t *a_arg /*[B,N]*/, double *b_min /*[B,M]*/,
+                          int32_t *b_arg /*[B,M]*/, double *stats /*[2,B,4]*/, int32_t *argmax /*[2,B]*/,
+                          void *workspace, size_t workspace_bytes, void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
