@@ -49,6 +49,8 @@ SIGNATURES = {
     "pcd_kappa_backward": (_I, _CLOUD + _CLOUD + [_P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "pcd_graph_laplacian": (_I, _CLOUD + [_P, _I, _I, _I, _P, _P]),
     "pcd_sor_forward": (_I, _CLOUD + [_I, _I, _I, _c.c_double, _P, _P, _P, _P, _P, _P]),
+    "pcd_sor_workspace_bytes": (_Z, [_I, _I, _I, _I]),
+    "pcd_sor_forward_len": (_I, _CLOUD + [_I, _I, _I, _c.c_double, _P, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "pcd_nn_dist64_workspace_bytes": (_Z, [_I, _I, _I, _I]),
     "pcd_nn_dist64_forward": (_I, _CLOUD + _CLOUD + [_I, _I, _I, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),

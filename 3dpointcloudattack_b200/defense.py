@@ -47,10 +47,11 @@ class SORDefense(nn.Module):
         self.alpha = alpha
         self.npoint = npoint
 
-    def outlier_removal(self, x):
+    def outlier_removal(self, x, lengths=None):
         """x [B,N,3] -> [x[b][keep[b]] for b], differentiable with respect to x (the mask is a constant).
+        lengths: None or an integer tensor [B]; sample b is then x[b, :lengths[b]] (see functional.sor).
         One device-to-host copy: the kept counts."""
-        r = F.sor(x, self.k, self.alpha)
+        r = F.sor(x, self.k, self.alpha, lengths)
         lengths = r.lengths.cpu().tolist()
         return [x[b].index_select(0, r.kept_idx[b, :n]) for b, n in enumerate(lengths)]
 
@@ -64,10 +65,10 @@ class SORDefense(nn.Module):
         return flat[torch.from_numpy(idx + offsets[:, None]).to(flat.device)]
 
     @torch.no_grad()
-    def forward(self, x):
-        """process_data(outlier_removal(x)) without building the list: the draws index the kept-index table,
+    def forward(self, x, lengths=None):
+        """process_data(outlier_removal(x, lengths)) without building the list: the draws index the kept-index table,
         and one gather reads the points."""
-        r = F.sor(x, self.k, self.alpha)
+        r = F.sor(x, self.k, self.alpha, lengths)
         idx = draw_indices(r.lengths.cpu().tolist(), self.npoint)
         pts = torch.gather(r.kept_idx, 1, torch.from_numpy(idx).to(x.device))
         return x[torch.arange(x.shape[0], device=x.device)[:, None], pts]

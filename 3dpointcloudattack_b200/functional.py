@@ -505,34 +505,47 @@ SORResult = namedtuple("SORResult", "value threshold keep kept_idx lengths")
 # kept_idx [B,N] int64 kept point indices ascending, then -1; lengths [B] int64 number of kept points
 
 
-def sor(pc, k=2, alpha=1.1):
-    """Statistical outlier removal in float64 (pcd_sor_forward in include/pcdist.h; the statistic of
+def sor(pc, k=2, alpha=1.1, lengths=None, col_split=0):
+    """Statistical outlier removal in float64 (pcd_sor_forward_len in include/pcdist.h; the statistic of
     attack/SIadv/baselines/defense/drop_points/SOR.py:24-54): pc [B,N,3] fp32 (any strides) -> SORResult.
-    Two kernels, no host synchronisation; pc is detached (the statistic carries no gradient)."""
+    lengths: None (all N points) or an integer tensor [B]; sample i is pc[i, :lengths[i]], clamped to [0, N] on the
+    device.  A sample with fewer than k + 1 points has no statistic: NaN values and threshold, nothing kept.  Rows past
+    a sample's length get value NaN, keep False.  col_split > 0 forces the number of column ranges per row tile
+    (testing and tuning only; results do not change).  Two kernels (three when the columns are split), no host
+    synchronisation; pc is detached (the statistic carries no gradient)."""
     global _launch_count
     _check_cloud(pc, "pc")
     k, alpha = int(k), float(alpha)
     B, N, _ = pc.shape
-    if not 1 <= k <= _lib.SOR_MAX_K or N < k + 1:
+    if not 1 <= k <= _lib.SOR_MAX_K or (lengths is None and N < k + 1):
         raise ValueError(f"SOR needs 1 <= k <= {_lib.SOR_MAX_K} and N >= k + 1, got k={k}, N={N}")
     if not math.isfinite(alpha):
         raise ValueError(f"alpha must be finite, got {alpha}")
     if B == 0:
         raise ValueError("pc holds no sample")
+    if N == 0:
+        raise ValueError("pc holds no point")
+    col_split = int(col_split)
+    if col_split < 0:
+        raise ValueError(f"col_split must be >= 0, got {col_split}")
     lib = _lib.load()
     dev = pc.device
     with _on(dev):
         x = pc.detach()
+        len32 = _lengths32(lengths, B, N, "lengths", dev)
         value = torch.empty((B, N), dtype=torch.float64, device=dev)
         thr = torch.empty((B,), dtype=torch.float64, device=dev)
         keep = torch.empty((B, N), dtype=torch.uint8, device=dev)
         kept = torch.empty((B, N), dtype=torch.int32, device=dev)
-        lengths = torch.empty((B,), dtype=torch.int32, device=dev)
-        st = lib.pcd_sor_forward(*_cloud_args(x), B, N, k, alpha, value.data_ptr(), thr.data_ptr(), keep.data_ptr(),
-                                 kept.data_ptr(), lengths.data_ptr(), _stream(dev))
-        _lib.check(st, "pcd_sor_forward")
-        res = SORResult(value, thr, keep.view(torch.bool), kept.long(), lengths.long())
-    _launch_count += 2
+        kept_n = torch.empty((B,), dtype=torch.int32, device=dev)
+        ws_bytes = lib.pcd_sor_workspace_bytes(B, N, k, col_split)
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+        st = lib.pcd_sor_forward_len(*_cloud_args(x), B, N, k, alpha, _ptr(len32), col_split, value.data_ptr(),
+                                     thr.data_ptr(), keep.data_ptr(), kept.data_ptr(), kept_n.data_ptr(), _ptr(ws),
+                                     ws_bytes, _stream(dev))
+        _lib.check(st, "pcd_sor_forward_len")
+        res = SORResult(value, thr, keep.view(torch.bool), kept.long(), kept_n.long())
+    _launch_count += 3 if ws_bytes else 2       # a workspace means split columns: the merge is one more launch
     return res
 
 

@@ -371,6 +371,36 @@ int pcd_sor_forward(const float *pc, int64_t sb, int64_t sp, int64_t sc, int B, 
                     int32_t *kept_idx /*[B,N]: kept indices ascending, then -1*/, int32_t *lengths /*[B]*/,
                     void *stream);
 
+/* SOR on the first len[b] points of every sample (ragged or padded batches), with the columns of a
+ * sample optionally split over several CTAs (small batches).
+ * len: int32 [B] on the device, or NULL for "all N".  Each length is clamped to [0, N] on the
+ * device (no host synchronisation); n = len[b] below, and sample b is pc[b, :n].  Nothing past n
+ * is read into a result, so NaN or inf padding changes no output.
+ *   n >= k + 1: value[b, :n], threshold[b], keep[b, :n], kept_idx[b, :] and lengths[b] are
+ *     bit-identical to pcd_sor_forward on pc[b:b+1, :n] alone (kept_idx padded with -1 to N),
+ *     whatever the rest of the batch, the layout or col_split: the reductions of the epilogue run
+ *     in an order that depends on n only, and the k + 1 smallest values are one multiset at any
+ *     split.  Rows i >= n get value NaN, keep 0 (and kept_idx holds -1 past lengths[b]).
+ *   n < k + 1 (n = 0 included): no statistic.  value is NaN on every row, threshold NaN, keep all 0,
+ *     kept_idx all -1, lengths[b] = 0 (value <= NaN is false).  Nothing faults.
+ * col_split: 0 picks the number of column ranges per row tile from (B, N, k): more while B * row
+ * tiles is small, never a range below one 64-column tile (so small inputs get one range).  Any
+ * value > 0 forces it (testing and tuning; results do not change).
+ * Workspace: at least pcd_sor_workspace_bytes(B, N, k, col_split) bytes, else PCD_ERR_WORKSPACE.
+ * That size is 0 exactly when the split resolves to one range (workspace may then be NULL).
+ * Constraints: B >= 1, N >= 1 (N may be below k + 1), 1 <= k <= PCD_SOR_MAX_K, alpha finite,
+ * col_split >= 0, no NULL pointer (len aside); anything else returns PCD_ERR_ARG before any CUDA
+ * call.  Non-finite coordinates inside the valid range never fault, as above.
+ * Launches: two kernels (the sweep, then one CTA per sample) with one column range; three with
+ * more (the sweep writes each range's sorted k + 1 smallest values to the workspace, and a
+ * per-row merge over many CTAs forms the values before the epilogue).
+ * ---------------------------------------------------------------------------------- */
+size_t pcd_sor_workspace_bytes(int B, int N, int k, int col_split);
+int pcd_sor_forward_len(const float *pc, int64_t sb, int64_t sp, int64_t sc, int B, int N, int k, double alpha,
+                        const int32_t *len /*[B] device, or NULL*/, int col_split, double *value /*[B,N]*/,
+                        double *threshold /*[B]*/, uint8_t *keep /*[B,N]*/, int32_t *kept_idx /*[B,N]*/,
+                        int32_t *lengths /*[B]*/, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------------------------------------
  * Exact float64 nearest-neighbour distances between two clouds, both directions, with the
  * per-sample Chamfer and Hausdorff reductions, for batches of clouds of unequal valid sizes.
