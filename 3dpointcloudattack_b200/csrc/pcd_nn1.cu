@@ -25,6 +25,8 @@
 // attack/GeoA3/knn_utils.py:10-55 (K=1); see include/pcdist.h.
 #include <type_traits>
 
+#include <cub/block/block_radix_sort.cuh>
+
 #include "pcd_common.cuh"
 
 namespace pcd {
@@ -39,15 +41,21 @@ constexpr int kFixupThreads = 256;
 constexpr int kFixupCtasPerSm = 2;                // 128 registers per thread: twelve 16-byte loads in flight per lane
 constexpr int kFixupMaxWarps = 16384;             // upper bound of the persistent fix-up grid (any device)
 
+constexpr int kPruneMaxPoints = 16384;            // bucketing capacity per cloud (nn1_bucket_kernel sorts in shared memory)
+constexpr int kPruneMinPoints = 4096;             // smaller clouds or batches: the bucketing pass (~30 us at any batch on a
+constexpr int kPruneMinBatch = 16;                // B200) costs more than the pruning saves (DESIGN.md section 4.0)
+
 struct Nn1Layout {
     int Npad, Mpad;
-    size_t rowkey, colkey, counters, partials, rowpk, rowpp, colpk, total;
+    size_t rowkey, colkey, counters, partials, rowpk, rowpp, colpk;
+    size_t queue, brec, bbox, bperm, total;
     size_t nkeys;
     int partial_slots;     // fix-up partials per sample (one per 32-point unit)
+    int bslots;            // pruned path: sorted slots per (sample, side) = 32 * chunks of the larger cloud
 };
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // keys + counters first (all the dense-input path touches), the packed records of the strided
-// path behind them
+// path behind them, then the bucketed clouds of the pruned path
 static Nn1Layout nn1_layout(int B, int N, int M) {
     Nn1Layout L;
     L.Npad = (int)align_up((size_t)N, kRowPadUnit);
@@ -62,6 +70,12 @@ static Nn1Layout nn1_layout(int B, int N, int M) {
     L.rowpk = off; off = align_up(off + (size_t)B * L.Npad * 16, 256);
     L.rowpp = off; off = align_up(off + (size_t)B * L.Npad * 16, 256);   // the same records in sweep (slot) order
     L.colpk = off; off = align_up(off + (size_t)B * L.Mpad * 16 + 64, 256);   // +64: the sweep prefetches one record past a tile
+    L.bslots = (int)align_up((size_t)(N > M ? N : M), 32);
+    const size_t nb = (size_t)B * 2 * L.bslots;                          // [B][side][slot]
+    L.queue = off; off = align_up(off + 4, 256);                         // work-queue cursor of the pruned sweep
+    L.brec = off; off = align_up(off + nb * 16, 256);                    // pair records in Morton order
+    L.bbox = off; off = align_up(off + nb / 32 * 32, 256);               // per chunk: (lo xyz, max norm), (hi xyz, never-prune)
+    L.bperm = off; off = align_up(off + nb * 4, 256);                    // sorted slot -> original index
     L.total = off;
     return L;
 }
@@ -141,6 +155,352 @@ __global__ void nn1_prep_kernel(const float *__restrict__ rows, int64_t r_sb, in
             rec[0] = x; rec[2] = y; rec[4] = z; rec[6] = n;
             colkey[(size_t)b * Mpad + j] = ~0ull;
         }
+    }
+}
+
+// ------------------------------------------------------------------- pruned path: bucketing
+// Dense clouds of kPruneMinPoints to kPruneMaxPoints points in batches of kPruneMinBatch or more (no tiling override) take
+// the pruned chain
+//   nn1_bucket  -> nn1_pruned_sweep -> nn1_fixup (pruned keys)
+// instead of arm -> sweep -> fix-up.  A nearest-neighbour search needs only the few chunk pairs
+// whose boxes are close; see DESIGN.md section 4.1 for the bound and the rounding margin.
+//
+// nn1_bucket: one CTA per (sample, side).  Both clouds of a sample are quantised on ONE grid (the
+// joint box of their finite points, 512 cells per axis), each side is sorted by the 27-bit Morton
+// code of its cell (stable block radix sort, so equal codes keep index order), and the sorted
+// cloud is cut into chunks of 32.  Written per (sample, side):
+//   brec [slot]  pair records {x0,x1,y0,y1},{z0,z1,n0,n1} in sorted order; slots past the cloud
+//                are inert (0, 0, 0, +inf), as in the packed sweep
+//   bperm[slot]  original index of the point in that slot
+//   bbox [chunk] (lo xyz, largest norm), (hi xyz, never-prune flag) over the chunk's points
+// Non-finite points get a code past every finite one, so they share the last chunks, whose
+// never-prune flag makes every comparison against them keep the pair.
+constexpr int kBucketThreads = 1024;
+constexpr int kMortonBits = 9;                    // cells per axis = 2^9
+constexpr uint32_t kNonFiniteCode = 1u << (3 * kMortonBits);
+
+__device__ __forceinline__ uint32_t spread3(uint32_t v) {     // bit k of v -> bit 3k
+    v &= 0x3ffu;
+    v = (v ^ (v << 16)) & 0xff0000ffu;
+    v = (v ^ (v << 8)) & 0x0300f00fu;
+    v = (v ^ (v << 4)) & 0x030c30c3u;
+    v = (v ^ (v << 2)) & 0x09249249u;
+    return v;
+}
+
+struct BucketArgs {
+    const float *rows; long long r_sb, r_sp, r_sc;
+    const float *cols; long long c_sb, c_sp, c_sc;
+    int N, M, norm_kind, bslots;
+    float *brec; float4 *bbox; int *bperm;
+    int *counters; int *queue;
+};
+
+template <int ITEMS>
+__global__ void __launch_bounds__(kBucketThreads, 1) nn1_bucket_kernel(BucketArgs a) {
+    using Sort = cub::BlockRadixSort<uint32_t, kBucketThreads, ITEMS, int>;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    __shared__ float red[6][kBucketThreads / 32];
+    pdl_launch_dependents();     // the pruned sweep may become resident; it waits for our completion
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = blockIdx.x >> 1, side = blockIdx.x & 1;
+    if (tid == 0) {
+        if (side == 0) a.counters[b] = 0;
+        if (blockIdx.x == 0) *a.queue = 0;
+    }
+    const float pinf = __int_as_float(0x7f800000);
+    auto load = [&](int s, int i, float &x, float &y, float &z) {
+        const float *p = s ? a.cols + b * a.c_sb + i * a.c_sp : a.rows + b * a.r_sb + i * a.r_sp;
+        const long long sc = s ? a.c_sc : a.r_sc;
+        x = __ldg(p); y = __ldg(p + sc); z = __ldg(p + 2 * sc);
+    };
+    auto finite3 = [](float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); };
+
+    // the CTA's own points (slots tid*ITEMS + k of the sort) stay in registers from here to their Morton codes
+    const int n = side ? a.M : a.N, n_other = side ? a.N : a.M;
+    float own[ITEMS][3];
+    float lo[3] = {pinf, pinf, pinf}, hi[3] = {-pinf, -pinf, -pinf};
+    auto widen = [&](const float *p) {
+        if (finite3(p[0], p[1], p[2])) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) { lo[c] = fminf(lo[c], p[c]); hi[c] = fmaxf(hi[c], p[c]); }
+        }
+    };
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+        const int i = tid * ITEMS + k;
+        own[k][0] = own[k][1] = own[k][2] = 0.f;
+        if (i < n) load(side, i, own[k][0], own[k][1], own[k][2]);
+    }
+    // joint box of the sample's finite points: both CTAs of the sample compute the same one
+#pragma unroll 4
+    for (int t = tid; t < n_other; t += kBucketThreads) {
+        float p[3];
+        load(side ^ 1, t, p[0], p[1], p[2]);
+        widen(p);
+    }
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k)
+        if (tid * ITEMS + k < n) widen(own[k]);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            lo[c] = fminf(lo[c], __shfl_xor_sync(0xffffffffu, lo[c], o));
+            hi[c] = fmaxf(hi[c], __shfl_xor_sync(0xffffffffu, hi[c], o));
+        }
+        if (lane == 0) { red[c][warp] = lo[c]; red[3 + c][warp] = hi[c]; }
+    }
+    __syncthreads();
+    float cell[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        lo[c] = red[c][lane]; hi[c] = red[3 + c][lane];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            lo[c] = fminf(lo[c], __shfl_xor_sync(0xffffffffu, lo[c], o));
+            hi[c] = fmaxf(hi[c], __shfl_xor_sync(0xffffffffu, hi[c], o));
+        }
+        cell[c] = hi[c] > lo[c] ? (float)(1 << kMortonBits) / (hi[c] - lo[c]) : 0.f;
+    }
+
+    uint32_t key[ITEMS];
+    int val[ITEMS];
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+        const int i = tid * ITEMS + k;
+        val[k] = i;
+        key[k] = kNonFiniteCode;          // non-finite points and the padding past n sort last, in index order
+        if (i < n && finite3(own[k][0], own[k][1], own[k][2])) {
+            uint32_t code = 0;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const float q = fminf(fmaxf((own[k][c] - lo[c]) * cell[c], 0.f), (float)((1 << kMortonBits) - 1));
+                code |= spread3((uint32_t)q) << c;
+            }
+            key[k] = code;
+        }
+    }
+    Sort(*reinterpret_cast<typename Sort::TempStorage *>(smem_raw)).Sort(key, val, 0, 3 * kMortonBits + 1);
+
+    // thread tid now holds the sorted slots tid*ITEMS + k
+    const size_t base = (size_t)(b * 2 + side) * a.bslots;
+    const int nslots = (n + 31) & ~31;
+    float blo[3] = {pinf, pinf, pinf}, bhi[3] = {-pinf, -pinf, -pinf}, bn = -pinf;
+    int bad = 0;
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+        const int s = tid * ITEMS + k;
+        if (s < nslots) {
+            float x = 0.f, y = 0.f, z = 0.f, nn = pinf;
+            if (s < n) {
+                load(side, val[k], x, y, z);
+                nn = sq_norm3(a.norm_kind, x, y, z);
+                a.bperm[base + s] = val[k];
+                if (finite3(x, y, z)) {
+                    blo[0] = fminf(blo[0], x); blo[1] = fminf(blo[1], y); blo[2] = fminf(blo[2], z);
+                    bhi[0] = fmaxf(bhi[0], x); bhi[1] = fmaxf(bhi[1], y); bhi[2] = fmaxf(bhi[2], z);
+                    bn = fmaxf(bn, nn);
+                } else {
+                    bad = 1;
+                }
+            }
+            float *rec = a.brec + (base + (s & ~1)) * 4 + (s & 1);
+            rec[0] = x; rec[2] = y; rec[4] = z; rec[6] = nn;
+        }
+    }
+    // chunk boxes: the 32 / ITEMS consecutive lanes that hold one chunk
+    constexpr int kLanesPerChunk = 32 / ITEMS;
+#pragma unroll
+    for (int o = 1; o < kLanesPerChunk; o <<= 1) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            blo[c] = fminf(blo[c], __shfl_xor_sync(0xffffffffu, blo[c], o));
+            bhi[c] = fmaxf(bhi[c], __shfl_xor_sync(0xffffffffu, bhi[c], o));
+        }
+        bn = fmaxf(bn, __shfl_xor_sync(0xffffffffu, bn, o));
+        bad |= __shfl_xor_sync(0xffffffffu, bad, o);
+    }
+    const int chunk = tid * ITEMS / 32;
+    if (tid % kLanesPerChunk == 0 && chunk * 32 < n) {
+        float4 *bx = a.bbox + 2 * (base / 32 + chunk);
+        bx[0] = make_float4(blo[0], blo[1], blo[2], bn);
+        bx[1] = make_float4(bhi[0], bhi[1], bhi[2], bad ? 1.f : 0.f);
+    }
+}
+
+// ---------------------------------------------------------------- pruned path: the sweep
+// Persistent grid, one warp per work item = (sample, side, chunk A of 32 sorted points), items
+// taken from a queue in (sample, side, chunk) order.  Lane l owns point l of A and takes its exact
+// minimum over the other side:
+//   seed    evaluate the other side's chunks of the same relative Morton rank (+-1); every lane's
+//           running minimum is then a computed pair value, and U = the largest of them over A
+//   filter  evaluate every other chunk C unless  LB(A, C) - E(A, C) > U  (a ballot over the
+//           chunk boxes, 32 at a time); every skipped pair value then exceeds U >= the row's
+//           minimum, so it can neither be the minimum nor tie it.  A NaN anywhere keeps the chunk.
+//   LB      squared gap of the two boxes, scaled down past its own rounding (lower bound)
+//   E       kPruneMarginRel * (largest norm of A + largest norm of C) + kPruneMarginAbs, a bound
+//           on |computed pair value - exact squared distance| for all three forms and both norm
+//           kinds (DESIGN.md section 4.1)
+//   arg-min once per distinct winning chunk of the item's lanes (neighbouring points share a few):
+//           the chunk is re-evaluated and its lanes take the lowest ORIGINAL index with d == minimum.
+//           A lane whose minimum two chunks reached (an exact tie) takes it over every evaluated
+//           chunk in a second pass of the item; skipped chunks cannot tie (see above).
+// Pair values use the sweep's instruction sequence (pair_dist_fixed_x2), so they are the sweep's
+// values bit for bit.  Key per point (at its original index) = (minimum, original arg-min): the
+// fix-up only transforms, stores and reduces.
+constexpr int kPruneThreads = 256;
+constexpr float kPruneLbScale = 1.0f - 0x1p-20f;
+constexpr float kPruneMarginRel = 40.0f * 0x1p-24f;
+constexpr float kPruneMarginAbs = 0x1p-100f;
+
+struct PruneArgs {
+    const float4 *brec, *bbox;
+    const int *bperm;
+    int *queue;
+    unsigned long long *rowkey, *colkey;
+    int B, N, M, Npad, Mpad, bslots;
+};
+
+// one item; SIDE 0 = a chunk of rows against the columns, 1 = a chunk of columns against the rows
+template <int FORM, int SIDE>
+__device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, float4 *sbuf, int *jbuf, int &sb, int lane) {
+    const float pinf = __int_as_float(0x7f800000);
+    const int n_own = SIDE ? a.M : a.N;
+    const int ncs = ((SIDE ? a.M : a.N) + 31) >> 5, nco = ((SIDE ? a.N : a.M) + 31) >> 5;
+    const size_t own = (size_t)(b * 2 + SIDE) * a.bslots, opp = (size_t)(b * 2 + (SIDE ^ 1)) * a.bslots;
+    const int slot = c * 32 + lane;
+    const bool valid = slot < n_own;
+    const float *orec = reinterpret_cast<const float *>(a.brec) + (own + (slot & ~1)) * 4 + (slot & 1);
+    const float m2x = -2.f * __ldg(orec), m2y = -2.f * __ldg(orec + 2), m2z = -2.f * __ldg(orec + 4), pn = __ldg(orec + 6);
+    const float4 *crec = a.brec + opp;
+
+    float best = pinf;
+    uint32_t tag = 0;
+    bool tie = false;
+    auto evaluate = [&](int cc, float4 v) {
+        float4 *s = sbuf + sb * 32;
+        sb ^= 1;
+        s[lane] = v;                  // the buffer was last read two chunks ago (this item or the last), before the previous __syncwarp
+        __syncwarp();
+        float m = pinf;
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+            const float4 A = s[2 * k], Bv = s[2 * k + 1];
+            const f32x2 d = pair_dist_fixed_x2<FORM>(SIDE == 0, m2x, m2y, m2z, pn, pack2(A.x, A.y), pack2(A.z, A.w),
+                                                     pack2(Bv.x, Bv.y), pack2(Bv.z, Bv.w));
+            float lo, hi;
+            unpack2(d, lo, hi);
+            m = min3(m, lo, hi);
+        }
+        if (m < best) { best = m; tag = (uint32_t)cc; tie = false; }
+        else if (m == best && m < pinf) tie = true;
+    };
+    // queue chunk cc (-1: none): its records are requested now, the chunk queued before it is evaluated
+    int pend = -1;
+    float4 pv = make_float4(0.f, 0.f, 0.f, 0.f);
+    auto push = [&](int cc) {
+        const float4 v = cc >= 0 ? __ldg(crec + (size_t)cc * 32 + lane) : make_float4(0.f, 0.f, 0.f, 0.f);
+        if (pend >= 0) evaluate(pend, pv);
+        pend = cc; pv = v;
+    };
+
+    const int cs = (int)((long long)c * nco / ncs);
+    const float4 *obox = a.bbox + 2 * (own / 32 + c), *cbox = a.bbox + 2 * (opp / 32);
+    const float4 alo = __ldg(obox), ahi = __ldg(obox + 1);
+    const bool keep_all = ahi.w != 0.f;
+    auto seeds = [&](auto &&fn) {
+        fn(cs);
+        if (cs > 0) fn(cs - 1);
+        if (cs + 1 < nco) fn(cs + 1);
+    };
+    float U = pinf;
+    auto kept = [&](auto &&fn) {         // every other chunk the bound keeps, in index order
+        for (int base = 0; base < nco; base += 32) {
+            const int cb = base + lane;
+            bool keep = false;
+            if (cb < nco && (cb < cs - 1 || cb > cs + 1)) {
+                const float4 clo = __ldg(cbox + 2 * cb), chi = __ldg(cbox + 2 * cb + 1);
+                const float gx = fmaxf(fmaxf(clo.x - ahi.x, alo.x - chi.x), 0.f);
+                const float gy = fmaxf(fmaxf(clo.y - ahi.y, alo.y - chi.y), 0.f);
+                const float gz = fmaxf(fmaxf(clo.z - ahi.z, alo.z - chi.z), 0.f);
+                const float lb = (gx * gx + gy * gy + gz * gz) * kPruneLbScale;
+                const float e = kPruneMarginRel * (alo.w + clo.w) + kPruneMarginAbs;
+                keep = keep_all || chi.w != 0.f || !(lb - e > U);
+            }
+            for (uint32_t msk = __ballot_sync(0xffffffffu, keep); msk; msk &= msk - 1) fn(base + __ffs(msk) - 1);
+        }
+    };
+    seeds(push);
+    push(-1);
+    U = ordered_to_f32(__reduce_max_sync(0xffffffffu, valid ? f32_to_ordered(best) : 0u));
+    kept(push);
+    push(-1);
+
+    // arg-min: the lowest original index with d == minimum among the candidates of chunk cc, for the lanes that ask
+    int arg = 0x7fffffff;
+    auto scan = [&](int cc, bool want) {
+        const float4 v = __ldg(crec + (size_t)cc * 32 + lane);
+        const int jv = __ldg(a.bperm + opp + (size_t)cc * 32 + lane);    // slots past the cloud are inert: never matched
+        float4 *s = sbuf + sb * 32;
+        int *js = jbuf + sb * 32;
+        sb ^= 1;
+        s[lane] = v; js[lane] = jv;
+        __syncwarp();
+        if (want) {
+#pragma unroll
+            for (int k = 0; k < 16; ++k) {
+                const float4 A = s[2 * k], Bv = s[2 * k + 1];
+                const f32x2 d = pair_dist_fixed_x2<FORM>(SIDE == 0, m2x, m2y, m2z, pn, pack2(A.x, A.y), pack2(A.z, A.w),
+                                                         pack2(Bv.x, Bv.y), pack2(Bv.z, Bv.w));
+                float lo, hi;
+                unpack2(d, lo, hi);
+                if (lo == best) arg = min(arg, js[2 * k]);
+                if (hi == best) arg = min(arg, js[2 * k + 1]);
+            }
+        }
+    };
+    // a lane whose minimum one chunk reached: that chunk, one pass per distinct winning chunk (neighbours share a few)
+    bool pending = valid && best < pinf && !tie;
+    for (uint32_t pm = __ballot_sync(0xffffffffu, pending); pm; pm = __ballot_sync(0xffffffffu, pending)) {
+        const int cc = __shfl_sync(0xffffffffu, (int)tag, __ffs(pm) - 1);
+        scan(cc, pending && tag == (uint32_t)cc);
+        if (tag == (uint32_t)cc) pending = false;
+    }
+    // a lane whose minimum two chunks reached (an exact tie, rare): every chunk the item evaluated, once more
+    const bool tied = valid && best < pinf && tie;
+    if (__any_sync(0xffffffffu, tied)) {
+        auto all = [&](int cc) { scan(cc, tied); };
+        seeds(all);
+        kept(all);
+    }
+
+    if (valid) {
+        const int p = __ldg(a.bperm + own + slot);
+        const uint32_t t = (uint32_t)arg;
+        // the sweep's conventions: a row always publishes its minimum, a column only a finite one
+        if (SIDE == 0) a.rowkey[(size_t)b * a.Npad + p] = make_key(best, t);
+        else a.colkey[(size_t)b * a.Mpad + p] = best < pinf ? make_key(best, t) : ~0ull;
+    }
+}
+
+template <int FORM>
+__global__ void __launch_bounds__(kPruneThreads, 3) nn1_pruned_sweep_kernel(PruneArgs a) {
+    __shared__ __align__(16) float4 stage[kPruneThreads / 32][2 * 32];
+    __shared__ int jstage[kPruneThreads / 32][2 * 32];
+    pdl_launch_dependents();
+    pdl_wait();                   // records, boxes, permutation and the queue cursor come from nn1_bucket
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int ncr = (a.N + 31) >> 5, per_b = ncr + ((a.M + 31) >> 5), items = a.B * per_b;
+    int sb = 0;                   // which of the warp's two chunk buffers is written next
+    for (;;) {
+        int item = 0;
+        if (lane == 0) item = atomicAdd(a.queue, 1);
+        item = __shfl_sync(0xffffffffu, item, 0);
+        if (item >= items) break;
+        const int b = item / per_b, r = item - b * per_b;
+        if (r < ncr) pruned_item<FORM, 0>(a, b, r, stage[warp], jstage[warp], sb, lane);
+        else pruned_item<FORM, 1>(a, b, r - ncr, stage[warp], jstage[warp], sb, lane);
     }
 }
 
@@ -530,7 +890,9 @@ struct FixupArgs {
     float row_scale, col_scale;
     float *stats_f; int32_t *stats_i;
     float4 *zero0; size_t nzero0; float4 *zero1; size_t nzero1;     // optional buffers to clear (float4 counts)
+    int pruned;                   // keys from nn1_pruned_sweep: at the original index, tag = the arg-min itself
 };
+
 
 // Persistent, barrier-free fix-up, ONE LANE PER POINT.  A row point re-evaluates the 32 columns of its
 // winning chunk, a column point the R rows of its winning lane -- with the sweep's exact arithmetic --
@@ -712,7 +1074,8 @@ nn1_fixup_kernel(FixupArgs a) {
         f.live = f.p < (f.is_col ? M : N);
         f.key = 0ull; f.ox = f.oy = f.oz = f.on = 0.f;
         if (f.live) {
-            f.key = f.is_col ? a.colkey[(size_t)f.b * a.Mpad + f.p] : a.rowkey[(size_t)f.b * a.Npad + row_slot(f.p, R)];
+            f.key = f.is_col ? a.colkey[(size_t)f.b * a.Mpad + f.p]
+                             : a.rowkey[(size_t)f.b * a.Npad + (a.pruned ? f.p : row_slot(f.p, R))];
             if (RAW) {
                 const float *s = f.is_col ? a.cols + (size_t)f.b * a.c_sb + (size_t)f.p * a.c_sp
                                           : a.rows + (size_t)f.b * a.r_sb + (size_t)f.p * a.r_sp;
@@ -762,8 +1125,10 @@ nn1_fixup_kernel(FixupArgs a) {
             if (RAW) on = sq_norm3(NORM, ox, oy, oz);
             int arg = 0x7fffffff;
             const bool finite = v < __int_as_float(0x7f800000);       // a non-finite minimum has no arg-min (arg 0)
-            if (!cur.is_col) {
-                if (RAW) { ox *= -2.f; oy *= -2.f; oz *= -2.f; }
+            if (!cur.is_col && RAW) { ox *= -2.f; oy *= -2.f; oz *= -2.f; }
+            if (RAW && a.pruned) {
+                if (finite) arg = (int)tag;
+            } else if (!cur.is_col) {
                 if (finite && tag < (uint32_t)a.nchunks) arg = fixup_scan_cols<FORM, RAW, NORM>(a, b, (int)tag * kColChunk, ox, oy, oz, on, v);
             } else if (finite && (tag >> 5) < (uint32_t)a.nrowgroups) {
                 arg = fixup_scan_rows<FORM, RAW, NORM>(a, b, (int)(tag >> 5) * (32 * R) + (int)(tag & 31u) * R, ox, oy, oz, on, v);
@@ -1103,6 +1468,28 @@ static cudaError_t launch_sweep(int form, int R, const SweepSrc &src, unsigned l
     });
 }
 
+template <int ITEMS>
+static cudaError_t launch_bucket(const BucketArgs &a, int B, cudaStream_t st) {
+    const auto kernel = nn1_bucket_kernel<ITEMS>;
+    const size_t smem = sizeof(typename cub::BlockRadixSort<uint32_t, kBucketThreads, ITEMS, int>::TempStorage);
+    cudaError_t e = opt_in_smem(kernel, smem);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(kernel, dim3((unsigned)(2 * B)), dim3(kBucketThreads), smem, st, false, a);
+}
+
+static cudaError_t launch_pruned_sweep(int form, const PruneArgs &a, int sms, cudaStream_t st) {
+    return with_form(form, [&](auto FORM) {
+        const auto kernel = nn1_pruned_sweep_kernel<FORM>;
+        int occ = 0;
+        const cudaError_t e = ctas_per_sm(kernel, kPruneThreads, 0, &occ);
+        if (e != cudaSuccess) return e;
+        const long long items = (long long)a.B * (((a.N + 31) >> 5) + ((a.M + 31) >> 5));
+        long long grid = (long long)sms * occ, wpc = kPruneThreads / 32;
+        if (grid * wpc > items) grid = (items + wpc - 1) / wpc;
+        return launch_kernel(kernel, dim3((unsigned)grid), dim3(kPruneThreads), 0, st, true, a);
+    });
+}
+
 static cudaError_t launch_fixup(int form, bool raw, const FixupArgs &a, dim3 grid, cudaStream_t st) {
     const auto kernel = with_form(form, [&](auto FORM) {
         // the norm rounding is a template parameter of the streamed variant only (the packed records carry their norms)
@@ -1265,7 +1652,17 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     const size_t stage_stride = align_up((size_t)nmax, 32);
     const size_t stage_bytes = stage_stride * 12;
     const bool staged = raw && stage_bytes <= kStageMaxBytes;
-    if (raw) {
+    // the pruned chain: dense clouds the bucketing sorts in shared memory, large enough that its bucketing pass pays off
+    // (DESIGN.md section 4.0); an explicit tiling keeps the full sweep
+    const bool pruned = raw && nmax <= kPruneMaxPoints && (N < M ? N : M) >= kPruneMinPoints && B >= kPruneMinBatch &&
+                        rows_per_lane == 0 && col_tile == 0;
+    int *bperm = (int *)(ws + L.bperm);
+    if (pruned) {
+        const BucketArgs ba{rows, (long long)r_sb, (long long)r_sp, (long long)r_sc, cols, (long long)c_sb, (long long)c_sp,
+                            (long long)c_sc, N, M, norm_kind, L.bslots, (float *)(ws + L.brec), (float4 *)(ws + L.bbox), bperm,
+                            counters, (int *)(ws + L.queue)};
+        PCD_CUDA_CHECK(nmax <= 4 * kBucketThreads ? launch_bucket<4>(ba, B, st) : launch_bucket<16>(ba, B, st));
+    } else if (raw) {
         PCD_CUDA_CHECK(launch_kernel(nn1_arm_kernel, dim3((unsigned)(sms * 2)), dim3(256), 0, st, false,
                                      (ulonglong2 *)rowkey, L.nkeys / 2, counters, B));
     } else {
@@ -1277,8 +1674,14 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     // an event between two kernels turns the programmatic edge into a full dependency: timing the sweep
     // alone (bench.py's roofline) costs the overlap, nothing else
     if (sweep_start_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_start_event, st));
-    PCD_CUDA_CHECK(raw ? launch_sweep<true>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st)
-                       : launch_sweep<false>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st));
+    if (pruned) {
+        const PruneArgs pa{(const float4 *)(ws + L.brec), (const float4 *)(ws + L.bbox), bperm, (int *)(ws + L.queue),
+                           rowkey, colkey, B, N, M, L.Npad, L.Mpad, L.bslots};
+        PCD_CUDA_CHECK(launch_pruned_sweep(form, pa, sms, st));
+    } else {
+        PCD_CUDA_CHECK(raw ? launch_sweep<true>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st)
+                           : launch_sweep<false>(form, R, src, rowkey, colkey, B, N, M, L.Npad, L.Mpad, mt, sms, st));
+    }
     if (sweep_stop_event) PCD_CUDA_CHECK(cudaEventRecord((cudaEvent_t)sweep_stop_event, st));
     {
         // persistent grid: every warp of every resident CTA owns a contiguous range of units (32 points of one side)
@@ -1295,8 +1698,8 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
                     (float4 *)(ws + L.partials), L.partial_slots, (int)nwarps, (int)(octets / nwarps), (int)(octets % nwarps),
                     (N + 32 * R - 1) / (32 * R), (M + kColChunk - 1) / kColChunk, N, M, L.Npad, L.Mpad, R, transform, B, row_min, row_arg, col_min, col_arg,
                     row_sum_scale, col_sum_scale, stats_f, stats_i,
-                    (float4 *)zero0, zero0_floats / 4, (float4 *)zero1, zero1_floats / 4};
-        if (staged) {
+                    (float4 *)zero0, zero0_floats / 4, (float4 *)zero1, zero1_floats / 4, pruned ? 1 : 0};
+        if (staged && !pruned) {
             // one CTA per (sample, side, slice): the re-scanned cloud is staged in shared memory
             const StagedArgs sa{a, 1, 1, (int)stage_stride};
             PCD_CUDA_CHECK(launch_fixup_staged(form, norm_kind, sa, B, sms, stage_bytes, st));
