@@ -15,6 +15,7 @@ NORM_MULSUM, NORM_FMA = 0, 1
 VALUE_SQUARED, VALUE_SQRT_CLAMP = 0, 1
 KNN_MAX_K, KNN_MAX_C = 64, 128
 SOR_MAX_K = 15
+SAMPLE_MAX_N = 16384
 EDGE_CENTER, EDGE_NEIGHBOR, EDGE_DIFF = 0, 1, 2
 
 _c = ctypes
@@ -53,6 +54,7 @@ SIGNATURES = {
     "pcd_sor_forward_len": (_I, _CLOUD + [_I, _I, _I, _c.c_double, _P, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "pcd_nn_dist64_workspace_bytes": (_Z, [_I, _I, _I, _I]),
     "pcd_nn_dist64_forward": (_I, _CLOUD + _CLOUD + [_I, _I, _I, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "pcd_sample_points": (_I, [_I, _I, _I, _P, _P, _L, _c.c_uint64, _L, _P, _P, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),
 }
 

@@ -18,7 +18,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
                    VALUE_SQRT_CLAMP, VALUE_SQUARED)
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
-           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "nn_dist64", "NNDist64Result",
+           "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "sample_points", "PointSampler", "nn_dist64", "NNDist64Result",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -513,6 +513,12 @@ def sor(pc, k=2, alpha=1.1, lengths=None, col_split=0):
     a sample's length get value NaN, keep False.  col_split > 0 forces the number of column ranges per row tile
     (testing and tuning only; results do not change).  Two kernels (three when the columns are split), no host
     synchronisation; pc is detached (the statistic carries no gradient)."""
+    value, thr, keep, kept, kept_n = _sor32(pc, k, alpha, lengths, col_split)
+    return SORResult(value, thr, keep.view(torch.bool), kept.long(), kept_n.long())
+
+
+def _sor32(pc, k, alpha, lengths, col_split=0):
+    """sor's launches -> (value, threshold, keep uint8, kept_idx int32, lengths int32), the C ABI's types"""
     global _launch_count
     _check_cloud(pc, "pc")
     k, alpha = int(k), float(alpha)
@@ -544,9 +550,82 @@ def sor(pc, k=2, alpha=1.1, lengths=None, col_split=0):
                                      thr.data_ptr(), keep.data_ptr(), kept.data_ptr(), kept_n.data_ptr(), _ptr(ws),
                                      ws_bytes, _stream(dev))
         _lib.check(st, "pcd_sor_forward_len")
-        res = SORResult(value, thr, keep.view(torch.bool), kept.long(), kept_n.long())
     _launch_count += 3 if ws_bytes else 2       # a workspace means split columns: the merge is one more launch
-    return res
+    return value, thr, keep, kept, kept_n
+
+
+def sample_points(n, N, npoint, sampler, table=None):
+    """Uniform draws without replacement, per sample, on the device (pcd_sample_points in include/pcdist.h): the
+    resampling of SORDefense.process_data and the SRS defence, without numpy and without a host synchronisation.
+    n: None (N points in every sample) or an integer tensor [B] of valid counts, clamped to [0, N] on the device;
+    N: the padded size; sampler: a PointSampler (seed, first_sample, device-side draw counter).  -> int64 [B, npoint]:
+      n > npoint  npoint distinct points in random order    (np.random.choice(n, npoint, replace=False))
+      n < npoint  arange(n) npoint // n times, then npoint % n distinct points in random order
+      n == npoint arange(n);  n == 0  -1 everywhere
+    table: None or an integer tensor [B, >= N] (SOR's kept_idx): every drawn value v becomes table[b, v].  B is n's
+    length, or table's when n is None.  One launch; the sampler's counter advances by one in stream order, so the call
+    is graph-capturable and a replayed graph draws afresh.  The draws follow numpy's in distribution, not its bits."""
+    global _launch_count
+    if not isinstance(sampler, PointSampler):
+        raise TypeError(f"sampler must be a PointSampler, got {type(sampler).__name__}")
+    N, npoint = int(N), int(npoint)
+    if n is None and table is None:
+        raise ValueError("sample_points needs n or table to know the batch size")
+    B = int(n.shape[0]) if n is not None else int(table.shape[0])
+    if B < 1 or N < 1 or npoint < 1:
+        raise ValueError(f"sample_points needs B, N, npoint >= 1, got B={B}, N={N}, npoint={npoint}")
+    if N > _lib.SAMPLE_MAX_N:
+        raise ValueError(f"sample_points supports N <= {_lib.SAMPLE_MAX_N}, got N={N}")
+    dev = sampler.state.device
+    if table is not None:
+        if not isinstance(table, torch.Tensor) or table.dim() != 2 or table.shape[0] != B or table.shape[1] < N \
+                or table.dtype.is_floating_point or table.dtype == torch.bool:
+            raise ValueError(f"table must be an integer tensor [{B}, >= {N}], got {table!r:.80}")
+        if table.device != dev:
+            raise ValueError(f"table is on {table.device} and the sampler on {dev}")
+        if table.dtype != torch.int32 or table.stride(1) != 1:
+            table = table.to(torch.int32).contiguous()
+    lib = _lib.load()
+    with _on(dev):
+        len32 = _lengths32(n, B, N, "n", dev)
+        out = torch.empty((B, npoint), dtype=torch.int64, device=dev)
+        st = lib.pcd_sample_points(B, N, npoint, _ptr(len32), _ptr(table), table.stride(0) if table is not None else 0,
+                                   sampler.seed, sampler.first_sample, sampler.state.data_ptr(), out.data_ptr(),
+                                   _stream(dev))
+        _lib.check(st, "pcd_sample_points")
+    _launch_count += 1
+    return out
+
+
+class PointSampler:
+    """Seed and device-side draw counter of sample_points.  Draw c of global sample first_sample + b is a pure function
+    of (seed, first_sample + b, c, n, npoint), so a run sharded over ranks (each with the first_sample of its shard)
+    draws what the unsharded run draws, as sharding.per_sample_noise does for the initial noise.
+    state: int64 [2] on the device; state[0] is the draw counter (each sample_points call adds one, on the stream),
+    state[1] scratch of the kernel (0 between calls)."""
+
+    def __init__(self, seed, first_sample=0, device=None):
+        seed, first_sample = int(seed), int(first_sample)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError(f"seed must be in [0, 2**64), got {seed}")
+        if first_sample < 0:
+            raise ValueError(f"first_sample must be >= 0, got {first_sample}")
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError(f"PointSampler on {device}: the sampler runs on CUDA only (no CPU fallback)")
+        self.seed, self.first_sample = seed, first_sample
+        self.state = torch.zeros(2, dtype=torch.int64, device=device)
+
+    @property
+    def counter(self):
+        """the draw counter: a 0-d view of state[0] on the device"""
+        return self.state[0]
+
+    def reset(self, counter=0):
+        """set the draw counter (stream-ordered; no synchronisation)"""
+        self.state[0].fill_(int(counter))
+        self.state[1].zero_()
+        return self
 
 
 # ------------------------------------------------ exact float64 nearest-neighbour distances (Chamfer / Hausdorff metrics)

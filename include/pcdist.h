@@ -450,6 +450,46 @@ int pcd_nn_dist64_forward(const float *a, int64_t sab, int64_t sap, int64_t sac,
                           void *workspace, size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * Uniform draws of points without replacement, per sample: the resampling of the SOR defence
+ * (SORDefense.process_data's np.random.choice calls) and the simple random sampling (SRS)
+ * defence, as one device-side, graph-capturable sampler.
+ *
+ * For every sample b, n = len[b] clamped to [0, N] on the device (len: int32 [B], or NULL for
+ * "all N").  Draw counter c = counter[0] as it is when the call runs; global sample id
+ * g = first_sample + b (its low 32 bits enter the counter block).  Key of point i < n:
+ *     (w0, w1, w2, w3) = Philox4x32-10(counter = (i, g, c_lo, c_hi), key = (seed_lo, seed_hi))
+ *                        (Random123 / curand round constants and Weyl increments)
+ *     r      = (w0 << 32) | w1
+ *     key[i] = (r & ~0x3FFF) | i                 distinct, totally ordered (unsigned 64-bit)
+ * The points ranked by ascending key form a uniformly random permutation P of 0 .. n-1 (up to
+ * the 2^-50 chance of equal random bits, which the index resolves).  out_idx[b, j], j < npoint:
+ *     n >  npoint  P[j]                            np.random.choice(n, npoint, replace=False)
+ *     n <  npoint  j < (npoint / n) * n: j % n;    the cloud npoint / n times, then
+ *                  then P[j - (npoint / n) * n]    npoint % n of its points, distinct
+ *     n == npoint  j                               the cloud as is (no draw)
+ *     n == 0       -1                              (no host-side error without a synchronisation)
+ * The draws follow np.random.choice in distribution, not its bits.  With a table (int32, row
+ * b at table + b * table_stride, SOR's kept_idx), every value v >= 0 above becomes table[b][v]:
+ * out_idx then indexes the original cloud.  A sample's draws depend only on (seed, g, c, n,
+ * npoint): not on B, its batch position, N or the rest of the batch.
+ * counter: int64 [2] on the device.  counter[0] is the draw counter; the call leaves it one
+ * higher, in stream order (the last CTA to have read it advances it), so a captured graph draws
+ * afresh on every replay.  counter[1] is the CTAs' arrival count: 0 between calls (the call
+ * leaves it 0); calls that share a counter must be stream-ordered.
+ * Constraints: B >= 1, 1 <= N, npoint >= 1, first_sample >= 0, table_stride >= N when a table
+ * is given, counter and out_idx not NULL; anything else returns PCD_ERR_ARG before any CUDA
+ * call.  N > PCD_SAMPLE_MAX_N returns PCD_ERR_UNSUPPORTED.
+ * Launches: one kernel, one CTA per sample (a block radix sort of the keys in shared memory);
+ * no workspace, no host synchronisation.  out_idx is int64 so that it feeds torch.gather as is.
+ * ---------------------------------------------------------------------------------- */
+#define PCD_SAMPLE_MAX_N 16384
+
+int pcd_sample_points(int B, int N, int npoint, const int32_t *len /*[B] device, or NULL*/,
+                      const int32_t *table /*[B, table_stride] device, or NULL*/, int64_t table_stride,
+                      uint64_t seed, int64_t first_sample, int64_t *counter /*[2] device*/,
+                      int64_t *out_idx /*[B, npoint]*/, void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
