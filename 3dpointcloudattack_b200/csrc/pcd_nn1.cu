@@ -166,7 +166,7 @@ __global__ void nn1_prep_kernel(const float *__restrict__ rows, int64_t r_sb, in
 // whose boxes are close; see DESIGN.md section 4.1 for the bound and the rounding margin.
 //
 // nn1_bucket: one CTA per (sample, side).  Both clouds of a sample are quantised on ONE grid (the
-// joint box of their finite points, 512 cells per axis), each side is sorted by the 27-bit Morton
+// joint box of their finite points, 32 cells per axis), each side is sorted by the 15-bit Morton
 // code of its cell (stable block radix sort, so equal codes keep index order), and the sorted
 // cloud is cut into chunks of 32.  Written per (sample, side):
 //   brec [slot]  pair records {x0,x1,y0,y1},{z0,z1,n0,n1} in sorted order; slots past the cloud
@@ -176,7 +176,8 @@ __global__ void nn1_prep_kernel(const float *__restrict__ rows, int64_t r_sb, in
 // Non-finite points get a code past every finite one, so they share the last chunks, whose
 // never-prune flag makes every comparison against them keep the pair.
 constexpr int kBucketThreads = 1024;
-constexpr int kMortonBits = 9;                    // cells per axis = 2^9
+constexpr int kMortonBits = 5;                    // cells per axis = 2^5: finer grids make no better chunks
+                                                  // (DESIGN.md section 4.0) and cost radix-sort passes
 constexpr uint32_t kNonFiniteCode = 1u << (3 * kMortonBits);
 
 __device__ __forceinline__ uint32_t spread3(uint32_t v) {     // bit k of v -> bit 3k
@@ -331,21 +332,27 @@ __global__ void __launch_bounds__(kBucketThreads, 1) nn1_bucket_kernel(BucketArg
 
 // ---------------------------------------------------------------- pruned path: the sweep
 // Persistent grid, one warp per work item = (sample, side, chunk A of 32 sorted points), items
-// taken from a queue in (sample, side, chunk) order.  Lane l owns point l of A and takes its exact
+// taken from a queue in (sample, side, chunk) order.  Lane l owns point p_l of A and takes its exact
 // minimum over the other side:
 //   seed    evaluate the other side's chunks of the same relative Morton rank (+-1); every lane's
-//           running minimum is then a computed pair value, and U = the largest of them over A
-//   filter  evaluate every other chunk C unless  LB(A, C) - E(A, C) > U  (a ballot over the
-//           chunk boxes, 32 at a time); every skipped pair value then exceeds U >= the row's
-//           minimum, so it can neither be the minimum nor tie it.  A NaN anywhere keeps the chunk.
-//   LB      squared gap of the two boxes, scaled down past its own rounding (lower bound)
-//   E       kPruneMarginRel * (largest norm of A + largest norm of C) + kPruneMarginAbs, a bound
-//           on |computed pair value - exact squared distance| for all three forms and both norm
-//           kinds (DESIGN.md section 4.1)
+//           running minimum best_l is then a computed pair value, and U = the largest of them over A
+//   filter  two stages over every other chunk C, in index order:
+//           box     a ballot over the chunk boxes, 32 at a time, keeps C unless  fl(LB(A, C) - E(A, C)) > U
+//           point   for each C the box stage keeps, lane l needs C unless  fl(LB(p_l, C) - E(p_l, C)) > best_l,
+//                   with best_l as it stands when C is queued; the warp evaluates C if any lane needs it
+//           Either way every pair value of a chunk a lane skips exceeds that lane's minimum, so it can
+//           neither be the minimum nor tie it.  A NaN anywhere keeps the chunk.
+//   LB      squared per-axis gap of the two boxes (or of the point and the box), scaled down past its
+//           own rounding (lower bound)
+//   E       kPruneMarginRel * (largest norm of A, or the norm of p_l, + largest norm of C) + kPruneMarginAbs,
+//           a bound on |computed pair value - exact squared distance| for all three forms and both norm
+//           kinds (DESIGN.md section 4.0)
 //   arg-min once per distinct winning chunk of the item's lanes (neighbouring points share a few):
 //           the chunk is re-evaluated and its lanes take the lowest ORIGINAL index with d == minimum.
-//           A lane whose minimum two chunks reached (an exact tie) takes it over every evaluated
-//           chunk in a second pass of the item; skipped chunks cannot tie (see above).
+//           A lane whose minimum two chunks reached (an exact tie) takes it over every chunk it did not
+//           skip, re-derived with the final minima, in a second pass of the item.
+// Candidate records are requested two chunks ahead of their evaluation, the next 32 boxes one ballot
+// ahead, and the next winning chunk's records while the current one is compared.
 // Pair values use the sweep's instruction sequence (pair_dist_fixed_x2), so they are the sweep's
 // values bit for bit.  Key per point (at its original index) = (minimum, original arg-min): the
 // fix-up only transforms, stores and reduces.
@@ -362,9 +369,25 @@ struct PruneArgs {
     int B, N, M, Npad, Mpad, bslots;
 };
 
+// 16-byte global -> shared copy that bypasses the registers (LDGSTS); completion is tracked per commit group
+__device__ __forceinline__ void cp_async16(void *dst, const void *src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async4(void *dst, const void *src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+#ifdef PCD_SWEEP_TRACE
+// development build only (tools/nn1_prune_bench.py --count): items, evaluated chunks, arg-min re-scans, tie passes
+__device__ unsigned long long *g_prune_count = nullptr;
+#endif
+
 // one item; SIDE 0 = a chunk of rows against the columns, 1 = a chunk of columns against the rows
 template <int FORM, int SIDE>
-__device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, float4 *sbuf, int *jbuf, int &sb, int lane) {
+__device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, float4 *ring, float4 *sbuf, int *jbuf, int lane) {
     const float pinf = __int_as_float(0x7f800000);
     const int n_own = SIDE ? a.M : a.N;
     const int ncs = ((SIDE ? a.M : a.N) + 31) >> 5, nco = ((SIDE ? a.N : a.M) + 31) >> 5;
@@ -374,17 +397,27 @@ __device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, fl
     const float *orec = reinterpret_cast<const float *>(a.brec) + (own + (slot & ~1)) * 4 + (slot & 1);
     const float m2x = -2.f * __ldg(orec), m2y = -2.f * __ldg(orec + 2), m2z = -2.f * __ldg(orec + 4), pn = __ldg(orec + 6);
     const float4 *crec = a.brec + opp;
+    const int cs = (int)((long long)c * nco / ncs);
+    const float4 *cbox = a.bbox + 2 * (opp / 32);
+    // boxes of chunks base + lane; lanes past the cloud get an empty box (never read by the filter)
+    auto load_boxes = [&](int base, float4 &lo, float4 &hi) {
+        const int cb = base + lane;
+        lo = cb < nco ? __ldg(cbox + 2 * cb) : make_float4(0.f, 0.f, 0.f, 0.f);
+        hi = cb < nco ? __ldg(cbox + 2 * cb + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
+    };
+    float4 nlo, nhi;
+    load_boxes(0, nlo, nhi);          // in flight during the seeds
+#ifdef PCD_SWEEP_TRACE
+    unsigned long long n_eval = 0, n_scan = 0, n_tie = 0;
+#endif
 
     float best = pinf;
     uint32_t tag = 0;
     bool tie = false;
-    auto evaluate = [&](int cc, float4 v) {
-        float4 *s = sbuf + sb * 32;
-        sb ^= 1;
-        s[lane] = v;                  // the buffer was last read two chunks ago (this item or the last), before the previous __syncwarp
-        __syncwarp();
+    auto evaluate = [&](int cc, const float4 *s) {
+        __syncwarp();                 // the copies of every lane into the slot are visible
         float m = pinf;
-#pragma unroll
+#pragma unroll 8                      // fully unrolled, the loop spills at the 3-CTA register budget
         for (int k = 0; k < 16; ++k) {
             const float4 A = s[2 * k], Bv = s[2 * k + 1];
             const f32x2 d = pair_dist_fixed_x2<FORM>(SIDE == 0, m2x, m2y, m2z, pn, pack2(A.x, A.y), pack2(A.z, A.w),
@@ -395,32 +428,52 @@ __device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, fl
         }
         if (m < best) { best = m; tag = (uint32_t)cc; tie = false; }
         else if (m == best && m < pinf) tie = true;
+#ifdef PCD_SWEEP_TRACE
+        ++n_eval;
+#endif
     };
-    // queue chunk cc (-1: none): its records are requested now, the chunk queued before it is evaluated
-    int pend = -1;
-    float4 pv = make_float4(0.f, 0.f, 0.f, 0.f);
+    // queue chunk cc (-1: none): its records are copied into ring slot rs now, and the chunk queued two pushes
+    // before it (slot rs + 1 of 3) is evaluated.  The copies bypass the registers, so the depth costs none.
+    int q0 = -1, q1 = -1, rs = 0;
     auto push = [&](int cc) {
-        const float4 v = cc >= 0 ? __ldg(crec + (size_t)cc * 32 + lane) : make_float4(0.f, 0.f, 0.f, 0.f);
-        if (pend >= 0) evaluate(pend, pv);
-        pend = cc; pv = v;
+        __syncwarp();                 // every lane is done with the chunk evaluated at the last push, the old tenant of slot rs
+        if (cc >= 0) cp_async16(ring + rs * 32 + lane, crec + (size_t)cc * 32 + lane);
+        cp_async_commit();
+        const int ev = rs == 2 ? 0 : rs + 1;
+        if (q0 >= 0) {
+            cp_async_wait<2>();
+            evaluate(q0, ring + ev * 32);
+        }
+        q0 = q1; q1 = cc; rs = ev;
     };
-
-    const int cs = (int)((long long)c * nco / ncs);
-    const float4 *obox = a.bbox + 2 * (own / 32 + c), *cbox = a.bbox + 2 * (opp / 32);
-    const float4 alo = __ldg(obox), ahi = __ldg(obox + 1);
-    const bool keep_all = ahi.w != 0.f;
+    auto drain = [&]() {
+#pragma unroll 1
+        for (int k = 0; k < 2; ++k) push(-1);
+    };
+    // the seeds cs, cs - 1, cs + 1 (those inside the other cloud)
     auto seeds = [&](auto &&fn) {
-        fn(cs);
-        if (cs > 0) fn(cs - 1);
-        if (cs + 1 < nco) fn(cs + 1);
+#pragma unroll 1
+        for (int k = 0; k < 3; ++k) {
+            const int cc = cs + (k == 0 ? 0 : (k == 1 ? -1 : 1));
+            if (cc >= 0 && cc < nco) fn(cc);
+        }
     };
-    float U = pinf;
-    auto kept = [&](auto &&fn) {         // every other chunk the bound keeps, in index order
+    seeds(push);
+    drain();
+    // box stage, once per item: lane g ends with the ballots of chunks 32g .. 32g + 31 (kmask: kept, fmask: kept
+    // whatever the point stage says), so nothing of it stays live while chunks are evaluated
+    uint32_t kmask = 0, fmask = 0;
+    {
+        const float4 *obox = a.bbox + 2 * (own / 32 + c);
+        const float4 alo = __ldg(obox), ahi = __ldg(obox + 1);
+        const bool keep_all = ahi.w != 0.f;
+        const float U = ordered_to_f32(__reduce_max_sync(0xffffffffu, valid ? f32_to_ordered(best) : 0u));
         for (int base = 0; base < nco; base += 32) {
+            const float4 clo = nlo, chi = nhi;
+            if (base + 32 < nco) load_boxes(base + 32, nlo, nhi);
             const int cb = base + lane;
             bool keep = false;
             if (cb < nco && (cb < cs - 1 || cb > cs + 1)) {
-                const float4 clo = __ldg(cbox + 2 * cb), chi = __ldg(cbox + 2 * cb + 1);
                 const float gx = fmaxf(fmaxf(clo.x - ahi.x, alo.x - chi.x), 0.f);
                 const float gy = fmaxf(fmaxf(clo.y - ahi.y, alo.y - chi.y), 0.f);
                 const float gz = fmaxf(fmaxf(clo.z - ahi.z, alo.z - chi.z), 0.f);
@@ -428,26 +481,37 @@ __device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, fl
                 const float e = kPruneMarginRel * (alo.w + clo.w) + kPruneMarginAbs;
                 keep = keep_all || chi.w != 0.f || !(lb - e > U);
             }
-            for (uint32_t msk = __ballot_sync(0xffffffffu, keep); msk; msk &= msk - 1) fn(base + __ffs(msk) - 1);
+            const uint32_t k = __ballot_sync(0xffffffffu, keep), f = __ballot_sync(0xffffffffu, keep && (keep_all || chi.w != 0.f));
+            if (lane == base >> 5) { kmask = k; fmask = f; }
+        }
+    }
+    // point stage: every chunk of the box stage that some lane with `need` set does not skip, in index order
+    auto kept = [&](auto &&fn, bool need) {
+        for (int base = 0; base < nco; base += 32) {
+            const uint32_t force = __shfl_sync(0xffffffffu, fmask, base >> 5);
+            for (uint32_t msk = __shfl_sync(0xffffffffu, kmask, base >> 5); msk; msk &= msk - 1) {
+                const int k = __ffs(msk) - 1;
+                const float4 blo = __ldg(cbox + 2 * (base + k)), bhi = __ldg(cbox + 2 * (base + k) + 1);     // L1 hits
+                const float px = -0.5f * m2x, py = -0.5f * m2y, pz = -0.5f * m2z;     // exact
+                const float gx = fmaxf(fmaxf(blo.x - px, px - bhi.x), 0.f);
+                const float gy = fmaxf(fmaxf(blo.y - py, py - bhi.y), 0.f);
+                const float gz = fmaxf(fmaxf(blo.z - pz, pz - bhi.z), 0.f);
+                const float lb = (gx * gx + gy * gy + gz * gz) * kPruneLbScale;
+                const float e = kPruneMarginRel * (pn + blo.w) + kPruneMarginAbs;
+                if (((force >> k) & 1u) || __any_sync(0xffffffffu, need && !(lb - e > best))) fn(base + k);
+            }
         }
     };
-    seeds(push);
-    push(-1);
-    U = ordered_to_f32(__reduce_max_sync(0xffffffffu, valid ? f32_to_ordered(best) : 0u));
-    kept(push);
-    push(-1);
+    kept(push, valid);
+    drain();
 
-    // arg-min: the lowest original index with d == minimum among the candidates of chunk cc, for the lanes that ask
+    // arg-min: the lowest original index with d == minimum among the candidates in stage buffer sb, for the lanes that ask
     int arg = 0x7fffffff;
-    auto scan = [&](int cc, bool want) {
-        const float4 v = __ldg(crec + (size_t)cc * 32 + lane);
-        const int jv = __ldg(a.bperm + opp + (size_t)cc * 32 + lane);    // slots past the cloud are inert: never matched
-        float4 *s = sbuf + sb * 32;
-        int *js = jbuf + sb * 32;
-        sb ^= 1;
-        s[lane] = v; js[lane] = jv;
-        __syncwarp();
+    auto compare = [&](int sb, bool want) {
+        __syncwarp();                 // the copies of every lane into the buffer are visible
         if (want) {
+            const float4 *s = sbuf + sb * 32;
+            const int *js = jbuf + sb * 32;
 #pragma unroll
             for (int k = 0; k < 16; ++k) {
                 const float4 A = s[2 * k], Bv = s[2 * k + 1];
@@ -460,20 +524,61 @@ __device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, fl
             }
         }
     };
-    // a lane whose minimum one chunk reached: that chunk, one pass per distinct winning chunk (neighbours share a few)
+    // records and original indices of chunk cc (-1: none) into stage buffer sb, one commit group; slots past the cloud
+    // are inert: never matched.  Every lane must be done with the buffer's last compare (a __syncwarp in between).
+    auto stage_scan = [&](int cc, int sb) {
+        if (cc >= 0) {
+            cp_async16(sbuf + sb * 32 + lane, crec + (size_t)cc * 32 + lane);
+            cp_async4(jbuf + sb * 32 + lane, a.bperm + opp + (size_t)cc * 32 + lane);
+        }
+        cp_async_commit();
+    };
+    // a lane whose minimum one chunk reached: that chunk, one pass per distinct winning chunk (neighbours share a few);
+    // the next one is copied into the other buffer while the current one is compared
     bool pending = valid && best < pinf && !tie;
-    for (uint32_t pm = __ballot_sync(0xffffffffu, pending); pm; pm = __ballot_sync(0xffffffffu, pending)) {
-        const int cc = __shfl_sync(0xffffffffu, (int)tag, __ffs(pm) - 1);
-        scan(cc, pending && tag == (uint32_t)cc);
-        if (tag == (uint32_t)cc) pending = false;
+    uint32_t pm = __ballot_sync(0xffffffffu, pending);
+    int cc = pm ? __shfl_sync(0xffffffffu, (int)tag, __ffs(pm) - 1) : -1;
+    int sb = 0;
+    stage_scan(cc, sb);
+    while (cc >= 0) {
+        const bool mine = pending && tag == (uint32_t)cc;
+        if (mine) pending = false;
+        pm = __ballot_sync(0xffffffffu, pending);
+        const int nc = pm ? __shfl_sync(0xffffffffu, (int)tag, __ffs(pm) - 1) : -1;
+        __syncwarp();                 // every lane is done with the last compare, which read buffer sb ^ 1
+        stage_scan(nc, sb ^ 1);
+        cp_async_wait<1>();
+        compare(sb, mine);
+        cc = nc; sb ^= 1;
+#ifdef PCD_SWEEP_TRACE
+        ++n_scan;
+#endif
     }
-    // a lane whose minimum two chunks reached (an exact tie, rare): every chunk the item evaluated, once more
+    // a lane whose minimum two chunks reached (an exact tie, rare): every chunk it does not skip at its final minimum,
+    // once more (a superset of the chunks that can hold a pair equal to it)
     const bool tied = valid && best < pinf && tie;
     if (__any_sync(0xffffffffu, tied)) {
-        auto all = [&](int cc) { scan(cc, tied); };
+        auto all = [&](int cc2) {
+            __syncwarp();
+            stage_scan(cc2, sb);
+            cp_async_wait<0>();
+            compare(sb, tied);
+            sb ^= 1;
+        };
         seeds(all);
-        kept(all);
+        kept(all, tied);
+#ifdef PCD_SWEEP_TRACE
+        ++n_tie;
+#endif
     }
+#ifdef PCD_SWEEP_TRACE
+    if (g_prune_count && lane == 0) {
+        atomicAdd(g_prune_count, 1ull);
+        atomicAdd(g_prune_count + 1, n_eval);
+        atomicAdd(g_prune_count + 2, n_scan);
+        atomicAdd(g_prune_count + 3, n_tie);
+    }
+#endif
 
     if (valid) {
         const int p = __ldg(a.bperm + own + slot);
@@ -486,21 +591,22 @@ __device__ __forceinline__ void pruned_item(const PruneArgs &a, int b, int c, fl
 
 template <int FORM>
 __global__ void __launch_bounds__(kPruneThreads, 3) nn1_pruned_sweep_kernel(PruneArgs a) {
-    __shared__ __align__(16) float4 stage[kPruneThreads / 32][2 * 32];
+    __shared__ __align__(16) float4 ring[kPruneThreads / 32][3 * 32];      // candidate records in flight and under evaluation
+    __shared__ __align__(16) float4 stage[kPruneThreads / 32][2 * 32];     // the arg-min passes' records and indices
     __shared__ int jstage[kPruneThreads / 32][2 * 32];
     pdl_launch_dependents();
     pdl_wait();                   // records, boxes, permutation and the queue cursor come from nn1_bucket
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int ncr = (a.N + 31) >> 5, per_b = ncr + ((a.M + 31) >> 5), items = a.B * per_b;
-    int sb = 0;                   // which of the warp's two chunk buffers is written next
     for (;;) {
+        // recomputed per item from the special and constant-bank registers: nothing stays live across an item
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        const int ncr = (a.N + 31) >> 5, per_b = ncr + ((a.M + 31) >> 5);
         int item = 0;
         if (lane == 0) item = atomicAdd(a.queue, 1);
         item = __shfl_sync(0xffffffffu, item, 0);
-        if (item >= items) break;
+        if (item >= a.B * per_b) break;
         const int b = item / per_b, r = item - b * per_b;
-        if (r < ncr) pruned_item<FORM, 0>(a, b, r, stage[warp], jstage[warp], sb, lane);
-        else pruned_item<FORM, 1>(a, b, r - ncr, stage[warp], jstage[warp], sb, lane);
+        if (r < ncr) pruned_item<FORM, 0>(a, b, r, ring[warp], stage[warp], jstage[warp], lane);
+        else pruned_item<FORM, 1>(a, b, r - ncr, ring[warp], stage[warp], jstage[warp], lane);
     }
 }
 
@@ -1570,6 +1676,12 @@ using namespace pcd;
 extern "C" int pcd_debug_set_sweep_trace(void *buf) {
     unsigned long long *p = (unsigned long long *)buf;
     PCD_CUDA_CHECK(cudaMemcpyToSymbol(g_sweep_trace, &p, sizeof(p)));
+    return PCD_OK;
+}
+// buf: 4 zeroed uint64 counters the pruned sweep adds to (items, evaluated chunks, arg-min re-scans, tie passes); NULL stops
+extern "C" int pcd_debug_set_prune_counters(void *buf) {
+    unsigned long long *p = (unsigned long long *)buf;
+    PCD_CUDA_CHECK(cudaMemcpyToSymbol(g_prune_count, &p, sizeof(p)));
     return PCD_OK;
 }
 #endif

@@ -8,13 +8,21 @@ N=M=4096, the worst case) it prints one JSON line each with
                           L2 overwritten before every rep)
   old_us                  the full chain (arm + sweep + fix-up) at the same inputs, selected by passing the tiling that the
                           library would choose for it (an explicit tiling keeps the full sweep)
-  kept_pairs_frac         evaluated pairs / B*N*M, both directions, from a numpy model of the bucketing, seed and bound (the
-                          kernel keeps no counters); float64 seed minima, so it is a model, not a count
+  kept_pairs_frac         evaluated pairs / B*N*M, both directions, from a numpy model of the bucketing, the seeds and the two
+                          filter stages (box against U, then point against the lane's running minimum, candidates in index
+                          order); float64 minima, so it is a model, not a count
   k2_gpairs_per_s         evaluated pairs per second of the pruned sweep, from the model's pair count
+
+    python tools/nn1_prune_bench.py --count
+
+runs the same workloads on a -DPCD_SWEEP_TRACE build of the library (tools/libpcdist_trace.so, built if missing) and prints
+what the pruned sweep counted instead of times: counted_pairs_frac (evaluated chunks * 32 * 32 / B*N*M, exact for whole
+chunks), and per item the evaluated chunks, arg-min re-scans and tie passes.
 """
 import argparse
 import ctypes
 import importlib
+import importlib.util
 import json
 import os
 import sys
@@ -23,9 +31,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+TRACE_LIB = os.path.join(ROOT, "tools", "libpcdist_trace.so")
+if "--count" in sys.argv:          # before the package import: the library path is read once, at import
+    os.environ["PCDIST_LIBRARY"] = TRACE_LIB
 synth = importlib.import_module("3dpointcloudattack_b200.synth")
 
-BITS = 9
+BITS = 5
 MARGIN_REL, MARGIN_ABS, LB_SCALE = 40.0 * 2.0 ** -24, 2.0 ** -100, 1.0 - 2.0 ** -20
 
 
@@ -58,13 +69,43 @@ def model_sample(rows, cols):
             cs = c * len(ch_c) // len(ch_o)
             seeds = [k for k in (cs - 1, cs, cs + 1) if 0 <= k < len(ch_c)]
             cand = np.concatenate([ch_c[k] for k in seeds])
-            U = ((pts[:, None, :] - cand[None]) ** 2).sum(-1).min(1).max()
+            best = ((pts[:, None, :] - cand[None]) ** 2).sum(-1).min(1)
+            kept += len(pts) * len(cand)
+            # box stage against U = the largest seed minimum
             gap = np.maximum(np.maximum(lo_c - hi_o[c], lo_o[c] - hi_c), 0)
             lb = (gap ** 2).sum(1) * LB_SCALE
-            keep = ~(lb - (MARGIN_REL * (n_o[c] + n_c) + MARGIN_ABS) > U)
-            keep[seeds] = True
-            kept += sum(len(pts) * len(ch_c[k]) for k in np.flatnonzero(keep))
+            keep = ~(lb - (MARGIN_REL * (n_o[c] + n_c) + MARGIN_ABS) > best.max())
+            keep[seeds] = False
+            # point stage, in index order, against each point's running minimum
+            pn = (pts ** 2).sum(1)
+            for k in np.flatnonzero(keep):
+                g = np.maximum(np.maximum(lo_c[k] - pts, pts - hi_c[k]), 0)
+                lbp = (g ** 2).sum(1) * LB_SCALE
+                if (~(lbp - (MARGIN_REL * (pn + n_c[k]) + MARGIN_ABS) > best)).any():
+                    best = np.minimum(best, ((pts[:, None, :] - ch_c[k][None]) ** 2).sum(-1).min(1))
+                    kept += len(pts) * len(ch_c[k])
     return kept
+
+
+def counts(adv, ori):
+    """The pruned sweep's own counters over one call (trace build): items, evaluated chunks, arg-min re-scans, tie passes."""
+    import torch
+    pcd = importlib.import_module("3dpointcloudattack_b200")
+    F, lib = pcd.functional, pcd._lib.load()
+    a, o = torch.from_numpy(adv).cuda(), torch.from_numpy(ori).cuda()
+    F.nn1(a, o, F.FORM_SUM_FIRST, F.NORM_FMA, cache=False)
+    buf = torch.zeros(4, dtype=torch.int64, device="cuda")
+    fn = lib.pcd_debug_set_prune_counters
+    fn.restype, fn.argtypes = ctypes.c_int, [ctypes.c_void_p]
+    torch.cuda.synchronize()
+    assert fn(buf.data_ptr()) == 0
+    F.nn1(a, o, F.FORM_SUM_FIRST, F.NORM_FMA, cache=False)
+    torch.cuda.synchronize()
+    assert fn(None) == 0
+    items, chunks, scans, ties = buf.tolist()
+    B, N, M = a.shape[0], a.shape[1], o.shape[1]
+    return {"counted_pairs_frac": chunks * 32 * 32 / (B * N * M), "chunks_per_item": chunks / items,
+            "rescans_per_item": scans / items, "tie_passes_per_item": ties / items}
 
 
 def inputs(kind, B, n):
@@ -118,14 +159,22 @@ def main():
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--model-only", action="store_true")
     ap.add_argument("--model-samples", type=int, default=2)
+    ap.add_argument("--count", action="store_true")
     args = ap.parse_args()
+    if args.count and not os.path.exists(TRACE_LIB):
+        spec = importlib.util.spec_from_file_location("_b", os.path.join(ROOT, "3dpointcloudattack_b200", "build.py"))
+        b = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(b)
+        b.build(extra_flags=["-DPCD_SWEEP_TRACE"], out=TRACE_LIB)
     for name, kind, B, n in (("configs1", "face", 32, 4096), ("face_b32_n8192", "face", 32, 8192), ("face_b16_n16384", "face", 16, 16384),
                              ("face_b64_n16384", "face", 64, 16384), ("configs4", "face", 512, 16384), ("uniform", "uniform", 32, 4096)):
         adv, ori = inputs(kind, B, n)
         S = min(args.model_samples, B)
         frac = sum(model_sample(adv[b], ori[b]) for b in range(S)) / (S * n * n)
         res = {"workload": name, "B": B, "N": n, "kept_pairs_frac": frac}
-        if not args.model_only:
+        if args.count:
+            res.update(counts(adv, ori))
+        elif not args.model_only:
             import torch
             res["gpu"] = torch.cuda.get_device_name(0)
             res.update(gpu_times(adv, ori, args.reps))
