@@ -25,8 +25,6 @@
 // attack/GeoA3/knn_utils.py:10-55 (K=1); see include/pcdist.h.
 #include <type_traits>
 
-#include <cub/block/block_radix_sort.cuh>
-
 #include "pcd_common.cuh"
 
 namespace pcd {
@@ -42,8 +40,8 @@ constexpr int kFixupCtasPerSm = 2;                // 128 registers per thread: t
 constexpr int kFixupMaxWarps = 16384;             // upper bound of the persistent fix-up grid (any device)
 
 constexpr int kPruneMaxPoints = 16384;            // bucketing capacity per cloud (nn1_bucket_kernel sorts in shared memory)
-constexpr int kPruneMinPoints = 4096;             // smaller clouds or batches: the bucketing pass (~30 us at any batch on a
-constexpr int kPruneMinBatch = 16;                // B200) costs more than the pruning saves (DESIGN.md section 4.0)
+constexpr int kPruneMinPoints = 4096;             // smaller clouds or batches: the bucketing pass costs more than the pruning
+constexpr int kPruneMinBatch = 16;                // saves; set when it took ~30 us on a B200, ~17 us now (DESIGN.md section 4.0)
 
 struct Nn1Layout {
     int Npad, Mpad;
@@ -167,18 +165,48 @@ __global__ void nn1_prep_kernel(const float *__restrict__ rows, int64_t r_sb, in
 //
 // nn1_bucket: one CTA per (sample, side).  Both clouds of a sample are quantised on ONE grid (the
 // joint box of their finite points, 32 cells per axis), each side is sorted by the 15-bit Morton
-// code of its cell (stable block radix sort, so equal codes keep index order), and the sorted
-// cloud is cut into chunks of 32.  Written per (sample, side):
+// code of its cell (stable, so equal codes keep index order), and the sorted cloud is cut into
+// chunks of 32.  Written per (sample, side):
 //   brec [slot]  pair records {x0,x1,y0,y1},{z0,z1,n0,n1} in sorted order; slots past the cloud
 //                are inert (0, 0, 0, +inf), as in the packed sweep
 //   bperm[slot]  original index of the point in that slot
 //   bbox [chunk] (lo xyz, largest norm), (hi xyz, never-prune flag) over the chunk's points
 // Non-finite points get a code past every finite one, so they share the last chunks, whose
 // never-prune flag makes every comparison against them keep the pair.
+//
+// The pass is latency bound (a few hundred KB per CTA), so it is built from as few dependent
+// steps as possible: 16-byte loads of 4 points at a time, codes packed with the point index into one
+// 32-bit word (code << 14 | index, so only the word moves through the sort), two 8-bit LSD radix
+// passes in shared memory with four barriers each, and one gather of the sorted points from L1 / L2
+// with every load in flight before the first store.
 constexpr int kBucketThreads = 1024;
+constexpr int kBucketWarps = kBucketThreads / 32;
 constexpr int kMortonBits = 5;                    // cells per axis = 2^5: finer grids make no better chunks
                                                   // (DESIGN.md section 4.0) and cost radix-sort passes
 constexpr uint32_t kNonFiniteCode = 1u << (3 * kMortonBits);
+constexpr int kBucketIndexBits = 14;              // kPruneMaxPoints = 2^14
+constexpr int kBucketDigits = 256;
+constexpr int kBucketCntStride = kBucketDigits + 1;   // per-warp digit counters; +1: the scan's transposed reads hit 32 banks
+static_assert(kPruneMaxPoints <= (1 << kBucketIndexBits), "the sort word holds the point index in its low bits");
+
+#ifdef PCD_SWEEP_TRACE
+// development build only (tools/trace_sweep.py, tools/nn1_prune_bench.py --count): per-CTA timestamps of the sweep or of
+// the bucketing pass (whichever chain runs)
+__device__ unsigned long long *g_sweep_trace = nullptr;
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+    return t;
+}
+// phase k of the bucketing pass ends (0 = start, 1 loads + joint box, 2 codes, 3 / 4 sort passes, 5 gather + stores), in
+// the CTA's 8 words of the trace buffer (tools/nn1_prune_bench.py --count reads them)
+#define PCD_BUCKET_STAMP(k)                                                                         \
+    do {                                                                                            \
+        if (g_sweep_trace && threadIdx.x == 0) g_sweep_trace[blockIdx.x * 8 + (k)] = globaltimer_ns(); \
+    } while (0)
+#else
+#define PCD_BUCKET_STAMP(k) do { } while (0)
+#endif
 
 __device__ __forceinline__ uint32_t spread3(uint32_t v) {     // bit k of v -> bit 3k
     v &= 0x3ffu;
@@ -193,15 +221,138 @@ struct BucketArgs {
     const float *rows; long long r_sb, r_sp, r_sc;
     const float *cols; long long c_sb, c_sp, c_sc;
     int N, M, norm_kind, bslots;
-    float *brec; float4 *bbox; int *bperm;
+    float4 *brec; float4 *bbox; int *bperm;
     int *counters; int *queue;
 };
 
+// One dense cloud of the pruned chain: point-major [n,3] (sc == 1) or channel-major [3,n] rows, 16-byte aligned, n % 4 == 0
+// (dense_layout), so 4 consecutive points are three 16-byte loads either way.
+struct BucketCloud {
+    const float *__restrict__ p;
+    long long sc;
+    __device__ __forceinline__ void quad(int g, float x[4], float y[4], float z[4]) const {
+        if (sc == 1) {
+            const float4 *q = reinterpret_cast<const float4 *>(p) + 3 * g;
+            const float4 a = __ldg(q), b = __ldg(q + 1), c = __ldg(q + 2);
+            x[0] = a.x; y[0] = a.y; z[0] = a.z; x[1] = a.w; y[1] = b.x; z[1] = b.y;
+            x[2] = b.z; y[2] = b.w; z[2] = c.x; x[3] = c.y; y[3] = c.z; z[3] = c.w;
+        } else {
+            const float4 a = __ldg(reinterpret_cast<const float4 *>(p) + g);
+            const float4 b = __ldg(reinterpret_cast<const float4 *>(p + sc) + g);
+            const float4 c = __ldg(reinterpret_cast<const float4 *>(p + 2 * sc) + g);
+            x[0] = a.x; x[1] = a.y; x[2] = a.z; x[3] = a.w; y[0] = b.x; y[1] = b.y; y[2] = b.z; y[3] = b.w;
+            z[0] = c.x; z[1] = c.y; z[2] = c.z; z[3] = c.w;
+        }
+    }
+    __device__ __forceinline__ void point(int i, float &x, float &y, float &z) const {
+        const float *q = p + (sc == 1 ? 3LL * i : (long long)i);
+        x = __ldg(q); y = __ldg(q + sc); z = __ldg(q + 2 * sc);
+    }
+};
+
+__device__ __forceinline__ bool finite3(float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); }
+
+// One stable LSD pass over the 8-bit digit at `shift` of n sort words, src -> dst (shared memory).  Warp w ranks the items
+// [w*S, w*S + S), S = 32 * steps, in index order: eight ballots group the lanes of one step by digit (a fixed cost, where
+// __match_any_sync serialises over the distinct digits), the highest lane of each group advances the warp's own counter of
+// that digit.  A block scan over (digit, warp) turns the counters into
+// output offsets.  4 barriers.
+template <int ITEMS>
+__device__ __forceinline__ void bucket_sort_pass(const uint32_t *src, uint32_t *dst, int *cnt, int *wsum, int n, int steps,
+                                                 int shift, int tid) {
+    const int lane = tid & 31, warp = tid >> 5, S = 32 * steps;
+    int *row = cnt + warp * kBucketCntStride;
+#pragma unroll
+    for (int d = lane; d < kBucketDigits; d += 32) row[d] = 0;
+    __syncwarp();
+    int local[ITEMS];
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+        if (k < steps) {
+            const int i = warp * S + 32 * k + lane;
+            const bool v = i < n;
+            const int d = v ? (int)((src[i] >> shift) & (kBucketDigits - 1)) : 0;
+            unsigned peers = __ballot_sync(0xffffffffu, v);     // the valid lanes with digit d: one ballot per digit bit
+#pragma unroll
+            for (int bit = 0; bit < 8; ++bit) {
+                const unsigned m = __ballot_sync(0xffffffffu, (d >> bit) & 1);
+                peers &= (d >> bit) & 1 ? m : ~m;
+            }
+            const int leader = 31 - __clz(peers);
+            int old = 0;
+            if (v && lane == leader) { old = row[d]; row[d] = old + __popc(peers); }
+            local[k] = __shfl_sync(0xffffffffu, old, leader) + __popc(peers & ((1u << lane) - 1));
+            __syncwarp();
+        }
+    }
+    __syncthreads();
+    // thread (digit d, quarter q) scans the counters of warps 8q .. 8q+7 for digit d; the warp holds digits 8*warp .. +7
+    const int d = tid >> 2, q = tid & 3;
+    int sum = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) sum += cnt[(8 * q + j) * kBucketCntStride + d];
+    int incl = sum;                                           // over the quarters of digit d
+#pragma unroll
+    for (int o = 1; o < 4; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (q >= o) incl += t;
+    }
+    const int total = __shfl_sync(0xffffffffu, incl, lane | 3);
+    int dig = total;                                          // over the digits of this warp, up to d
+#pragma unroll
+    for (int o = 4; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, dig, o);
+        if (lane >= o) dig += t;
+    }
+    if (lane == 31) wsum[warp] = dig;
+    __syncthreads();
+    int below = lane < warp ? wsum[lane] : 0;                 // digits of the warps before this one
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) below += __shfl_xor_sync(0xffffffffu, below, o);
+    int run = below + dig - total + incl - sum;               // only this thread writes the counters it read
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        int *c = cnt + (8 * q + j) * kBucketCntStride + d;
+        const int v = *c;
+        *c = run;
+        run += v;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+        if (k < steps) {
+            const int i = warp * S + 32 * k + lane;
+            if (i < n) {
+                const uint32_t w = src[i];
+                dst[row[(w >> shift) & (kBucketDigits - 1)] + local[k]] = w;
+            }
+        }
+    }
+    __syncthreads();
+}
+
+// Clouds of up to 4096 points keep their coordinates in shared memory (48 KB) for the gather; larger ones (192 KB would not
+// fit beside the sort) gather from L1 / L2.
+template <int ITEMS>
+__host__ __device__ constexpr bool bucket_stages_points() { return ITEMS <= 4; }
+// dynamic shared memory: two word buffers of kBucketThreads * ITEMS, the per-warp digit counters, then x, y, z if staged
+template <int ITEMS>
+constexpr size_t bucket_smem_bytes() {
+    return ((2 + (bucket_stages_points<ITEMS>() ? 3 : 0)) * (size_t)kBucketThreads * ITEMS +
+            (size_t)kBucketWarps * kBucketCntStride) * sizeof(uint32_t);
+}
+
 template <int ITEMS>
 __global__ void __launch_bounds__(kBucketThreads, 1) nn1_bucket_kernel(BucketArgs a) {
-    using Sort = cub::BlockRadixSort<uint32_t, kBucketThreads, ITEMS, int>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ float red[6][kBucketThreads / 32];
+    uint32_t *wa = reinterpret_cast<uint32_t *>(smem_raw), *wb = wa + kBucketThreads * ITEMS;
+    int *cnt = reinterpret_cast<int *>(wb + kBucketThreads * ITEMS);
+    constexpr bool kStaged = bucket_stages_points<ITEMS>();
+    float *sx = reinterpret_cast<float *>(cnt + kBucketWarps * kBucketCntStride), *sy = sx + kBucketThreads * ITEMS,
+          *sz = sy + kBucketThreads * ITEMS;     // used only if kStaged
+    __shared__ float red[6][kBucketWarps];
+    __shared__ int wsum[kBucketWarps];
+    PCD_BUCKET_STAMP(0);
     pdl_launch_dependents();     // the pruned sweep may become resident; it waits for our completion
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.x >> 1, side = blockIdx.x & 1;
@@ -210,39 +361,28 @@ __global__ void __launch_bounds__(kBucketThreads, 1) nn1_bucket_kernel(BucketArg
         if (blockIdx.x == 0) *a.queue = 0;
     }
     const float pinf = __int_as_float(0x7f800000);
-    auto load = [&](int s, int i, float &x, float &y, float &z) {
-        const float *p = s ? a.cols + b * a.c_sb + i * a.c_sp : a.rows + b * a.r_sb + i * a.r_sp;
-        const long long sc = s ? a.c_sc : a.r_sc;
-        x = __ldg(p); y = __ldg(p + sc); z = __ldg(p + 2 * sc);
+    // built where it is used, from the parameter bank: kept live across the phases, the pointers spill
+    auto cloud = [&](int s) {
+        return s ? BucketCloud{a.cols + b * a.c_sb, a.c_sc} : BucketCloud{a.rows + b * a.r_sb, a.r_sc};
     };
-    auto finite3 = [](float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); };
+    const int n = side ? a.M : a.N;
 
-    // the CTA's own points (slots tid*ITEMS + k of the sort) stay in registers from here to their Morton codes
-    const int n = side ? a.M : a.N, n_other = side ? a.N : a.M;
-    float own[ITEMS][3];
+    // joint box of the sample's finite points: both CTAs of the sample compute the same one
     float lo[3] = {pinf, pinf, pinf}, hi[3] = {-pinf, -pinf, -pinf};
-    auto widen = [&](const float *p) {
-        if (finite3(p[0], p[1], p[2])) {
+    auto widen = [&](const BucketCloud &c, int g) {
+        float x[4], y[4], z[4];
+        c.quad(g, x, y, z);
 #pragma unroll
-            for (int c = 0; c < 3; ++c) { lo[c] = fminf(lo[c], p[c]); hi[c] = fmaxf(hi[c], p[c]); }
+        for (int e = 0; e < 4; ++e) {
+            if (finite3(x[e], y[e], z[e])) {
+                lo[0] = fminf(lo[0], x[e]); lo[1] = fminf(lo[1], y[e]); lo[2] = fminf(lo[2], z[e]);
+                hi[0] = fmaxf(hi[0], x[e]); hi[1] = fmaxf(hi[1], y[e]); hi[2] = fmaxf(hi[2], z[e]);
+            }
         }
     };
-#pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
-        const int i = tid * ITEMS + k;
-        own[k][0] = own[k][1] = own[k][2] = 0.f;
-        if (i < n) load(side, i, own[k][0], own[k][1], own[k][2]);
-    }
-    // joint box of the sample's finite points: both CTAs of the sample compute the same one
-#pragma unroll 4
-    for (int t = tid; t < n_other; t += kBucketThreads) {
-        float p[3];
-        load(side ^ 1, t, p[0], p[1], p[2]);
-        widen(p);
-    }
-#pragma unroll
-    for (int k = 0; k < ITEMS; ++k)
-        if (tid * ITEMS + k < n) widen(own[k]);
+    const int gr = a.N >> 2, gt = gr + (a.M >> 2);             // 4-point groups of the rows, then of the columns
+#pragma unroll 2
+    for (int g = tid; g < gt; g += kBucketThreads) widen(cloud(g >= gr), g < gr ? g : g - gr);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
 #pragma unroll
@@ -264,70 +404,122 @@ __global__ void __launch_bounds__(kBucketThreads, 1) nn1_bucket_kernel(BucketArg
         }
         cell[c] = hi[c] > lo[c] ? (float)(1 << kMortonBits) / (hi[c] - lo[c]) : 0.f;
     }
+    PCD_BUCKET_STAMP(1);
 
-    uint32_t key[ITEMS];
-    int val[ITEMS];
+    // sort words in index order (the own cloud is read again: L1 / L2 hits); non-finite points sort last, in index order
+    static_assert((kBucketWarps * kBucketCntStride) % 4 == 0, "the staged coordinates are stored as float4");
 #pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
-        const int i = tid * ITEMS + k;
-        val[k] = i;
-        key[k] = kNonFiniteCode;          // non-finite points and the padding past n sort last, in index order
-        if (i < n && finite3(own[k][0], own[k][1], own[k][2])) {
-            uint32_t code = 0;
+    for (int j = 0; j < ITEMS / 4; ++j) {
+        const int g = tid + j * kBucketThreads;
+        if (4 * g < n) {
+            float x[4], y[4], z[4];
+            cloud(side).quad(g, x, y, z);
+            uint32_t w[4];
 #pragma unroll
-            for (int c = 0; c < 3; ++c) {
-                const float q = fminf(fmaxf((own[k][c] - lo[c]) * cell[c], 0.f), (float)((1 << kMortonBits) - 1));
-                code |= spread3((uint32_t)q) << c;
+            for (int e = 0; e < 4; ++e) {
+                uint32_t code = kNonFiniteCode;
+                if (finite3(x[e], y[e], z[e])) {
+                    const float p[3] = {x[e], y[e], z[e]};
+                    code = 0;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) {
+                        const float qc = fminf(fmaxf((p[c] - lo[c]) * cell[c], 0.f), (float)((1 << kMortonBits) - 1));
+                        code |= spread3((uint32_t)qc) << c;
+                    }
+                }
+                w[e] = code << kBucketIndexBits | (uint32_t)(4 * g + e);
             }
-            key[k] = code;
+            reinterpret_cast<uint4 *>(wa)[g] = make_uint4(w[0], w[1], w[2], w[3]);
+            if (kStaged) {
+                reinterpret_cast<float4 *>(sx)[g] = make_float4(x[0], x[1], x[2], x[3]);
+                reinterpret_cast<float4 *>(sy)[g] = make_float4(y[0], y[1], y[2], y[3]);
+                reinterpret_cast<float4 *>(sz)[g] = make_float4(z[0], z[1], z[2], z[3]);
+            }
         }
     }
-    Sort(*reinterpret_cast<typename Sort::TempStorage *>(smem_raw)).Sort(key, val, 0, 3 * kMortonBits + 1);
+    __syncthreads();
+    PCD_BUCKET_STAMP(2);
+    const int steps = (n + kBucketThreads - 1) / kBucketThreads;
+    bucket_sort_pass<ITEMS>(wa, wb, cnt, wsum, n, steps, kBucketIndexBits, tid);
+    PCD_BUCKET_STAMP(3);
+    bucket_sort_pass<ITEMS>(wb, wa, cnt, wsum, n, steps, kBucketIndexBits + 8, tid);
+    PCD_BUCKET_STAMP(4);
 
-    // thread tid now holds the sorted slots tid*ITEMS + k
+    // wa holds the sorted words.  Thread tid writes the slot pairs (2t, 2t+1), t = tid + j * kBucketThreads: one 32-byte
+    // pair record and one 8-byte permutation entry; the 16 consecutive lanes that hold one chunk reduce its box.  The points
+    // come from shared memory if staged, else from L1 / L2.
+    const BucketCloud own = cloud(side);
     const size_t base = (size_t)(b * 2 + side) * a.bslots;
     const int nslots = (n + 31) & ~31;
-    float blo[3] = {pinf, pinf, pinf}, bhi[3] = {-pinf, -pinf, -pinf}, bn = -pinf;
-    int bad = 0;
+    constexpr int kBatch = ITEMS / 2 < 4 ? ITEMS / 2 : 4;     // slot pairs per thread with their loads in flight together
 #pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
-        const int s = tid * ITEMS + k;
-        if (s < nslots) {
-            float x = 0.f, y = 0.f, z = 0.f, nn = pinf;
-            if (s < n) {
-                load(side, val[k], x, y, z);
-                nn = sq_norm3(a.norm_kind, x, y, z);
-                a.bperm[base + s] = val[k];
-                if (finite3(x, y, z)) {
-                    blo[0] = fminf(blo[0], x); blo[1] = fminf(blo[1], y); blo[2] = fminf(blo[2], z);
-                    bhi[0] = fmaxf(bhi[0], x); bhi[1] = fmaxf(bhi[1], y); bhi[2] = fmaxf(bhi[2], z);
-                    bn = fmaxf(bn, nn);
-                } else {
-                    bad = 1;
+    for (int j0 = 0; j0 < ITEMS / 2; j0 += kBatch) {
+        float px[kBatch][2], py[kBatch][2], pz[kBatch][2];
+        int idx[kBatch][2];
+#pragma unroll
+        for (int j = 0; j < kBatch; ++j) {
+            const int s = 2 * (tid + (j0 + j) * kBucketThreads);
+            px[j][0] = px[j][1] = py[j][0] = py[j][1] = pz[j][0] = pz[j][1] = 0.f;
+            if (s < n) {                                      // n is even: both slots hold points
+                const uint2 w = reinterpret_cast<const uint2 *>(wa)[s >> 1];
+                idx[j][0] = (int)(w.x & ((1u << kBucketIndexBits) - 1));
+                idx[j][1] = (int)(w.y & ((1u << kBucketIndexBits) - 1));
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    if (kStaged) {
+                        px[j][e] = sx[idx[j][e]]; py[j][e] = sy[idx[j][e]]; pz[j][e] = sz[idx[j][e]];
+                    } else {
+                        own.point(idx[j][e], px[j][e], py[j][e], pz[j][e]);
+                    }
                 }
             }
-            float *rec = a.brec + (base + (s & ~1)) * 4 + (s & 1);
-            rec[0] = x; rec[2] = y; rec[4] = z; rec[6] = nn;
+        }
+#pragma unroll
+        for (int j = 0; j < kBatch; ++j) {
+            const int s = 2 * (tid + (j0 + j) * kBucketThreads);
+            float blo[3] = {pinf, pinf, pinf}, bhi[3] = {-pinf, -pinf, -pinf}, bn = -pinf, nn[2] = {pinf, pinf};
+            int bad = 0;
+            if (s < n) {
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    nn[e] = sq_norm3(a.norm_kind, px[j][e], py[j][e], pz[j][e]);
+                    if (finite3(px[j][e], py[j][e], pz[j][e])) {
+                        blo[0] = fminf(blo[0], px[j][e]); blo[1] = fminf(blo[1], py[j][e]); blo[2] = fminf(blo[2], pz[j][e]);
+                        bhi[0] = fmaxf(bhi[0], px[j][e]); bhi[1] = fmaxf(bhi[1], py[j][e]); bhi[2] = fmaxf(bhi[2], pz[j][e]);
+                        bn = fmaxf(bn, nn[e]);
+                    } else {
+                        bad = 1;
+                    }
+                }
+                reinterpret_cast<int2 *>(a.bperm + base)[s >> 1] = make_int2(idx[j][0], idx[j][1]);
+            }
+            if (s < nslots) {
+                float4 *rec = a.brec + base + s;                 // slots s, s+1 = the two float4 of one pair record
+                rec[0] = make_float4(px[j][0], px[j][1], py[j][0], py[j][1]);
+                rec[1] = make_float4(pz[j][0], pz[j][1], nn[0], nn[1]);
+            }
+#pragma unroll
+            for (int o = 1; o < 16; o <<= 1) {
+#pragma unroll
+                for (int c = 0; c < 3; ++c) {
+                    blo[c] = fminf(blo[c], __shfl_xor_sync(0xffffffffu, blo[c], o));
+                    bhi[c] = fmaxf(bhi[c], __shfl_xor_sync(0xffffffffu, bhi[c], o));
+                }
+                bn = fmaxf(bn, __shfl_xor_sync(0xffffffffu, bn, o));
+                bad |= __shfl_xor_sync(0xffffffffu, bad, o);
+            }
+            const int chunk = s >> 5;
+            if ((lane & 15) == 0 && chunk * 32 < n) {
+                float4 *bx = a.bbox + 2 * (base / 32 + chunk);
+                bx[0] = make_float4(blo[0], blo[1], blo[2], bn);
+                bx[1] = make_float4(bhi[0], bhi[1], bhi[2], bad ? 1.f : 0.f);
+            }
         }
     }
-    // chunk boxes: the 32 / ITEMS consecutive lanes that hold one chunk
-    constexpr int kLanesPerChunk = 32 / ITEMS;
-#pragma unroll
-    for (int o = 1; o < kLanesPerChunk; o <<= 1) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            blo[c] = fminf(blo[c], __shfl_xor_sync(0xffffffffu, blo[c], o));
-            bhi[c] = fmaxf(bhi[c], __shfl_xor_sync(0xffffffffu, bhi[c], o));
-        }
-        bn = fmaxf(bn, __shfl_xor_sync(0xffffffffu, bn, o));
-        bad |= __shfl_xor_sync(0xffffffffu, bad, o);
-    }
-    const int chunk = tid * ITEMS / 32;
-    if (tid % kLanesPerChunk == 0 && chunk * 32 < n) {
-        float4 *bx = a.bbox + 2 * (base / 32 + chunk);
-        bx[0] = make_float4(blo[0], blo[1], blo[2], bn);
-        bx[1] = make_float4(bhi[0], bhi[1], bhi[2], bad ? 1.f : 0.f);
-    }
+#ifdef PCD_SWEEP_TRACE
+    __syncthreads();
+    PCD_BUCKET_STAMP(5);
+#endif
 }
 
 // ---------------------------------------------------------------- pruned path: the sweep
@@ -650,16 +842,6 @@ struct SweepSmemPacked {
 };
 
 constexpr int kQuad = 4;   // columns per scheduling unit (two packed steps)
-
-#ifdef PCD_SWEEP_TRACE
-// development build only (tools/trace_sweep.py): per-CTA timestamps of the sweep
-__device__ unsigned long long *g_sweep_trace = nullptr;
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#endif
 
 template <int FORM, int R, bool RAW>
 __global__ void __launch_bounds__(kSweepThreads, (R >= 16) ? 2 : ((R >= 8) ? 4 : ((R >= 4) ? 5 : 6)))
@@ -1577,7 +1759,7 @@ static cudaError_t launch_sweep(int form, int R, const SweepSrc &src, unsigned l
 template <int ITEMS>
 static cudaError_t launch_bucket(const BucketArgs &a, int B, cudaStream_t st) {
     const auto kernel = nn1_bucket_kernel<ITEMS>;
-    const size_t smem = sizeof(typename cub::BlockRadixSort<uint32_t, kBucketThreads, ITEMS, int>::TempStorage);
+    const size_t smem = bucket_smem_bytes<ITEMS>();
     cudaError_t e = opt_in_smem(kernel, smem);
     if (e != cudaSuccess) return e;
     return launch_kernel(kernel, dim3((unsigned)(2 * B)), dim3(kBucketThreads), smem, st, false, a);
@@ -1771,7 +1953,7 @@ extern "C" int pcd_nn1_forward(const float *rows, int64_t r_sb, int64_t r_sp, in
     int *bperm = (int *)(ws + L.bperm);
     if (pruned) {
         const BucketArgs ba{rows, (long long)r_sb, (long long)r_sp, (long long)r_sc, cols, (long long)c_sb, (long long)c_sp,
-                            (long long)c_sc, N, M, norm_kind, L.bslots, (float *)(ws + L.brec), (float4 *)(ws + L.bbox), bperm,
+                            (long long)c_sc, N, M, norm_kind, L.bslots, (float4 *)(ws + L.brec), (float4 *)(ws + L.bbox), bperm,
                             counters, (int *)(ws + L.queue)};
         PCD_CUDA_CHECK(nmax <= 4 * kBucketThreads ? launch_bucket<4>(ba, B, st) : launch_bucket<16>(ba, B, st));
     } else if (raw) {

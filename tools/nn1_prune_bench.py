@@ -17,7 +17,10 @@ N=M=4096, the worst case) it prints one JSON line each with
 
 runs the same workloads on a -DPCD_SWEEP_TRACE build of the library (tools/libpcdist_trace.so, built if missing) and prints
 what the pruned sweep counted instead of times: counted_pairs_frac (evaluated chunks * 32 * 32 / B*N*M, exact for whole
-chunks), and per item the evaluated chunks, arg-min re-scans and tie passes.
+chunks), and per item the evaluated chunks, arg-min re-scans and tie passes.  It also reads the bucketing pass's phase stamps
+(%globaltimer, thread 0 of every CTA) and prints k1_phases_us: the median over CTAs of each phase (start -> loads and joint
+box -> codes -> sort pass 1 -> sort pass 2 -> gather and stores), and k1_span_us, first CTA start to last CTA end.  The
+stamps of the trace build add barriers of their own, so the phases are a breakdown, not the release kernel's time.
 """
 import argparse
 import ctypes
@@ -87,8 +90,12 @@ def model_sample(rows, cols):
     return kept
 
 
+K1_PHASES = ("loads_box", "codes", "sort1", "sort2", "gather_store")     # the ends of nn1_bucket's phases: stamps 1 .. 5
+
+
 def counts(adv, ori):
-    """The pruned sweep's own counters over one call (trace build): items, evaluated chunks, arg-min re-scans, tie passes."""
+    """The pruned sweep's own counters over one call (trace build): items, evaluated chunks, arg-min re-scans, tie passes,
+    and the bucketing pass's phase stamps (8 words per CTA: its start, then the end of each phase of K1_PHASES)."""
     import torch
     pcd = importlib.import_module("3dpointcloudattack_b200")
     F, lib = pcd.functional, pcd._lib.load()
@@ -104,8 +111,19 @@ def counts(adv, ori):
     assert fn(None) == 0
     items, chunks, scans, ties = buf.tolist()
     B, N, M = a.shape[0], a.shape[1], o.shape[1]
+    stamps = torch.zeros(2 * B * 8, dtype=torch.int64, device="cuda")
+    st = lib.pcd_debug_set_sweep_trace
+    st.restype, st.argtypes = ctypes.c_int, [ctypes.c_void_p]
+    assert st(stamps.data_ptr()) == 0
+    F.nn1(a, o, F.FORM_SUM_FIRST, F.NORM_FMA, cache=False)
+    torch.cuda.synchronize()
+    assert st(None) == 0
+    t = stamps.cpu().numpy().reshape(-1, 8).astype(np.float64)
+    end = len(K1_PHASES)
+    phases = {name: round(float(np.median(t[:, k + 1] - t[:, k])) / 1e3, 2) for k, name in enumerate(K1_PHASES)}
     return {"counted_pairs_frac": chunks * 32 * 32 / (B * N * M), "chunks_per_item": chunks / items,
-            "rescans_per_item": scans / items, "tie_passes_per_item": ties / items}
+            "rescans_per_item": scans / items, "tie_passes_per_item": ties / items,
+            "k1_phases_us": phases, "k1_span_us": round(float(t[:, end].max() - t[:, 0].min()) / 1e3, 2)}
 
 
 def inputs(kind, B, n):

@@ -1,6 +1,7 @@
 """Per-CTA timeline of the NN-1 sweep (development tool): builds a -DPCD_SWEEP_TRACE variant of the
 library, runs BASELINE config 2 and prints when CTAs start, reach their first tile, leave the loop
-and finish, relative to the earliest CTA start.
+and finish, relative to the earliest CTA start.  It passes the tiling the library would choose, which
+keeps the full sweep on shapes the pruned chain serves (whose bucketing pass writes other stamps).
 
     python tools/trace_sweep.py [B N M]
 """
@@ -32,6 +33,9 @@ def main():
     ori = synth.face_clouds(min(B, 4), N, seed=1).cuda().repeat((B + 3) // 4, 1, 1)[:B].contiguous()
     adv = (ori + 0.01 * torch.randn_like(ori))[:, :M].contiguous()
     trace = torch.zeros(4096 * 8, dtype=torch.int64, device="cuda")
+    R, mt = ctypes.c_int(), ctypes.c_int()
+    assert lib.pcd_nn1_query_tiling(B, N, M, ctypes.byref(R), ctypes.byref(mt)) == 0
+    F.force_tiling(R.value, mt.value)
     for _ in range(3):
         F.nn1(ori, adv, F.FORM_SUM_FIRST, F.NORM_FMA, cache=False)
     torch.cuda.synchronize()
@@ -41,6 +45,7 @@ def main():
     F.nn1(ori, adv, F.FORM_SUM_FIRST, F.NORM_FMA, cache=False)
     torch.cuda.synchronize()
     fn(None)
+    F.force_tiling(0, 0)
     t = trace.cpu().numpy().reshape(-1, 8)
     t = t[t[:, 0] > 0]
     t0 = t[:, 0].min()
