@@ -16,6 +16,7 @@ VALUE_SQUARED, VALUE_SQRT_CLAMP = 0, 1
 KNN_MAX_K, KNN_MAX_C = 64, 128
 SOR_MAX_K = 15
 SAMPLE_MAX_N = 16384
+SI_MAX_N, SI_MAX_SPLIT = 16384, 16
 EDGE_CENTER, EDGE_NEIGHBOR, EDGE_DIFF = 0, 1, 2
 
 _c = ctypes
@@ -55,6 +56,7 @@ SIGNATURES = {
     "pcd_nn_dist64_workspace_bytes": (_Z, [_I, _I, _I, _I]),
     "pcd_nn_dist64_forward": (_I, _CLOUD + _CLOUD + [_I, _I, _I, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "pcd_sample_points": (_I, [_I, _I, _I, _P, _P, _L, _c.c_uint64, _L, _P, _P, _P]),
+    "pcd_si_step": (_I, [_P, _L, _L, _L] + _CLOUD * 3 + [_I, _I, _c.c_double, _c.c_double, _F, _I, _P, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),
 }
 

@@ -19,6 +19,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
            "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "sample_points", "PointSampler", "nn_dist64", "NNDist64Result",
+           "shape_invariant_step_", "estimate_normals", "SI_STEP_SCALE",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -898,3 +899,58 @@ def offset_proj(offset, ori_normal, idx):
 def find_offset(adv, ori, idx):
     """GeoA3_attack.py:83-89 after its knn_points(K=1) (pcd_find_offset): adv - ori[:, :, idx].  No gradient."""
     return _offset_gather("pcd_find_offset", adv, ori, idx)
+
+
+# ------------------------------------------------ the SI-Adv shape-invariant step and the normals it re-estimates
+SI_STEP_SCALE = math.sqrt(3 * 1024)     # the reference's hard-coded step scale (SIadv_attack.py), whatever N is
+
+
+def shape_invariant_step_(pc, ori, normal, grad, step_size, eps, step_scale=SI_STEP_SCALE, split=0):
+    """One step of SI-Adv's shape_invariant_ifgm IN PLACE on pc (pcd_si_step in include/pcdist.h; get_spin_axis_matrix,
+    get_transformed_point_cloud, get_original_point_cloud of attack/SIadv/SIadv_attack.py): the gradient restricted to
+    every point's tangent plane, normalised over the sample, a step of step_size * step_scale against it, and the
+    reference's clip of the perturbation to eps, which on [B,N,3] clouds bounds each axis's norm over the whole cloud.
+    pc, ori, normal, grad [B,N,3] fp32 (any strides; grad = dL/d pc; the projection g - (g.n)n does not depend on the
+    sign of the normal).  -> gnorm [B], the per-sample norm of the tangent gradient.  One launch, no gradient, no host
+    synchronisation.  split > 0 forces the CTAs per sample (testing; the results do not change)."""
+    global _launch_count
+    for t, name in ((pc, "pc"), (ori, "ori"), (normal, "normal"), (grad, "grad")):
+        _check_cloud(t, name)
+        if t.shape != pc.shape or t.device != pc.device:
+            raise ValueError(f"{name} {tuple(t.shape)} on {t.device} does not match pc {tuple(pc.shape)} on {pc.device}")
+    B, N, _ = pc.shape
+    if not 1 <= N <= _lib.SI_MAX_N:
+        raise ValueError(f"shape_invariant_step_ supports 1 <= N <= {_lib.SI_MAX_N}, got N={N}")
+    if not float(eps) >= 0:
+        raise ValueError(f"eps must be >= 0, got {eps}")
+    split = int(split)
+    if split < 0 or split > _lib.SI_MAX_SPLIT or split & (split - 1):
+        raise ValueError(f"split must be 0 or a power of two <= {_lib.SI_MAX_SPLIT}, got {split}")
+    if any(t.data_ptr() == pc.data_ptr() for t in (ori, normal, grad)) and B:
+        raise ValueError("pc is updated in place and must not alias ori, normal or grad")
+    lib = _lib.load()
+    dev = pc.device
+    with _on(dev):
+        gnorm = torch.empty((B,), dtype=torch.float32, device=dev)
+        st = lib.pcd_si_step(*_cloud_args(pc), *_cloud_args(ori), *_cloud_args(normal), *_cloud_args(grad), B, N,
+                             float(step_size), float(step_scale), float(eps), split, gnorm.data_ptr(), _stream(dev))
+        _lib.check(st, "pcd_si_step")
+    torch.autograd.graph.increment_version(pc)      # written through its pointer: autograd must see the change
+    _launch_count += 1
+    return gnorm
+
+
+def estimate_normals(pc, k=20):
+    """Unit normals [B,N,3] of pc [B,N,3] (any strides): the eigenvector of the smallest eigenvalue of the covariance of
+    each point's k nearest neighbours, the point itself included (knn, then local_frames with skip_first=False; three
+    launches, no gradient).  It stands in for SI-Adv's get_normal_vector (open3d estimate_normals with
+    KDTreeSearchParamKNN(knn=20) on the host).  The sign of a normal and the order among neighbours at equal distance
+    are this library's, not open3d's; every consumer here is sign-free."""
+    _check_cloud(pc, "pc")
+    k = int(k)
+    if not 2 <= k <= min(pc.shape[1], _lib.KNN_MAX_K):
+        raise ValueError(f"k={k} out of range: need 2 <= k <= min(N={pc.shape[1]}, {_lib.KNN_MAX_K})")
+    x = pc.detach()
+    with torch.no_grad():
+        _, idx = knn(x, x, k)
+    return local_frames(x, idx, skip_first=False)[0]

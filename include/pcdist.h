@@ -490,6 +490,48 @@ int pcd_sample_points(int B, int N, int npoint, const int32_t *len /*[B] device,
                       int64_t *out_idx /*[B, npoint]*/, void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * One step of the SI-Adv shape-invariant attack, in place on pc: the tangent-plane gradient step and
+ * the clip of attack/SIadv/SIadv_attack.py (PointCloudAttack.shape_invariant_ifgm, with
+ * get_spin_axis_matrix, get_transformed_point_cloud and get_original_point_cloud) as one launch.
+ *
+ * pc, ori, normal, grad [B,N,3] fp32 via element strides (grad = dL/d pc).  All arithmetic is fp32
+ * with every operation rounded on its own, none contracted.  Per sample b and point i, with
+ * (x, y, z) = normal and p = the point:
+ *   1. c = (px*x + py*y) + pz*z;  t = (c*x, c*y, c*z);  q = p + t
+ *   2. spin-axis rows, den = sqrt(1 - z*z):  u0 = (y/den, -x/den, 0),
+ *      u1 = ((x*z)/den, (y*z)/den, -den),  u2 = (x, y, z);  where |z*z - 1| < 1e-4 instead
+ *      u0 = (r, -r, 0), u1 = (z/s2, z/s2, 0), u2 = (0, 0, z), r = fp32(1/sqrt 2), s2 = fp32(sqrt 2)
+ *   3. p' = U q, g' = U grad, each component (u_r0*a0 + u_r1*a1) + u_r2*a2; then g'_2 = 0
+ *      (dL/dP' = U dL/dP: the gradient restricted to the tangent plane, in the frame)
+ *   4. norm_b = sqrt(S), S = the tree sum over the points of g'_0*g'_0 + g'_1*g'_1
+ *   5. a = fp32(step_size * step_scale) (product in double); p''_r = p'_r - (a*g'_r) / (norm_b + 1e-9f)
+ *   6. p_new_r = ((u_0r*p''_0 + u_1r*p''_1) + u_2r*p''_2) - t_r      (the explicit inverse transform)
+ *   7. the clip: d = p_new - ori; per axis c, n_c = sqrt(tree sum over i of d_ic*d_ic);
+ *      s_c = min(eps / (n_c + 1e-9f), 1);  pc = ori + d*s_c
+ *      (ClipPointsLinf applied to [B,N,3] clouds, as the attack does: its "per-point" norm runs over
+ *      the N points of each axis; the per-point clip is pcd_clip_points)
+ *   8. gnorm [B] (optional, NULL when not wanted) = norm_b.
+ * Tree sum: a node covering the aligned block [k*2^l, min((k+1)*2^l, N)) is left + right, or left when
+ * the right half is empty; the leaves are the points in order.  A zero gradient gives a zero step; the
+ * point then moves only by the rounding of the round trip through its frame.
+ * A sample's outputs depend only on its own inputs and N: not on B, split or the strides.  A sample
+ * with a non-finite gradient or normal goes non-finite alone.
+ * split: 0 picks how many CTAs (a thread-block cluster, up to 8, 16 where the device schedules it)
+ * share a sample from B, N and the SM count; a power of two <= 16 forces it (testing; results do not
+ * change).  A split that leaves more than 2048 points per CTA returns PCD_ERR_ARG; 16 on a device
+ * that cannot schedule it PCD_ERR_UNSUPPORTED.
+ * Constraints: B >= 0 (0 is a no-op), N >= 1, eps >= 0, no NULL cloud; anything else returns
+ * PCD_ERR_ARG before any CUDA call.  N > PCD_SI_MAX_N returns PCD_ERR_UNSUPPORTED.
+ * Launches: one kernel; no workspace, no host synchronisation.  pc must not alias the inputs.
+ * ---------------------------------------------------------------------------------- */
+#define PCD_SI_MAX_N 16384
+
+int pcd_si_step(float *pc, int64_t sb, int64_t sp, int64_t sc, const float *ori, int64_t o_sb, int64_t o_sp,
+                int64_t o_sc, const float *normal, int64_t n_sb, int64_t n_sp, int64_t n_sc, const float *grad,
+                int64_t g_sb, int64_t g_sp, int64_t g_sc, int B, int N, double step_size, double step_scale,
+                float eps, int split, float *gnorm /*[B] or NULL*/, void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
