@@ -16,7 +16,8 @@ through the reference's own Python call surface:
     pointnet2_utils   <- model/pointnet2_utils.py (square_distance, query_ball_point)
     defense           <- attack/SIadv/baselines/defense/drop_points/SOR.py (SORDefense; float64, no install() patch)
     metrics           <- utils/dis_utils_numpy.py (float64 Chamfer / Hausdorff for reporting; no install() patch)
-    siadv             <- attack/SIadv/SIadv_attack.py (shape_invariant_ifgm as SIAdvAttack; no install() patch)
+    siadv             <- attack/SIadv/SIadv_attack.py (shape_invariant_ifgm as SIAdvAttack, shape_invariant_query_attack
+                         as SIAdvQueryAttack; no install() patch)
 
 `install.install()` patches these into an importable copy of the reference.  The package
 directory name starts with a digit; import it with importlib or through the `pcdist` alias

@@ -57,6 +57,9 @@ SIGNATURES = {
     "pcd_nn_dist64_forward": (_I, _CLOUD + _CLOUD + [_I, _I, _I, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "pcd_sample_points": (_I, [_I, _I, _I, _P, _P, _L, _c.c_uint64, _L, _P, _P, _P]),
     "pcd_si_step": (_I, [_P, _L, _L, _L] + _CLOUD * 3 + [_I, _I, _c.c_double, _c.c_double, _F, _I, _P, _P]),
+    "pcd_si_sensitivity": (_I, _CLOUD * 2 + [_I, _I, _P, _P, _P]),
+    "pcd_si_query_round": (_I, [_P, _L, _L, _I, _P] + _CLOUD * 2 + [_P, _P] + _CLOUD * 2 + [_P, _P, _I, _I, _F, _F, _I, _I,
+                                                                                          _P, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),
 }
 

@@ -15,6 +15,8 @@
 // Every operation is rounded on its own (the file is compiled with --fmad=false and uses the _rn intrinsics).
 #include <cooperative_groups.h>
 
+#include <cmath>
+
 #include "pcd_common.cuh"
 
 namespace cg = cooperative_groups;
@@ -240,6 +242,208 @@ static int launch_si(int B, int S, int T, float *pc, long long sb, long long sp,
     return PCD_OK;
 }
 
+// ------------------------------------------------------------------------------------------------------------------------
+// SI-Adv's query-based attack (shape_invariant_query_attack; pcd_si_sensitivity and pcd_si_query_round in include/pcdist.h).
+// The frames, the tangent-plane move and the clip are the step kernel's, with the same rounding.
+
+// Per point: the surrogate's gradient in the frame, its tangent length s and unit direction (one thread per point)
+__global__ void __launch_bounds__(256)
+si_sensitivity_kernel(SiCloud grd, SiCloud nrm, int B, int N, float *__restrict__ s, float *__restrict__ dir) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= (long long)B * N) return;
+    const int b = (int)(k / N), i = (int)(k - (long long)b * N);
+    float g[3], u[3][3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) g[r] = grd.at(b, i, r);
+    spin_axis(nrm.at(b, i, 0), nrm.at(b, i, 1), nrm.at(b, i, 2), u);
+    const float gx = dot3(u[0][0], u[0][1], u[0][2], g[0], g[1], g[2]);
+    const float gy = dot3(u[1][0], u[1][1], u[1][2], g[0], g[1], g[2]);
+    float v = __fsqrt_rn(__fadd_rn(__fmul_rn(gx, gx), __fmul_rn(gy, gy))), dx = 0.f, dy = 0.f;
+    if (isnan(v)) {
+        v = -1.f;                                     // ranks last and moves nothing
+    } else {
+        const float den = __fadd_rn(v, 1e-16f);
+        dx = __fdiv_rn(gx, den);
+        dy = __fdiv_rn(gy, den);
+    }
+    s[k] = v;
+    dir[2 * k] = dx;
+    dir[2 * k + 1] = dy;
+}
+
+struct SiCloudOut {
+    float *p;
+    long long sb, sp, sc;
+    __device__ __forceinline__ float &at(int b, int i, int c) const { return p[b * sb + i * sp + c * sc]; }
+};
+
+constexpr int kSqThreads = 256;
+constexpr int kSqMaxBlocks = PCD_SI_MAX_N / 32;      // 32-point block totals per axis
+enum : int { kSqIdle = 0, kSqStep = 1, kSqTake = 2, kSqDone = 4 };
+
+// Point i of the next trial before the clip: src's point, and for the chosen one the step's transform, a move of
+// sigma * a * (dx, dy) in the tangent plane and the explicit inverse transform
+__device__ __forceinline__ void sq_point(const SiCloudOut &src, const SiCloud &nrm, int b, int i, int moved, float sa,
+                                         float dx, float dy, float (&p)[3]) {
+#pragma unroll
+    for (int r = 0; r < 3; ++r) p[r] = src.at(b, i, r);
+    if (i != moved) return;
+    float n[3], u[3][3], t[3], q[3], pp[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) n[r] = nrm.at(b, i, r);
+    const float c = dot3(p[0], p[1], p[2], n[0], n[1], n[2]);
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        t[r] = __fmul_rn(c, n[r]);
+        q[r] = __fadd_rn(p[r], t[r]);
+    }
+    spin_axis(n[0], n[1], n[2], u);
+#pragma unroll
+    for (int r = 0; r < 3; ++r) pp[r] = dot3(u[r][0], u[r][1], u[r][2], q[0], q[1], q[2]);
+    pp[0] = __fadd_rn(pp[0], __fmul_rn(sa, dx));
+    pp[1] = __fadd_rn(pp[1], __fmul_rn(sa, dy));
+#pragma unroll
+    for (int r = 0; r < 3; ++r) p[r] = __fsub_rn(dot3(u[0][r], u[1][r], u[2][r], pp[0], pp[1], pp[2]), t[r]);
+}
+
+// One CTA per sample.  Warp 0 scores the logits row and lane 0 makes the decision; then the CTA writes the next trial.
+// Thread t owns points t, t + T, ...: a warp's 32 consecutive points are summed by the lane butterfly, the 32-point
+// block totals by an in-place aligned tree in shared memory, so the clip's norms follow the fixed tree of pcd_si_step.
+__global__ void __launch_bounds__(kSqThreads)
+si_query_round_kernel(const float *__restrict__ logits, long long l_sb, long long l_sc, int C,
+                      const long long *__restrict__ target, SiCloud ori, SiCloud nrm, const int *__restrict__ order,
+                      const float *__restrict__ dir, SiCloudOut cloud, SiCloudOut trial, int *__restrict__ state,
+                      float *__restrict__ best, int N, float a, float eps, int max_query, int targeted,
+                      int *__restrict__ active) {
+    __shared__ int dec[3];                            // mode, moved point, sigma of the next trial
+    __shared__ float tot[3][kSqMaxBlocks];
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, T = blockDim.x;
+    if (tid < 32) {
+        int *st = state + 4 * (long long)b;
+        int mode = kSqIdle, moved = -1, sigma = st[0];
+        if (st[3] == 0) {
+            const long long y = target[b];
+            const bool y_ok = y >= 0 && y < C;
+            const float *row = logits + b * l_sb;
+            bool nan = false;
+            float other = -10000.f, top = -INFINITY;  // other: the max of (1 - onehot) * logits - onehot * 10000
+            int arg = 0x7fffffff;
+            for (int j = lane; j < C; j += 32) {
+                const float v = row[j * l_sc];
+                nan |= isnan(v);
+                if (j != y) other = fmaxf(other, v);
+                if (v > top) top = v, arg = j;
+            }
+#pragma unroll
+            for (int o = 1; o < 32; o *= 2) {         // max and first arg-max are exact: any combining order agrees
+                nan |= __shfl_xor_sync(0xffffffffu, (int)nan, o) != 0;
+                other = fmaxf(other, __shfl_xor_sync(0xffffffffu, other, o));
+                const float tv = __shfl_xor_sync(0xffffffffu, top, o);
+                const int ta = __shfl_xor_sync(0xffffffffu, arg, o);
+                if (tv > top || (tv == top && ta < arg)) top = tv, arg = ta;
+            }
+            if (lane == 0) {
+                const float real = y_ok ? row[y * l_sc] : 0.f;
+                const float margin = targeted ? __fsub_rn(other, real) : __fsub_rn(real, other);
+                const bool valid = y_ok && !nan && isfinite(margin);
+                const bool success = valid && (targeted ? arg == y : arg != y);
+                int cur = st[1], q = st[2] + 1, status = 0;
+                bool take = false;
+                if (q == 1) {                         // round 0: the trial is the cloud itself
+                    best[b] = margin;
+                    if (success) status = 1, take = true;
+                } else if (success) {
+                    status = 1, take = true;
+                } else if (valid && margin < best[b]) {
+                    best[b] = margin;
+                    take = true, cur += 1, sigma = -1;
+                } else if (sigma == -1) {
+                    sigma = 1;
+                } else {
+                    cur += 1, sigma = -1;
+                }
+                if (status == 0 && q >= max_query) status = 2;
+                st[0] = sigma, st[1] = cur, st[2] = q, st[3] = status;
+                if (status != 0 && active) atomicSub(active, 1);
+                mode = (take ? kSqTake : 0) | (status != 0 ? kSqDone : kSqStep);
+                if (status == 0) {
+                    moved = order[(long long)b * N + (int)((unsigned)cur % (unsigned)N)];
+                    if (moved < 0 || moved >= N) moved = -1;
+                }
+                dec[0] = mode, dec[1] = moved, dec[2] = sigma;
+            }
+        } else if (lane == 0) {
+            dec[0] = kSqIdle;
+        }
+    }
+    __syncthreads();
+    const int mode = dec[0], moved = dec[1];
+    if (mode == kSqIdle) return;
+    const SiCloudOut src = (mode & kSqTake) ? trial : cloud;
+    if (mode & kSqDone) {                             // the sample ends here: its trial and its cloud become equal
+        const SiCloudOut dst = (mode & kSqTake) ? cloud : trial;
+        for (int i = tid; i < N; i += T) {
+#pragma unroll
+            for (int r = 0; r < 3; ++r) dst.at(b, i, r) = src.at(b, i, r);
+        }
+        return;
+    }
+    float dx = 0.f, dy = 0.f;
+    if (moved >= 0) {
+        dx = dir[2 * ((long long)b * N + moved)];
+        dy = dir[2 * ((long long)b * N + moved) + 1];
+    }
+    const float sa = __fmul_rn((float)dec[2], a);
+    const int nb = (N + 31) / 32, W = T / 32, warp = tid >> 5;
+    int nbp = 1;
+    while (nbp < nb) nbp *= 2;
+    for (int m = warp; m < nb; m += W) {
+        const int i = m * 32 + lane;
+        float sq[3] = {0.f, 0.f, 0.f};
+        if (i < N) {
+            float p[3];
+            sq_point(src, nrm, b, i, moved, sa, dx, dy, p);
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                const float d = __fsub_rn(p[r], ori.at(b, i, r));
+                sq[r] = __fmul_rn(d, d);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 3; ++r) sq[r] = tree_warp(sq[r]);
+        if (lane == 0) {
+#pragma unroll
+            for (int r = 0; r < 3; ++r) tot[r][m] = sq[r];
+        }
+    }
+    for (int m = nb + tid; m < nbp; m += T) tot[0][m] = tot[1][m] = tot[2][m] = 0.f;
+    __syncthreads();
+    for (int w = 1; w < nbp; w *= 2) {
+        for (int m = tid * 2 * w; m < nbp; m += T * 2 * w) {
+#pragma unroll
+            for (int r = 0; r < 3; ++r) tot[r][m] = __fadd_rn(tot[r][m], tot[r][m + w]);
+        }
+        __syncthreads();
+    }
+    float scale[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const float s = __fdiv_rn(eps, __fadd_rn(__fsqrt_rn(tot[r][0]), 1e-9f));
+        scale[r] = s > 1.f ? 1.f : s;                // NaN stays NaN
+    }
+    // the same points as above, in the same threads: a thread reads src before it writes trial or cloud there
+    for (int i = tid; i < N; i += T) {
+        float p[3];
+        sq_point(src, nrm, b, i, moved, sa, dx, dy, p);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            const float o = ori.at(b, i, r);
+            if (mode & kSqTake) cloud.at(b, i, r) = src.at(b, i, r);
+            trial.at(b, i, r) = __fadd_rn(o, __fmul_rn(__fsub_rn(p[r], o), scale[r]));
+        }
+    }
+}
+
 }  // namespace pcd
 
 using namespace pcd;
@@ -288,4 +492,51 @@ extern "C" int pcd_si_step(float *pc, int64_t sb, int64_t sp, int64_t sc, const 
     case 4: return launch_si<4>(B, S, T, pc, sb, sp, sc, o, n, g, N, a, eps, gnorm, st);
     default: return launch_si<8>(B, S, T, pc, sb, sp, sc, o, n, g, N, a, eps, gnorm, st);
     }
+}
+
+extern "C" int pcd_si_sensitivity(const float *grad, int64_t g_sb, int64_t g_sp, int64_t g_sc, const float *normal,
+                                  int64_t n_sb, int64_t n_sp, int64_t n_sc, int B, int N, float *s, float *dir,
+                                  void *stream) {
+    if (B < 0 || N < 1 || (B > 0 && (!grad || !normal || !s || !dir))) {
+        set_error("pcd_si_sensitivity: bad argument (need B >= 0, N >= 1, no NULL pointer) B=%d N=%d", B, N);
+        return PCD_ERR_ARG;
+    }
+    if (B == 0) return PCD_OK;
+    const long long total = (long long)B * N;
+    si_sensitivity_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        SiCloud{grad, g_sb, g_sp, g_sc}, SiCloud{normal, n_sb, n_sp, n_sc}, B, N, s, dir);
+    PCD_CUDA_CHECK(cudaGetLastError());
+    return PCD_OK;
+}
+
+extern "C" int pcd_si_query_round(const float *logits, int64_t l_sb, int64_t l_sc, int C, const int64_t *target,
+                                  const float *ori, int64_t o_sb, int64_t o_sp, int64_t o_sc, const float *normal,
+                                  int64_t n_sb, int64_t n_sp, int64_t n_sc, const int32_t *order, const float *dir,
+                                  float *cloud, int64_t c_sb, int64_t c_sp, int64_t c_sc, float *trial, int64_t t_sb,
+                                  int64_t t_sp, int64_t t_sc, int32_t *state, float *best, int B, int N,
+                                  float step_size, float eps, int max_query, int targeted, int32_t *active,
+                                  void *stream) {
+    if (B < 0 || N < 1 || C < 2 || !std::isfinite(step_size) || !(eps >= 0.f) || max_query < 1 ||
+        (targeted != 0 && targeted != 1) ||
+        (B > 0 && (!logits || !target || !ori || !normal || !order || !dir || !cloud || !trial || !state || !best ||
+                   cloud == trial))) {
+        set_error("pcd_si_query_round: bad argument (need B >= 0, N >= 1, C >= 2, finite step_size, eps >= 0, "
+                  "max_query >= 1, targeted 0 or 1, no NULL pointer but active, cloud != trial) B=%d N=%d C=%d "
+                  "step_size=%g eps=%g max_query=%d targeted=%d",
+                  B, N, C, (double)step_size, (double)eps, max_query, targeted);
+        return PCD_ERR_ARG;
+    }
+    if (N > PCD_SI_MAX_N) {
+        set_error("pcd_si_query_round: N = %d exceeds %d points per sample", N, PCD_SI_MAX_N);
+        return PCD_ERR_UNSUPPORTED;
+    }
+    if (B == 0) return PCD_OK;
+    int T = 32;                                      // one warp per 32 points, at most kSqThreads threads
+    while (T < kSqThreads && T < N) T *= 2;
+    si_query_round_kernel<<<(unsigned)B, T, 0, (cudaStream_t)stream>>>(
+        logits, l_sb, l_sc, C, (const long long *)target, SiCloud{ori, o_sb, o_sp, o_sc},
+        SiCloud{normal, n_sb, n_sp, n_sc}, order, dir, SiCloudOut{cloud, c_sb, c_sp, c_sc},
+        SiCloudOut{trial, t_sb, t_sp, t_sc}, state, best, N, step_size, eps, max_query, targeted, active);
+    PCD_CUDA_CHECK(cudaGetLastError());
+    return PCD_OK;
 }

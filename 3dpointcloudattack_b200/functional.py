@@ -19,7 +19,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
            "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "sample_points", "PointSampler", "nn_dist64", "NNDist64Result",
-           "shape_invariant_step_", "estimate_normals", "SI_STEP_SCALE",
+           "shape_invariant_step_", "estimate_normals", "SI_STEP_SCALE", "si_sensitivity", "si_query_round_",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -954,3 +954,78 @@ def estimate_normals(pc, k=20):
     with torch.no_grad():
         _, idx = knn(x, x, k)
     return local_frames(x, idx, skip_first=False)[0]
+
+
+# ------------------------------------------------ SI-Adv's query-based attack: the sensitivity map and one query round
+def si_sensitivity(grad, normal):
+    """The sensitivity map of SI-Adv's query-based attack (pcd_si_sensitivity in include/pcdist.h): grad (a surrogate's
+    dL/d cloud) and normal [B,N,3] fp32 (any strides) -> (order int32 [B,N]: the points by descending tangent-gradient
+    length, ties by the lower index; dir [B,N,2]: the unit tangent direction of each point's gradient in its frame).
+    A point whose length is NaN ranks last with dir (0, 0).  One launch, then a stable torch.sort; no gradient."""
+    global _launch_count
+    for t, name in ((grad, "grad"), (normal, "normal")):
+        _check_cloud(t, name)
+    if normal.shape != grad.shape or normal.device != grad.device:
+        raise ValueError(f"normal {tuple(normal.shape)} on {normal.device} does not match grad {tuple(grad.shape)} on "
+                         f"{grad.device}")
+    B, N, _ = grad.shape
+    if N < 1:
+        raise ValueError("si_sensitivity needs N >= 1")
+    lib = _lib.load()
+    dev = grad.device
+    with _on(dev):
+        s = torch.empty((B, N), dtype=torch.float32, device=dev)
+        dir = torch.empty((B, N, 2), dtype=torch.float32, device=dev)
+        st = lib.pcd_si_sensitivity(*_cloud_args(grad.detach()), *_cloud_args(normal.detach()), B, N, s.data_ptr(),
+                                    dir.data_ptr(), _stream(dev))
+        _lib.check(st, "pcd_si_sensitivity")
+        order = torch.sort(s, dim=1, descending=True, stable=True)[1].to(torch.int32)
+    _launch_count += 1
+    return order, dir
+
+
+def si_query_round_(logits, target, ori, normal, order, dir, cloud, trial, state, best, step_size, eps, max_query,
+                    targeted=False, active=None):
+    """One round of SI-Adv's query-based attack for every sample, IN PLACE on cloud, trial, state, best and active
+    (pcd_si_query_round in include/pcdist.h), after the black box has scored the trials: logits [B,C] fp32 (any
+    strides, C >= 2), target [B] int64.  Each active sample takes or rejects its trial, and the next trial moves one point
+    of the cloud by +-step_size in its tangent plane, clipped to eps.
+    ori, normal, cloud, trial [B,N,3] fp32 (any strides); order int32 [B,N] and dir [B,N,2] from si_sensitivity;
+    state int32 [B,4] = (sigma, cursor, queries, status: 0 active, 1 success, 2 failed), best [B] fp32; active: None or
+    an int32 [1] tensor that every sample ending in this round decrements.  One launch, no host synchronisation."""
+    global _launch_count
+    for t, name in ((ori, "ori"), (normal, "normal"), (cloud, "cloud"), (trial, "trial")):
+        _check_cloud(t, name)
+        if t.shape != ori.shape or t.device != ori.device:
+            raise ValueError(f"{name} {tuple(t.shape)} on {t.device} does not match ori {tuple(ori.shape)} on {ori.device}")
+    B, N, _ = ori.shape
+    dev = ori.device
+    if not 1 <= N <= _lib.SI_MAX_N:
+        raise ValueError(f"si_query_round_ supports 1 <= N <= {_lib.SI_MAX_N}, got N={N}")
+    if not isinstance(logits, torch.Tensor) or logits.dim() != 2 or logits.shape[0] != B or logits.shape[1] < 2 \
+            or logits.dtype != torch.float32 or logits.device != dev:
+        raise ValueError(f"logits must be float32 [{B}, C >= 2] on {dev}, got {logits!r:.80}")
+    for t, name, shape, dtype in ((target, "target", (B,), torch.int64), (order, "order", (B, N), torch.int32),
+                                  (dir, "dir", (B, N, 2), torch.float32), (state, "state", (B, 4), torch.int32),
+                                  (best, "best", (B,), torch.float32)):
+        if not isinstance(t, torch.Tensor) or tuple(t.shape) != shape or t.dtype != dtype or t.device != dev \
+                or not t.is_contiguous():
+            raise ValueError(f"{name} must be a contiguous {dtype} tensor {shape} on {dev}, got {t!r:.80}")
+    if active is not None and (not isinstance(active, torch.Tensor) or active.dtype != torch.int32
+                               or active.numel() != 1 or active.device != dev):
+        raise ValueError(f"active must be None or an int32 tensor of one element on {dev}")
+    if not math.isfinite(float(step_size)) or not float(eps) >= 0 or int(max_query) < 1:
+        raise ValueError(f"need a finite step_size, eps >= 0 and max_query >= 1, got {step_size}, {eps}, {max_query}")
+    if cloud.data_ptr() == trial.data_ptr() and B:
+        raise ValueError("cloud and trial must not be the same memory")
+    lib = _lib.load()
+    with _on(dev):
+        st = lib.pcd_si_query_round(logits.data_ptr(), logits.stride(0), logits.stride(1), logits.shape[1],
+                                    target.data_ptr(), *_cloud_args(ori), *_cloud_args(normal), order.data_ptr(),
+                                    dir.data_ptr(), *_cloud_args(cloud), *_cloud_args(trial), state.data_ptr(),
+                                    best.data_ptr(), B, N, float(step_size), float(eps), int(max_query), int(bool(targeted)),
+                                    _ptr(active), _stream(dev))
+        _lib.check(st, "pcd_si_query_round")
+    for t in (cloud, trial, state, best) + (() if active is None else (active,)):
+        torch.autograd.graph.increment_version(t)      # written through its pointer: autograd must see the change
+    _launch_count += 1

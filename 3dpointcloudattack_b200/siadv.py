@@ -12,14 +12,19 @@ One whole iteration can be captured into a CUDA graph and replayed (`use_graph=T
 
 Defences come in through the model: DefendedVictim(victim, SRSDefense / SORDefense(..., sampler=PointSampler(...)))
 is the reference's wb_classifier(pre_head(points)), and eval_model plays its black-box classifier in transfer runs.
+SI-Adv's query-based black-box attack (shape_invariant_query_attack) is SIAdvQueryAttack: B clouds are queried
+together, and one query round is a no-grad forward of the black box on the B trial clouds plus ONE library launch
+(functional.si_query_round_), which scores the logits, makes every sample's accept / reject decision and builds every
+sample's next trial.  Only a periodic stop check reads back to the host.
+
 There is no install() patch for this module: the class layout of PointCloudAttack is not recorded here, as for
-defense.py.  The query-based attack (shape_invariant_query_attack) is not restated.
+defense.py.
 """
 import torch
 
 from . import functional as F
 
-__all__ = ["SIAdvAttack"]
+__all__ = ["SIAdvAttack", "SIAdvQueryAttack"]
 
 
 def _samplers(model):
@@ -81,11 +86,7 @@ class SIAdvAttack:
             raise ValueError(f"points must be [B, N, 3] or [B, N, 6], got {tuple(points.shape)}")
         data = points.detach().float()
         ori = data[..., :3].contiguous()
-        if data.shape[2] == 6:
-            n = data[..., 3:]
-            normal = (n / torch.sqrt(torch.sum(n * n, dim=-1, keepdim=True))).contiguous()
-        else:
-            normal = F.estimate_normals(ori, self.knn)
+        normal = _unit_normals(data, self.knn)
         st = {"ori": ori, "pc": ori.clone(), "normal": normal, "target": target.long().to(dev),
               "loss": torch.zeros((), device=dev)}
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -125,6 +126,124 @@ class SIAdvAttack:
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, stream=side):
             self._iteration(st)
+        for k, v in saved.items():
+            st[k].copy_(v)
+        for s, c in zip(samplers, counters):
+            s.state.copy_(c)
+        return g
+
+
+def _unit_normals(data, knn):
+    """the normals of [B,N,6] input (channels 3:6, normalised), else estimate_normals of the cloud"""
+    if data.shape[2] == 6:
+        n = data[..., 3:]
+        return (n / torch.sqrt(torch.sum(n * n, dim=-1, keepdim=True))).contiguous()
+    return F.estimate_normals(data[..., :3].contiguous(), knn)
+
+
+class SIAdvQueryAttack:
+    """SI-Adv's query-based black-box attack (shape_invariant_query_attack) for batches.  This restates the published
+    algorithm and is not pinned against the reference's code, which is not recorded here (as defense.SRSDefense):
+      1. normals as SIAdvAttack takes them, once, on the clean cloud; U_i = the spin-axis frame of pcd_si_step;
+      2. the sensitivity map, once: G = d sum_b margin(surrogate(ori)) / d ori (margin: the C&W margin of
+         SIAdvAttack._loss without the clamp); per point the tangent length s_i = |(U_i G_i)_xy| and its direction; the
+         points ranked by descending s (functional.si_sensitivity);
+      3. query rounds: round 0 scores the clean cloud; afterwards the trial moves the point at the cursor by -step_size,
+         then +step_size, along its direction in its tangent plane, and clips the cloud to eps as the step does.  A trial
+         that fools the black box ends the sample; one that lowers the margin is kept and the cursor moves on; after
+         both signs fail the cursor moves on (functional.si_query_round_, include/pcdist.h for the exact rules).
+    A sample ends on success or after max_query queries.  step_size = 0.05 is this library's default: the reference's
+    value is not recorded here.  model is the black box and runs only under no_grad; surrogate (default: model) gives
+    the gradient in one forward and one backward; neither gets a .grad.  Defences come in through the model, e.g.
+    DefendedVictim with a device-sampled SRS or SOR.  The host reads the active count every check_every rounds and
+    stops when it is 0; with use_graph=True one round is captured and replayed.  A sample's result depends only on its
+    own inputs (given a black box whose logits for a cloud do not depend on the batch), so sharding needs no extra code."""
+
+    def __init__(self, model, surrogate=None, eps=0.16, step_size=0.05, max_query=2000, knn=20, targeted=False,
+                 check_every=50, use_graph=False):
+        self.model = model.eval()
+        self.surrogate = surrogate.eval() if surrogate is not None else None
+        self.eps, self.step_size, self.max_query = float(eps), float(step_size), int(max_query)
+        self.knn, self.targeted, self.check_every, self.use_graph = int(knn), bool(targeted), int(check_every), bool(use_graph)
+        if self.max_query < 1 or self.check_every < 1:
+            raise ValueError(f"max_query and check_every must be >= 1, got {max_query}, {check_every}")
+        self.rounds = 0                          # query rounds run by the last attack()
+        self.loop_ms = 0.0                       # device time of those rounds
+
+    def _margin(self, logits, target):
+        one_hot = torch.zeros_like(logits).scatter_(1, target.view(-1, 1), 1.)
+        real = torch.sum(one_hot * logits, dim=1)
+        other = torch.max((1. - one_hot) * logits - one_hot * 10000., dim=1)[0]
+        return other - real if self.targeted else real - other
+
+    def _round(self, st):
+        with torch.no_grad():
+            logits = self.model(st["trial"].transpose(1, 2))[0]
+            if logits.dtype != torch.float32:
+                logits = logits.float()
+            F.si_query_round_(logits, st["target"], st["ori"], st["normal"], st["order"], st["dir"], st["cloud"],
+                              st["trial"], st["state"], st["best"], self.step_size, self.eps, self.max_query,
+                              self.targeted, st["active"])
+
+    def attack(self, points, target):
+        """points [B,N,3] (or [B,N,6] with normals in channels 3:6), target [B] ->
+        (adv [B,N,3], pred [B] = argmax of the black box on adv (one more forward, not counted), success [B] (the
+        query that ended the sample fooled the black box), queries [B] int64)"""
+        dev = points.device
+        if dev.type != "cuda":
+            raise RuntimeError("SIAdvQueryAttack runs on CUDA only")
+        if points.dim() != 3 or points.shape[2] not in (3, 6):
+            raise ValueError(f"points must be [B, N, 3] or [B, N, 6], got {tuple(points.shape)}")
+        data = points.detach().float()
+        ori = data[..., :3].contiguous()
+        normal = _unit_normals(data, self.knn)
+        target = target.long().to(dev).contiguous()
+        B = ori.shape[0]
+        surrogate = self.model if self.surrogate is None else self.surrogate
+        with torch.enable_grad():
+            x = ori.clone().requires_grad_(True)
+            grad, = torch.autograd.grad(self._margin(surrogate(x.transpose(1, 2))[0], target).sum(), x)
+        order, dir = F.si_sensitivity(grad, normal)
+        st = {"ori": ori, "normal": normal, "target": target, "order": order, "dir": dir, "cloud": ori.clone(),
+              "trial": ori.clone(), "state": torch.tensor([[-1, 0, 0, 0]], dtype=torch.int32, device=dev).repeat(B, 1),
+              "best": torch.zeros(B, device=dev), "active": torch.full((1,), B, dtype=torch.int32, device=dev)}
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        graph = self._capture(st) if self.use_graph else None
+        e0.record()
+        self.rounds = 0
+        while self.rounds < self.max_query:
+            if graph is not None:
+                graph.replay()
+            else:
+                self._round(st)
+            self.rounds += 1
+            if self.rounds % self.check_every == 0 and self.rounds < self.max_query and int(st["active"].item()) == 0:
+                break
+        e1.record()
+        with torch.no_grad():
+            pred = torch.argmax(self.model(st["cloud"].transpose(1, 2))[0], dim=1)
+        torch.cuda.synchronize(dev)
+        self.loop_ms = e0.elapsed_time(e1)
+        return st["cloud"], pred, st["state"][:, 3] == 1, st["state"][:, 2].long()
+
+    def _capture(self, st, warmup=3):
+        """Capture one round.  The warm-up rounds run on the real state (the graph records its addresses), so the
+        clouds, the decision state and the draw counters of any device-sampled defence are saved before and restored
+        after: replaying k times is exactly k rounds."""
+        saved = {k: st[k].clone() for k in ("cloud", "trial", "state", "best", "active")}
+        samplers = _samplers(self.model)
+        counters = [s.state.clone() for s in samplers]
+        cur = torch.cuda.current_stream()
+        side = torch.cuda.Stream()
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            for _ in range(warmup):
+                self._round(st)
+        cur.wait_stream(side)
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, stream=side):
+            self._round(st)
         for k, v in saved.items():
             st[k].copy_(v)
         for s, c in zip(samplers, counters):

@@ -532,6 +532,62 @@ int pcd_si_step(float *pc, int64_t sb, int64_t sp, int64_t sc, const float *ori,
                 float eps, int split, float *gnorm /*[B] or NULL*/, void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * SI-Adv's query-based attack (attack/SIadv/SIadv_attack.py, shape_invariant_query_attack), restated
+ * from the published algorithm: a sensitivity map from a surrogate's gradient in every point's tangent
+ * plane, then SimBA-style trials of -step and +step at the most sensitive points, each scored by one
+ * query of the black box.  Frames, rounding and the clip are those of pcd_si_step.
+ *
+ * pcd_si_sensitivity: grad (the surrogate's dL/d ori), normal [B,N,3] fp32 via element strides.  Per
+ * point, with U the spin-axis rows of pcd_si_step step 2:  g'x, g'y = rows 0 and 1 of U grad (step 3's
+ * rows product);  s = sqrt(g'x*g'x + g'y*g'y);  dir = (g'x / (s + 1e-16f), g'y / (s + 1e-16f)).
+ * A NaN s is stored as -1 with dir (0, 0): such points rank last and move nothing.
+ * s [B,N] and dir [B,N,2] are contiguous outputs.  One launch.  B >= 0 (0 is a no-op), N >= 1, no
+ * NULL pointer, else PCD_ERR_ARG before any CUDA call.  The caller ranks the points by descending s,
+ * ties by the lower index (a stable sort).
+ *
+ * pcd_si_query_round: one query round of every sample, after the black box has scored the trials.
+ *   logits [B,C] fp32 via element strides (C >= 2), target [B] int64, ori / normal [B,N,3] (any
+ *   strides), order [B,N] int32 and dir [B,N,2] contiguous (pcd_si_sensitivity's ranking); in/out:
+ *   cloud (the current cloud P) and trial [B,N,3] (any strides, not the same memory), state [B,4]
+ *   int32 contiguous = (sigma, cursor, queries, status), best [B] fp32.  status: 0 active, 1 success,
+ *   2 failed.  The caller starts every sample at cloud = trial = ori, state = (-1, 0, 0, 0).
+ *   Scoring a row: other = max(max over j != y of logits_j, -10000) (the max of (1 - onehot)*logits -
+ *   onehot*10000), real = logits_y;  margin = real - other, or other - real when targeted;  the first
+ *   arg-max decides success (!= y, or == y when targeted).  A row with a NaN, a non-finite margin or
+ *   y outside [0, C) is neither a success nor an improvement.
+ *   An active sample (others are left alone): q = queries + 1, then
+ *     q == 1 (round 0, the trial is the cloud):  best = margin;  success -> status 1
+ *     success                                   -> cloud = trial, status 1
+ *     margin < best                             -> cloud = trial, best = margin, cursor += 1, sigma = -1
+ *     sigma == -1                               -> sigma = +1 (the same point again)
+ *     otherwise                                 -> cursor += 1, sigma = -1
+ *   and q >= max_query leaves an active sample failed (status 2).  A sample that ends in this round gets
+ *   trial = cloud.  One that goes on gets its next trial: point i = order[cursor mod N] of the cloud moved
+ *   by the step's transform (pcd_si_step steps 1-3), pp_0 += (sigma*a)*dir_x, pp_1 += (sigma*a)*dir_y,
+ *   a = step_size, and the inverse transform (step 6); every other point copied; then the whole cloud
+ *   clipped as in pcd_si_step step 7 (per-axis norms of trial - ori over the fixed tree, eps).  An order
+ *   entry outside [0, N) moves no point.
+ *   active (optional, NULL when not wanted): every sample that leaves the active status in this round
+ *   subtracts 1 from *active, so a caller that sets it to B before the first round reads the number of
+ *   active samples there.
+ *   A sample's bits depend only on its own inputs and N: not on B, C, strides or the launch geometry.
+ *   Constraints: B >= 0 (0 is a no-op), N >= 1, C >= 2, finite step_size, eps >= 0, max_query >= 1,
+ *   targeted 0 or 1, no NULL pointer but active, cloud != trial; anything else returns PCD_ERR_ARG before
+ *   any CUDA call.  N > PCD_SI_MAX_N returns PCD_ERR_UNSUPPORTED.
+ *   Launches: one kernel (one CTA per sample); no workspace, no host synchronisation.
+ * ---------------------------------------------------------------------------------- */
+int pcd_si_sensitivity(const float *grad, int64_t g_sb, int64_t g_sp, int64_t g_sc, const float *normal,
+                       int64_t n_sb, int64_t n_sp, int64_t n_sc, int B, int N, float *s /*[B,N]*/,
+                       float *dir /*[B,N,2]*/, void *stream);
+
+int pcd_si_query_round(const float *logits, int64_t l_sb, int64_t l_sc, int C, const int64_t *target,
+                       const float *ori, int64_t o_sb, int64_t o_sp, int64_t o_sc, const float *normal,
+                       int64_t n_sb, int64_t n_sp, int64_t n_sc, const int32_t *order, const float *dir,
+                       float *cloud, int64_t c_sb, int64_t c_sp, int64_t c_sc, float *trial, int64_t t_sb,
+                       int64_t t_sp, int64_t t_sc, int32_t *state, float *best, int B, int N, float step_size,
+                       float eps, int max_query, int targeted, int32_t *active /*or NULL*/, void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
