@@ -10,7 +10,8 @@ through the reference's own Python call surface:
     knn_utils         <- attack/GeoA3/knn_utils.py
     loss_utils        <- attack/GeoA3/loss_utils.py (the knn_points consumers and the brute-force k-NN losses)
     utility           <- attack/GeoA3/utility.py (estimate_normal, estimate_perpendicular, ...)
-    taof              <- attack/AOF/TAOF_attack.py (knn, get_Laplace_from_pc)
+    taof              <- attack/AOF/TAOF_attack.py (knn, get_Laplace_from_pc; the AOF attack as AOFAttack, with
+                         low_frequency_basis and functional.low_pass; no install() patch for the attack)
     dgcnn             <- model/dgcnn.py (knn, get_graph_feature)
     curvenet_util     <- model/curvenet_util.py (knn, normal_knn)
     pointnet2_utils   <- model/pointnet2_utils.py (square_distance, query_ball_point)

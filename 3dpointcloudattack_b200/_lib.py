@@ -17,6 +17,7 @@ KNN_MAX_K, KNN_MAX_C = 64, 128
 SOR_MAX_K = 15
 SAMPLE_MAX_N = 16384
 SI_MAX_N, SI_MAX_SPLIT = 16384, 16
+LP_MAX_N, LP_MAX_SPLIT = 16384, 16
 EDGE_CENTER, EDGE_NEIGHBOR, EDGE_DIFF = 0, 1, 2
 
 _c = ctypes
@@ -60,6 +61,7 @@ SIGNATURES = {
     "pcd_si_sensitivity": (_I, _CLOUD * 2 + [_I, _I, _P, _P, _P]),
     "pcd_si_query_round": (_I, [_P, _L, _L, _I, _P] + _CLOUD * 2 + [_P, _P] + _CLOUD * 2 + [_P, _P, _I, _I, _F, _F, _I, _I,
                                                                                           _P, _P]),
+    "pcd_low_pass": (_I, [_P, _L, _I] + _CLOUD + [_I, _I] + _CLOUD + [_I, _P]),
     "pcd_fp32_probe_launch": (_I, [_I, _I, _P, _c.POINTER(_c.c_double), _P]),
 }
 

@@ -95,10 +95,16 @@ class CWAttack:
         self.use_graph = use_graph
         self.loop_ms = 0.0                        # device time spent in the iteration loops of the last attack()
 
+    def _victim(self, adv, target):
+        """the victim's forward: (logits of adv [B, classes], which tracking and success use; the adversarial term summed
+        over the batch).  AOFAttack overrides it."""
+        logits = self.model(adv)[0]
+        return logits, self.adv_func(logits, target, reduce=False).sum()
+
     # one optimisation iteration on the state tensors (all updates in place -> graph capturable)
     def _iteration(self, st):
         adv, ori, target = st["adv"], st["ori"], st["target"]
-        logits = self.model(adv)[0]
+        logits, adv_sum = self._victim(adv, target)
         pred = torch.argmax(logits, dim=1)
         with torch.no_grad():
             dist_val = torch.sqrt(torch.sum((adv - ori) ** 2, dim=[1, 2]))
@@ -113,7 +119,7 @@ class CWAttack:
             st["o_bestattack"].copy_(torch.where(o_better[:, None, None], adv, st["o_bestattack"]))
         B = adv.shape[0]
         denom = float(self.global_batch or B)
-        adv_loss = self.adv_func(logits, target, reduce=False).sum() / denom
+        adv_loss = adv_sum / denom
         dist_loss = self.dist_func(adv.transpose(1, 2), ori.transpose(1, 2), st["weight"], batch_avg=False).sum() / denom
         loss = adv_loss + dist_loss
         st["opt"].zero_grad(set_to_none=False)

@@ -1,6 +1,6 @@
 """Drop-in for the point-set distance wrappers of attack/CW/CW_utils/dist_utils.py (copies:
 attack/Gen3DAdv/utils/dist_utils.py, attack/SIadv/baselines/attack/util/dist_utils.py):
-ChamferDist, HausdorffDist, KNNDist, ChamferkNNDist -- same constructor / forward signatures.
+L2Dist, ChamferDist, HausdorffDist, KNNDist, ChamferkNNDist -- same constructor / forward signatures.
 
 Differences that do not change results: `weights` is moved to the input's device instead of
 the hard-coded `.cuda()` (dist_utils.py:68,105,156), so one process per GPU works unchanged.
@@ -16,6 +16,19 @@ def _weights(weights, B, device):
     if weights is None:
         return torch.ones((B,), device=device)
     return torch.as_tensor(weights).float().to(device)
+
+
+class L2Dist(nn.Module):
+    """dist_utils.py:9-35: per sample sqrt(sum((adv - ori)^2)) over the points and channels, times weights; the distance
+    AOF runs with.  Either layout ([B, K, 3] or [B, 3, K]) as long as both clouds share it."""
+
+    def forward(self, adv_pc, ori_pc, weights=None, batch_avg=True):
+        B = adv_pc.shape[0]
+        dist = torch.sqrt(torch.sum((adv_pc - ori_pc) ** 2, dim=[1, 2]))
+        dist = dist * _weights(weights, B, adv_pc.device)
+        if batch_avg:
+            return dist.mean()
+        return dist
 
 
 class _SetDist(nn.Module):

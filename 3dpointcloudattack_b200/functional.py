@@ -19,7 +19,7 @@ from ._lib import (EDGE_CENTER, EDGE_DIFF, EDGE_NEIGHBOR, FORM_COL_ROW, FORM_ROW
 
 __all__ = ["nn1", "NN1Result", "time_next_sweep", "clear_cache", "knn", "ball_query", "edge_feature", "deterministic_edge_backward", "clip_points_", "lp_clip", "offset_proj", "find_offset", "farthest_point_sample", "fp32_peak_flops",
            "local_frames", "kappa", "graph_laplacian", "knn_outlier_loss", "sor", "SORResult", "sample_points", "PointSampler", "nn_dist64", "NNDist64Result",
-           "shape_invariant_step_", "estimate_normals", "SI_STEP_SCALE", "si_sensitivity", "si_query_round_",
+           "shape_invariant_step_", "estimate_normals", "SI_STEP_SCALE", "si_sensitivity", "si_query_round_", "low_pass",
            "EDGE_CENTER", "EDGE_NEIGHBOR", "EDGE_DIFF",
            "FORM_ROW_COL", "FORM_COL_ROW", "FORM_SUM_FIRST", "NORM_MULSUM", "NORM_FMA",
            "VALUE_SQUARED", "VALUE_SQRT_CLAMP"]
@@ -1029,3 +1029,55 @@ def si_query_round_(logits, target, ori, normal, order, dir, cloud, trial, state
     for t in (cloud, trial, state, best) + (() if active is None else (active,)):
         torch.autograd.graph.increment_version(t)      # written through its pointer: autograd must see the change
     _launch_count += 1
+
+
+# ------------------------------------------------ AOF's low-frequency projection
+def _low_pass_launch(basis, x, split):
+    global _launch_count
+    lib = _lib.load()
+    B, N, _ = x.shape
+    dev = x.device
+    with _on(dev):
+        y = torch.empty_like(x)                      # x's layout: [B,N,3] or a transposed [B,3,N]
+        st = lib.pcd_low_pass(basis.data_ptr(), basis.stride(0), basis.shape[1], *_cloud_args(x), B, N, *_cloud_args(y),
+                              split, _stream(dev))
+        _lib.check(st, "pcd_low_pass")
+    _launch_count += 1
+    return y
+
+
+class _LowPass(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, basis, split):
+        ctx.save_for_backward(basis)
+        ctx.split = split
+        return _low_pass_launch(basis, x.detach(), split)
+
+    @staticmethod
+    def backward(ctx, g):
+        basis, = ctx.saved_tensors
+        return _low_pass_launch(basis, g, ctx.split), None, None    # P = V^T V is symmetric
+
+
+def low_pass(x, basis, split=None):
+    """AOF's low-frequency component y = V^T (V x) per sample and channel (pcd_low_pass in include/pcdist.h):
+    x [B,N,3] fp32 (any strides; y has x's layout), basis V [B,Kl,N] fp32 with rows contiguous along N (a sample stride
+    of 0, e.g. V.expand(B, -1, -1), shares one basis), 1 <= Kl <= N.  Differentiable in x: the backward is the same
+    projection of the incoming gradient, one launch each way; no host synchronisation, so it can be captured in a CUDA
+    graph.  The basis gets no gradient.  split forces the CTAs per sample (testing; the results do not change)."""
+    _check_cloud(x, "x")
+    B, N, _ = x.shape
+    if not 1 <= N <= _lib.LP_MAX_N:
+        raise ValueError(f"low_pass supports 1 <= N <= {_lib.LP_MAX_N}, got N={N}")
+    if not isinstance(basis, torch.Tensor) or basis.dim() != 3 or basis.shape[0] != B or basis.shape[2] != N \
+            or not 1 <= basis.shape[1] <= N:
+        raise ValueError(f"basis must be [{B}, Kl, {N}] with 1 <= Kl <= {N}, got "
+                         f"{tuple(basis.shape) if isinstance(basis, torch.Tensor) else basis!r}")
+    if basis.dtype != torch.float32 or basis.device != x.device:
+        raise ValueError(f"basis must be float32 on {x.device}, got {basis.dtype} on {basis.device}")
+    if basis.stride(2) != 1 or (basis.shape[1] > 1 and basis.stride(1) != N) or basis.stride(0) < 0:
+        raise ValueError(f"basis rows must be contiguous along N, got strides {basis.stride()}")
+    split = 0 if split is None else int(split)
+    if split < 0 or split > _lib.LP_MAX_SPLIT or split & (split - 1):
+        raise ValueError(f"split must be None, 0 or a power of two <= {_lib.LP_MAX_SPLIT}, got {split}")
+    return _LowPass.apply(x, basis.detach(), split)

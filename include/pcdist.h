@@ -588,6 +588,34 @@ int pcd_si_query_round(const float *logits, int64_t l_sb, int64_t l_sc, int C, c
                        float eps, int max_query, int targeted, int32_t *active /*or NULL*/, void *stream);
 
 /* ------------------------------------------------------------------------------------
+ * pcd_low_pass: the low-frequency component of AOF (attack on frequency, attack/AOF/TAOF_attack.py),
+ * restated from the published method: y = V^T (V x) per sample and per channel, where the rows of
+ * V [Kl,N] are the eigenvectors of the Kl smallest eigenvalues of the cloud's graph Laplacian
+ * (pcd_graph_laplacian, then an eigensolver).  With orthonormal rows P = V^T V is a symmetric projector,
+ * so the same call also gives the backward (y = P g).
+ *   basis: V of sample b at basis + b*b_sb, row k at + k*N, contiguous along N (b_sb = 0 shares one
+ *   basis over the batch).  x, y [B,N,3] fp32 via element strides (both the [B,N,3] and the [B,3,N]
+ *   layouts); y must not overlap x.
+ *   1. c[k][ch] = sum over n of V[k,n]*x[n][ch]: lane l of 32 sums the products of n = l (mod 32) in
+ *      ascending n, starting from +0; then the 32 lane sums by an xor butterfly, s += s(lane ^ o) for
+ *      o = 16, 8, 4, 2, 1 (every lane ends with the same value)
+ *   2. y[n][ch] = sum over k ascending of V[k,n]*c[k][ch], starting from +0
+ *   Every multiply and add is rounded to fp32 on its own.
+ * split: 0 picks how many CTAs (a thread-block cluster, up to 8, 16 where the device schedules it)
+ * share a sample from B, N, Kl and the SM count; a power of two <= 16 forces it (testing; the results
+ * do not change).  16 on a device that cannot schedule it returns PCD_ERR_UNSUPPORTED.
+ * A sample's outputs depend only on its own inputs: not on B, split or the strides.
+ * Constraints: B >= 0 (0 is a no-op), N >= 1, 1 <= Kl <= N, b_sb >= 0, no NULL pointer; anything else
+ * returns PCD_ERR_ARG before any CUDA call.  N > PCD_LP_MAX_N returns PCD_ERR_UNSUPPORTED.
+ * Launches: one kernel; no workspace, no host synchronisation.
+ * ---------------------------------------------------------------------------------- */
+#define PCD_LP_MAX_N 16384
+
+int pcd_low_pass(const float *basis, int64_t b_sb, int Kl, const float *x, int64_t x_sb, int64_t x_sp,
+                 int64_t x_sc, int B, int N, float *y, int64_t y_sb, int64_t y_sp, int64_t y_sc, int split,
+                 void *stream);
+
+/* ------------------------------------------------------------------------------------
  * Measurement helper (bench.py): launches ONE FFMA-only probe kernel on `stream` (variant 0 =
  * scalar FFMA, 1 = packed FFMA2) and stores the number of FLOPs that launch performs in
  * *flop_count (HOST pointer).  The caller times it with its own CUDA events: achieved FLOP/s =
